@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the B200-native proposal + NMS + RoI-layer hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload C1 (SURVEY.md 8d): ResNet-50 at 600x1000 -> 38x63 feature map, 9 anchors (scales 128/256/512),
@@ -39,6 +39,7 @@ ROWS, COLS, CHANNELS = 38, 63, 1024
 SCALES = [128, 256, 512]
 STRIDE, TOPK, NMS_THRESH, MAX_BOXES, NUM_ROIS, POOL = 16, 8000, 0.7, 300, 64, 7
 PADDED = -(-MAX_BOXES // NUM_ROIS) * NUM_ROIS          # 320
+POOLED_SAMPLE = 128                                     # RoI rows of the pooled output kept by --dump-outputs
 METRIC = "img/s proposal+NMS+RoIpool @600x1000"
 UNIT = "img/s"
 WORKLOAD = ("C1: ResNet-50 600x1000 -> 38x63x9 anchors (21546/img), top-k 8000, NMS 0.7->300, pad to 320 RoIs, "
@@ -368,6 +369,21 @@ def measure_stages(ops, dev, rank, world, peak, want_dump):
     return ms, nbytes, sizes, dump
 
 
+def output_arrays(rois, scores, count, pooled):
+    """What one step of the timed path returned, as float32 host arrays for --dump-outputs, so that two builds can be
+    compared output for output on the same seeded inputs.  RoIs, scores and counts are kept whole (rows past an image's
+    count are zero); the pooled features (4.1 GB at 64 images) as a fixed, seeded sample of POOLED_SAMPLE (image, RoI
+    row) pairs, 25.7 MB, with the pairs in `pooled_sample_index`."""
+    import torch
+    b, m = pooled.shape[:2]
+    pick = np.sort(np.random.default_rng(0).choice(b * m, size=min(POOLED_SAMPLE, b * m), replace=False))
+    sample = pooled.reshape((b * m,) + tuple(pooled.shape[2:]))[torch.from_numpy(pick).to(pooled.device)]
+    arrays = {"rois": rois, "scores": scores, "count": count, "pooled_sample": sample}
+    arrays = {k: v.cpu().numpy().astype(np.float32) for k, v in arrays.items()}
+    arrays["pooled_sample_index"] = np.stack([pick // m, pick % m], axis=1).astype(np.float32)
+    return arrays
+
+
 def run_ours(args, rank, world, local_rank):
     import tempfile
 
@@ -422,7 +438,7 @@ def run_ours(args, rank, world, local_rank):
             events.append((e0, e1))
         if pending is not None:
             pending.wait()
-        return rois, count, pooled
+        return rois, scores, count, pooled
 
     from faster_rcnn_b200 import ops as pipe_ops
 
@@ -435,7 +451,7 @@ def run_ours(args, rank, world, local_rank):
     for _ in range(args.warmup):
         out = step()
     fence()
-    count0 = out[1].cpu().numpy()
+    count0 = out[2].cpu().numpy()
     sampler = ClockSampler(physical_gpu_index(local_rank)) if rank == 0 else None
     if sampler:
         sampler.start()
@@ -452,6 +468,8 @@ def run_ours(args, rank, world, local_rank):
     launches = ctx.launches - launches0
     ms = start.elapsed_time(stop)
     roi_ms = float(np.mean([a.elapsed_time(b) for a, b in events]))
+    # with several GPUs only rank 0's own images are kept
+    dumped = output_arrays(*out) if args.dump_outputs and rank == 0 else None
     del out
 
     # ---- end to end through the public API: pinned host inputs, H2D + compute + D2H every step -----------------
@@ -484,6 +502,11 @@ def run_ours(args, rank, world, local_rank):
     assert np.array_equal(res[2], count0), "device-feature e2e path and device path disagree"
     del res
     clocks = sampler.stop() if sampler else None
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
+        del dumped
 
     # ---- sustained window: >= 2 s of back-to-back steps (the GPU reaches its power cap), RoI kernel timed every 8th step
     sus_sampler = ClockSampler(physical_gpu_index(local_rank)) if rank == 0 else None
@@ -607,6 +630,10 @@ def main():
     ap.add_argument("--cpu-images", type=int, default=128, help="bounded sample for cpu_baseline")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--sustained-seconds", type=float, default=2.2, help="length of the power-capped window")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="--impl ours: after the timed steps, write the last step's RoIs, scores, counts and a seeded "
+                         "sample of the pooled features to DIR/<name>.npy (float32); with several GPUs, those of "
+                         "rank 0's own images")
     ap.add_argument("--check-decode", default="", help=argparse.SUPPRESS)
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
@@ -614,6 +641,8 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to --impl ours only")
         run_reference(args, rank, world if world == args.gpus else args.gpus)
         return
     if world != args.gpus:

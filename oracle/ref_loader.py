@@ -1,10 +1,11 @@
 """Loads the UNMODIFIED reference modules for oracle validation and golden generation.
 
-Test infrastructure only.  Works only where /root/reference exists (the
-authoring container); the GPU box has no reference, so nothing under
+Test infrastructure only.  Works only where a checkout of the reference
+(Kelicious/faster_rcnn) is present: at oracle/_ref/ (git-ignored), or wherever
+FRCNN_REFERENCE_DIR names its `faster_rcnn` module folder.  Nothing under
 `-m gpu`, smoke() or bench.py may call this.  The reference is a flat script
-directory (modules import each other by bare name), so its folder is pushed
-on sys.path; `@profile` (custom_decorators.py:8-33) prints a call tree on every
+directory (modules import each other by bare name), so its folder is pushed on
+sys.path; `@profile` (custom_decorators.py:8-33) prints a call tree on every
 call, which `quiet()` swallows.
 """
 import contextlib
@@ -12,7 +13,10 @@ import io
 import os
 import sys
 
-REF_DIR = os.environ.get("FRCNN_REFERENCE_DIR", "/root/reference/faster_rcnn")
+REF_DIR = os.environ.get("FRCNN_REFERENCE_DIR",
+                         os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref", "faster_rcnn"))
+# the VOC2007 annotations the reference ships next to its module folder
+VOC_DIR = os.path.join(os.path.dirname(os.path.abspath(REF_DIR)), "test_data", "VOC_test")
 
 
 def available():
@@ -22,7 +26,8 @@ def available():
 def load():
     """Returns a namespace with the numpy-only reference modules."""
     if not available():
-        raise RuntimeError("reference not present at %s" % REF_DIR)
+        raise RuntimeError("reference not present: check it out at oracle/_ref/ or set FRCNN_REFERENCE_DIR "
+                           "to its faster_rcnn folder")
     if REF_DIR not in sys.path:
         sys.path.insert(0, REF_DIR)
     import types

@@ -1,9 +1,9 @@
-"""Generates tests/golden/*.npz by running the UNMODIFIED reference (imported from
-/root/reference/faster_rcnn) on seeded synthetic inputs and on the one VOC image it ships.
+"""Generates tests/golden/*.npz by running the UNMODIFIED reference (a checkout of
+Kelicious/faster_rcnn, see oracle/ref_loader.py) on seeded synthetic inputs and on the
+one VOC image it ships:
 
-Run in the authoring container only (the GPU box has no reference checkout):
-
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py     # reference checked out at oracle/_ref/, or
+    FRCNN_REFERENCE_DIR=<checkout>/faster_rcnn python tests/golden/make_golden.py
 
 Every fixture stores the inputs next to the reference's outputs, so the tests do not depend on
 regenerating the inputs bit-for-bit.  Sizes are kept small (a few hundred KB compressed in total).
@@ -71,7 +71,7 @@ def voc_gt_case(ref, n_images=200):
     """Real ground truth: the first `n_images` VOC2007 trainval annotations the reference ships
     (test_data/VOC_test, XML only), resized like training (600/1000), with a digest of the reference's labels."""
     import hashlib
-    root = '/root/reference/test_data/VOC_test'
+    root = ref_loader.VOC_DIR
     names = [l.strip() for l in open(root + '/ImageSets/Main/trainval.txt')][:n_images]
     dims = ref.util.get_anchors([128, 256, 512])
     rows, offs, whs, digests, npos, nuse = [], [0], [], [], [], []
@@ -100,7 +100,7 @@ def voc_eval_case(n_images=400):
     sys.path.insert(0, ref_loader.REF_DIR)
     import eval_dets as ref_eval
     from data.voc_data_helpers import extract_img_data
-    root = '/root/reference/test_data/VOC_test'
+    root = ref_loader.VOC_DIR
     names = [l.strip() for l in open(root + '/ImageSets/Main/trainval.txt')][:n_images]
     rng = np.random.default_rng(7)
     out = {'names': np.array(names)}
@@ -151,7 +151,7 @@ def main():
     proposals_case(ref, "kitti_small", 10, 24, None, 103, 3000, 500, True)
 
     # T1-T7: RPN labels.  (a) the one real VOC image, (b) synthetic 50 GT
-    img = ref.voc.extract_img_data('/root/reference/test_data/VOC_test', '000005').resize_within_bounds(600, 1000)[0]
+    img = ref.voc.extract_img_data(ref_loader.VOC_DIR, '000005').resize_within_bounds(600, 1000)[0]
     dims = ref.util.get_anchors([128, 256, 512])
     labels_case(ref, "000005_resnet", img, dims, O.conv_dims_resnet)
     labels_case(ref, "000005_vgg", img, dims, O.conv_dims_vgg)

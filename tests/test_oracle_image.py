@@ -6,9 +6,10 @@ import numpy as np
 import pytest
 
 from oracle import image_oracle as IO
+from oracle import ref_loader
 
 cv2 = pytest.importorskip("cv2")
-REF_VOC = "/root/reference/test_data/VOC_test"
+REF_VOC = ref_loader.VOC_DIR
 
 
 def _natural(h, w, seed):
@@ -92,10 +93,9 @@ def test_voc_loader_conventions(tmp_path):
     assert np.array_equal(big.data, want)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_VOC), reason="reference checkout not present")
+@pytest.mark.skipif(not (ref_loader.available() and os.path.isdir(REF_VOC)), reason="reference checkout not present")
 def test_voc_loader_equals_the_reference_on_its_own_test_data():
     from faster_rcnn_b200.data import voc_data_helpers as V
-    from oracle import ref_loader
     ref = ref_loader.load()
     from data import voc_data_helpers as RV                         # the reference's module (ref_loader set sys.path)
     names = RV.get_img_names_from_set(REF_VOC, "trainval")

@@ -1,8 +1,9 @@
 """Pins the numpy oracle against the UNMODIFIED reference, imported live.
 
-Runs only where /root/reference exists (authoring container); on the GPU box
-the committed fixtures under tests/golden/ (made by make_golden.py from the
-same reference) take over -- see test_oracle_golden.py.
+Runs only where a reference checkout is present (oracle/_ref/ or
+FRCNN_REFERENCE_DIR, see oracle/ref_loader.py); everywhere else the committed fixtures under
+tests/golden/ (made by make_golden.py from the same reference) take over --
+see test_oracle_golden.py and test_oracle_eval.py.
 """
 import random
 
@@ -174,7 +175,7 @@ def test_det_postprocess(ref):
 
 def test_known_answer_000005(ref):
     """SURVEY.md section 8c (ii): labelling known-answer on the one shipped VOC image."""
-    img = ref.voc.extract_img_data('/root/reference/test_data/VOC_test', '000005').resize_within_bounds(600, 1000)[0]
+    img = ref.voc.extract_img_data(ref_loader.VOC_DIR, '000005').resize_within_bounds(600, 1000)[0]
     assert (img.width, img.height) == (800, 600)
     dims = O.anchor_table([128, 256, 512])
     gt = ref.util.get_bbox_coords(img.gt_boxes)
@@ -194,7 +195,7 @@ def test_voc_eval_live(ref, tmp_path):
     from oracle import eval_oracle as E
     sys.path.insert(0, ref_loader.REF_DIR)
     import eval_dets as ref_eval
-    root = '/root/reference/test_data/VOC_test'
+    root = ref_loader.VOC_DIR
     names = [l.strip() for l in open(root + '/ImageSets/Main/trainval.txt')][400:520]
     rng = np.random.default_rng(11)
     iset = tmp_path / 'set.txt'
