@@ -38,8 +38,7 @@ def build(force=False, verbose=False):
     """Compile every CUDA source into faster_rcnn_b200/libfrcnn_b200.so.  Returns the path."""
     if not force and not _stale():
         return OUT
-    extra = os.environ.get("FRCNN_NVCC_EXTRA", "").split()          # experiments only, e.g. -DFRCNN_NMS_THREADS=1024
-    cmd = [_nvcc()] + NVCC_FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + SOURCES + ["-o", OUT + ".tmp"]
+    cmd = [_nvcc()] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + SOURCES + ["-o", OUT + ".tmp"]
     res = subprocess.run(cmd, cwd=CSRC, capture_output=True, text=True)
     if res.returncode != 0:
         raise RuntimeError("nvcc failed:\n%s\n%s" % (res.stdout, res.stderr))

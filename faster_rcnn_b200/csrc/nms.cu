@@ -22,7 +22,6 @@
 #include <cooperative_groups.h>
 
 #include <math.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 
@@ -526,8 +525,6 @@ int launch_nms_i16(frcnn_handle* h, cudaStream_t stream, const int16_t* boxes, c
     // while SMs are idle
     while (cl < 8 && (long long)batch * cl * 2 <= h->sm_count) cl <<= 1;
   }
-  if (getenv("FRCNN_NMS_CL")) cl = atoi(getenv("FRCNN_NMS_CL"));     // experiment knob
-  if (cl < 1 || cl > 16 || (cl & (cl - 1))) cl = 1;
   const int keep_local = (max_keep + cl - 1) / cl;
   const size_t smem = align_up((size_t)buf_elems * 8, 16) + (size_t)keep_local * (16 + 4) + (size_t)max_keep * 4 + 16;
   if (smem + 2048 > (size_t)h->max_smem_optin)

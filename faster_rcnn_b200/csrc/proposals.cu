@@ -30,8 +30,6 @@
 //   det_util.py:179-192 sanitize order, :196-205 validity, :68-76/:147-155 sort + top-k + int16
 #include <cooperative_groups.h>
 
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace cg = cooperative_groups;
@@ -686,11 +684,6 @@ static int launch_proposals_e(frcnn_handle* h, cudaStream_t stream, const Propos
   }
 }
 
-static int env_int(const char* name, int fallback) {
-  const char* v = getenv(name);
-  return (v && *v) ? atoi(v) : fallback;
-}
-
 int launch_decode_topk(frcnn_handle* h, cudaStream_t stream, const float* regr, const float* cls,
                        const AnchorTable& tab, int rows, int cols, int k, int batch,
                        int16_t* out_boxes, float* out_scores, int32_t* out_index,
@@ -738,12 +731,9 @@ int launch_decode_topk(frcnn_handle* h, cudaStream_t stream, const float* regr, 
     const int half = (k + 1999) / 2000;
     if ((long long)batch * splits > 4LL * h->sm_count && (long long)batch * half <= 3LL * h->sm_count && half >= 1) splits = half;
   }
-  splits = env_int("FRCNN_TOPK_SPLITS", splits);      // experiment knobs (benchmarks/prop_one.py)
-  if (splits < 1) splits = 1;
+  // 1000-rank slices number more than 16 above k = 16000, 2000-rank ones above k = 32000
   if (splits > MAX_SPLITS) splits = MAX_SPLITS;
-  bool wide = (long long)batch * splits <= h->sm_count;
-  const int force_threads = env_int("FRCNN_TOPK_THREADS", 0);
-  if (force_threads) wide = force_threads == 1024;
+  const bool wide = (long long)batch * splits <= h->sm_count;
   for (;; splits = (splits + 1) / 2) {
     const int slice = (k + splits - 1) / splits;
     int e = 1;

@@ -23,8 +23,6 @@
 //   top = tl + (tr-tl)*lx; bottom = bl + (br-bl)*lx; out = top + (bottom-top)*ly
 // MAX mode: bin rows y1+floor(ph*h/P) .. y1+ceil((ph+1)*h/P)-1, first maximum in row-major scan.
 // This TU is compiled with -fmad=false so that a*b+c keeps two roundings like the CPU oracle.
-#include <stdlib.h>
-
 #include "roi_common.cuh"
 
 namespace frcnn {
@@ -761,11 +759,8 @@ int launch_roi_bwd(frcnn_handle* h, cudaStream_t stream, int mode, const float* 
   }
   const bool aligned = (reinterpret_cast<uintptr_t>(gout) % 16 == 0) && (reinterpret_cast<uintptr_t>(gfeat) % 16 == 0) &&
                        (mode != FRCNN_ROI_MAX || reinterpret_cast<uintptr_t>(argmax) % 16 == 0);
-  {
-    const char* impl = getenv("FRCNN_BWD_IMPL");          // "cell": force the round-1 cell-stationary kernels (A/B runs)
-    if (aligned && roi_bwd_blk_eligible(mode, H, W, C, N, P) && !(impl && impl[0] == 'c'))
-      return launch_roi_bwd_blk(h, stream, mode, gout, rois, dtype, argmax, H, W, C, N, P, batch, gfeat, 0);
-  }
+  if (aligned && roi_bwd_blk_eligible(mode, H, W, C, N, P))
+    return launch_roi_bwd_blk(h, stream, mode, gout, rois, dtype, argmax, H, W, C, N, P, batch, gfeat, 0);
   if (C % 4 == 0 && aligned && P <= ROI_MAX_TABLE_P && H < 32768 && W < 32768) {
     int4 *crops = nullptr, *taps = nullptr;
     int rc = build_tables(h, stream, mode, rois, dtype, batch * N, W, H, P, &crops, &taps);

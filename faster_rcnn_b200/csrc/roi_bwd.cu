@@ -20,8 +20,6 @@
 // take) a dY row is fetched by 2.06 blocks instead of 3.48 cells in resize mode (2.64 instead of 5.02 bin
 // covers in max mode, C5 RoIs), the crop / tap-table round trips that serialised every RoI chunk are gone, and
 // twice the bytes are in flight per SM.
-#include <stdlib.h>
-
 #include <type_traits>
 
 #include "roi_common.cuh"
@@ -550,15 +548,10 @@ static int launch_blk_parts(frcnn_handle* h, cudaStream_t stream, int parts, int
     FRCNN_BLK_CASE(1)
     FRCNN_BLK_CASE(2)
     FRCNN_BLK_CASE(4)
+    default:
     FRCNN_BLK_CASE(8)
   }
 #undef FRCNN_BLK_CASE
-  return fail(h, FRCNN_ERR_INVALID, "roi_bwd: bad slice count%s%s");
-}
-
-static int env_int(const char* name, int dflt) {
-  const char* v = getenv(name);
-  return (v && *v) ? atoi(v) : dflt;
 }
 
 // true when the block path takes this problem
@@ -617,12 +610,10 @@ int launch_roi_bwd_blk(frcnn_handle* h, cudaStream_t stream, int mode, const flo
   FRCNN_LAUNCH_CHECK(h, "roi_bwd_plan_kernel");
 
   // (channels per lane, ring depth): 2 x 8 = 8 KB of dY in flight per warp where 256 channels exist; the int32 max mode
-  // carries an arg-max row as large as the dY row and keeps 1 x 8 (same-box A/B, benchmarks/bwd_ab.py: C5 x 8 resize
-  // 0.66 ms against 0.68 (2 x 4) / 0.75 (1 x 8) / 0.80 (1 x 16); max 1.32 against 1.30 (2 x 4) / 1.56 (1 x 4);
-  // one-byte arg-max 1.15 (2 x 8) against 1.25 (2 x 4) / 1.40 (1 x 8)).  FRCNN_BWD_CPB=1 selects the narrow variant.
-  int cpb = env_int("FRCNN_BWD_CPB", C >= 256 ? 2 : 1);
-  const int depth = 8;
-  if (cpb != 1 && cpb != 2) cpb = 1;
+  // carries an arg-max row as large as the dY row and keeps 1 x 8 (same-box A/B on a B200, C5 x 8: resize 0.66 ms
+  // against 0.68 (2 x 4) / 0.75 (1 x 8) / 0.80 (1 x 16); max 1.32 against 1.30 (2 x 4) / 1.56 (1 x 4); one-byte
+  // arg-max 1.15 (2 x 8) against 1.25 (2 x 4) / 1.40 (1 x 8)).
+  int cpb = C >= 256 ? 2 : 1;
   if (mode == FRCNN_ROI_MAX && !compact) cpb = 1;
   const int slabs = (C + cpb * 128 - 1) / (cpb * 128);
   const bool full = C % (cpb * 128) == 0;
@@ -636,7 +627,6 @@ int launch_roi_bwd_blk(frcnn_handle* h, cudaStream_t stream, int mode, const flo
   if (parts < 4 && avg_list >= 256) parts = 4;
   else if (parts < 2 && avg_list >= 128) parts = 2;
   if (N < 256) parts = 1;                              // short lists: one warp walks the whole list (reference order)
-  parts = env_int("FRCNN_BWD_PARTS", parts);
   const int2* tab = static_cast<int2*>(p_tab);
   const unsigned* eidx = static_cast<unsigned*>(p_idx);
   const float4* ew = static_cast<float4*>(p_w);
@@ -645,7 +635,6 @@ int launch_roi_bwd_blk(frcnn_handle* h, cudaStream_t stream, int mode, const flo
                                                      W, C, N, P, blocks_x, n_blocks, gfeat)                         \
               : launch_blk_parts<MODE, CPB, D, false>(h, stream, parts, slabs, batch, gout, argmax, tab, eidx, ew,  \
                                                       H, W, C, N, P, blocks_x, n_blocks, gfeat);
-  (void)depth;
   if (mode == FRCNN_ROI_RESIZE) {
     if (cpb == 2) { FRCNN_BLK_GO(FRCNN_ROI_RESIZE, 2, 8) }
     FRCNN_BLK_GO(FRCNN_ROI_RESIZE, 1, 8)

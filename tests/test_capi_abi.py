@@ -49,6 +49,14 @@ def test_library_carries_sm100a_code_only(lib):
     assert archs == {"100a"}, archs
 
 
+def test_sources_read_no_environment_variables():
+    """Launch configurations follow from the source, the problem shape and the device alone."""
+    csrc = os.path.join(ROOT, "faster_rcnn_b200", "csrc")
+    for name in sorted(os.listdir(csrc)):
+        with open(os.path.join(csrc, name)) as f:
+            assert "getenv" not in f.read(), name
+
+
 def test_abi_version_and_loud_failure_without_gpu(lib):
     import torch
     assert lib.frcnn_abi_version() == 1

@@ -126,6 +126,29 @@ def test_roi_backward_kernel_variants(ops, b, h, w, c, n, pool):
             assert np.abs(gm[i] - wm).max() <= 1e-5 * np.abs(wm).max()
 
 
+def test_roi_backward_ignores_environment(ops, monkeypatch):
+    """The work-list backward picks its variant from the shape and the device: variables that once overrode the variant,
+    the channels per lane or the list slices change neither the gradients nor whether the call succeeds."""
+    import torch
+    b, h, w, c, n, pool = 2, 14, 15, 256, 40, 7
+    rng = np.random.default_rng(b * h + c + n)
+    feat = rng.standard_normal((b, h, w, c), dtype=np.float32)
+    rois = dev(np.stack([_rois(rng, n, h, w) for _ in range(b)]))
+    gout = dev(rng.standard_normal((b, n, pool, pool, c), dtype=np.float32))
+    _, arg = ops.roi_forward(dev(feat), rois, pool, "max")
+
+    def grads():
+        return (ops.roi_backward(gout, rois, (b, h, w, c), "resize"),
+                ops.roi_backward(gout, rois, (b, h, w, c), "max", argmax=arg))
+
+    first = grads()
+    for name, value in (("FRCNN_BWD_PARTS", "3"), ("FRCNN_BWD_IMPL", "cell"), ("FRCNN_BWD_CPB", "1")):
+        with monkeypatch.context() as m:
+            m.setenv(name, value)
+            for got, want in zip(grads(), first):
+                assert torch.equal(got, want), name
+
+
 def test_roi_full_size_properties(ops):
     """C5 shape (38x63x1024, 2000 RoIs): <dY, fwd(X)> == <bwd(dY), X> (the backward is the exact adjoint of
     the forward), linearity of the forward, and a spot check of 16 RoIs against the oracle."""
