@@ -2,7 +2,7 @@
 // the per-handle scratch arena and the dispatch to the kernel launchers of the other TUs.
 #include <new>
 
-#include "common.cuh"
+#include "roi_common.cuh"
 
 namespace frcnn {
 
@@ -23,7 +23,6 @@ int launch_roi_fwd(frcnn_handle*, cudaStream_t, int, const float*, int, int, int
                    float*, int32_t*, int);
 int launch_roi_bwd(frcnn_handle*, cudaStream_t, int, const float*, const void*, int, const int32_t*, int, int, int,
                    int, int, int, float*, int);
-bool roi_compact_supported(int, int, int, int);
 int launch_det_postprocess(frcnn_handle*, cudaStream_t, const int16_t*, const float*, const float*, const double*,
                            const int32_t*, int, int, int, int, double, double, int, int, int32_t*, float*, int32_t*, int32_t*);
 

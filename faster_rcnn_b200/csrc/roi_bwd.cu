@@ -16,10 +16,14 @@
 // oldest one issue, and the list entries are staged the same way 32 at a time.  Slices of one block are added
 // in slice order through shared memory: no atomics, one fixed summation order, bit-reproducible run to run.
 //
-// Against the cell-stationary gather of round 1 (kept in roi.cu for pool sizes / layouts this path does not
-// take) a dY row is fetched by 2.06 blocks instead of 3.48 cells in resize mode (2.64 instead of 5.02 bin
-// covers in max mode, C5 RoIs), the crop / tap-table round trips that serialised every RoI chunk are gone, and
-// twice the bytes are in flight per SM.
+// Against the cell-stationary gather of round 1 a dY row is fetched by 2.06 blocks instead of 3.48 cells in resize
+// mode (2.64 instead of 5.02 bin covers in max mode, C5 RoIs), the crop / tap-table round trips that serialised every
+// RoI chunk are gone, and twice the bytes are in flight per SM.
+//
+// This path takes every pool size up to ROI_MAX_TABLE_P and any RoI count whose work list fits its index formats
+// (roi_bwd_blk_eligible); the plan step has a narrow instance (one-byte masks, P <= 8 and N < 65536: the tuned shapes)
+// and a wide one (32-bit masks).  Everything else -- C % 4 != 0, unaligned buffers, larger pools or maps -- takes the
+// scalar-channel kernel at the end of this file.
 #include <type_traits>
 
 #include "roi_common.cuh"
@@ -58,19 +62,19 @@ __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_gr
 // ---------------------------------------------------------------------------------------
 // Which outputs of a RoI touch a block separates per axis: bin (ph, pw) touches block (by, bx) iff output row ph
 // touches block row by and output column pw touches block column bx.  roi_bwd_mask_kernel writes those two
-// relations once per (RoI, block row) and (RoI, block column) as P-bit masks (P <= 8), laid out [axis block][RoI]
-// so that the plan kernel's RoI sweep is a coalesced byte stream: the sweep then costs a few instructions per
-// 32 RoIs instead of re-deriving the taps of every RoI in every block (the first version of this file did that
-// and spent 270 us on the C5 x 8 plan against 630 us for the streaming kernel).
-template <int MODE>
+// relations once per (RoI, block row) and (RoI, block column) as P-bit masks M (uint8_t for P <= 8, else uint32_t),
+// laid out [axis block][RoI] so that the plan kernel's RoI sweep is a coalesced stream: the sweep then costs a few
+// instructions per 32 RoIs instead of re-deriving the taps of every RoI in every block (the first version of this
+// file did that and spent 270 us on the C5 x 8 plan against 630 us for the streaming kernel).
+template <int MODE, typename M>
 __global__ void __launch_bounds__(256)
 roi_bwd_mask_kernel(const void* __restrict__ rois, int dtype, int N, int n_pad, int H, int W, int P, int blocks_y,
-                    int blocks_x, uint8_t* __restrict__ ymask, uint8_t* __restrict__ xmask, unsigned* __restrict__ counter) {
+                    int blocks_x, M* __restrict__ ymask, M* __restrict__ xmask, unsigned* __restrict__ counter) {
   const int r = blockIdx.x * 256 + threadIdx.x, ab = blockIdx.y, img = blockIdx.z;   // ab: block rows, then block columns
   if (r == 0 && ab == 0) counter[img] = 0u;              // the plan kernel's bump allocators (saves a memset node per call)
   if (r >= n_pad) return;
   const bool is_y = ab < blocks_y;
-  uint8_t* dst = is_y ? ymask + ((size_t)img * blocks_y + ab) * n_pad : xmask + ((size_t)img * blocks_x + (ab - blocks_y)) * n_pad;
+  M* dst = is_y ? ymask + ((size_t)img * blocks_y + ab) * n_pad : xmask + ((size_t)img * blocks_x + (ab - blocks_y)) * n_pad;
   if (r >= N) {                                        // padding reads as "touches nothing"
     dst[r] = 0;
     return;
@@ -93,7 +97,7 @@ roi_bwd_mask_kernel(const void* __restrict__ rois, int dtype, int N, int n_pad, 
       }
     }
   }
-  dst[r] = (uint8_t)m;
+  dst[r] = (M)m;
 }
 
 // weights of the block's two rows (columns) for output index p of one axis, and which of them a tap lands on
@@ -111,7 +115,7 @@ __device__ __forceinline__ unsigned axis_weights(int p, float scale, int in_size
   return hit;
 }
 
-// k / n for k < 64, 1 <= n <= 8 (multiply-shift, exact on that range)
+// k / n for k < 64, 1 <= n <= 8 (multiply-shift, exact on that range): the narrow plan's entry decode
 __constant__ unsigned short c_div_magic[9] = {0, 512, 256, 171, 128, 103, 86, 74, 64};
 
 // One CTA per block; warp w sweeps the w-th contiguous eighth of the RoIs (so the list order is warp-major = RoI
@@ -123,16 +127,23 @@ constexpr int PLAN_ROUND = 256;              // RoIs per queue round and warp
 // PER_WARP: every warp of the CTA plans a block of its own (short RoI lists, e.g. 320 RoIs x 64 images = 38912 blocks:
 // with one CTA per block the launch is a queue of tiny CTAs whose barriers and allocation round trip are exposed 260
 // times per SM; with independent warps four times as many chains are in flight).
-template <int MODE, int WARPS, bool PER_WARP>
+// M: the mask word.  uint8_t (P <= 8, N < 65536) packs a queued RoI into one word and decodes an entry with a
+// multiply-shift division and bit clearing; uint32_t keeps the full RoI index and both masks, whose rounds can hold
+// 256 RoIs x 1024 entries.
+template <int MODE, typename M, int WARPS, bool PER_WARP>
 __global__ void __launch_bounds__(WARPS * 32)
 roi_bwd_plan_kernel(const void* __restrict__ rois, int dtype, int N, int n_pad, int H, int W, int P, int blocks_y,
-                    int blocks_x, unsigned capacity, const uint8_t* __restrict__ ymask,
-                    const uint8_t* __restrict__ xmask, unsigned* __restrict__ counter, int2* __restrict__ blk_tab,
+                    int blocks_x, unsigned capacity, const M* __restrict__ ymask,
+                    const M* __restrict__ xmask, unsigned* __restrict__ counter, int2* __restrict__ blk_tab,
                     unsigned* __restrict__ ent_idx, float4* __restrict__ ent_w) {
+  constexpr bool WIDE = sizeof(M) == 4;
+  using M4 = std::conditional_t<WIDE, uint4, uchar4>;
+  using Rec = std::conditional_t<WIDE, uint3, unsigned>;   // narrow: RoI index | my << 16 | mx << 24; wide: (r, my, mx)
+  using Start = std::conditional_t<WIDE, int, unsigned short>;
   __shared__ int s_wtot[WARPS];
   __shared__ unsigned s_wbase[WARPS];
-  __shared__ unsigned s_qroi[WARPS][PLAN_ROUND];            // RoI index | my << 16 | mx << 24
-  __shared__ unsigned short s_qstart[WARPS][PLAN_ROUND];    // first entry of the RoI inside the round
+  __shared__ Rec s_qroi[WARPS][PLAN_ROUND];
+  __shared__ Start s_qstart[WARPS][PLAN_ROUND];             // first entry of the RoI inside the round
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   constexpr int VW = PER_WARP ? 1 : WARPS;                  // warps that share one block's RoIs
   const int vwarp = PER_WARP ? 0 : warp;
@@ -140,15 +151,15 @@ roi_bwd_plan_kernel(const void* __restrict__ rois, int dtype, int N, int n_pad, 
   if (PER_WARP && b >= n_blocks) return;
   const int by = b / blocks_x, bx = b - by * blocks_x;
   const int Y0 = by * BLK, X0 = bx * BLK;
-  const uint8_t* ym = ymask + ((size_t)img * blocks_y + by) * n_pad;
-  const uint8_t* xm = xmask + ((size_t)img * blocks_x + bx) * n_pad;
+  const M* ym = ymask + ((size_t)img * blocks_y + by) * n_pad;
+  const M* xm = xmask + ((size_t)img * blocks_x + bx) * n_pad;
   const int per_warp = ((N + VW - 1) / VW + 31) / 32 * 32;
   const int r_lo = min(n_pad, vwarp * per_warp), r_hi = min(n_pad, r_lo + per_warp);   // padding masks are zero
 
   // pass 1: entries of this warp's RoI range (four RoIs per lane and step)
   int mine = 0;
   for (int r = r_lo + 4 * lane; r < r_hi; r += 128) {
-    const uchar4 a = *reinterpret_cast<const uchar4*>(ym + r), c = *reinterpret_cast<const uchar4*>(xm + r);
+    const M4 a = *reinterpret_cast<const M4*>(ym + r), c = *reinterpret_cast<const M4*>(xm + r);
     mine += __popc(a.x) * __popc(c.x) + __popc(a.y) * __popc(c.y) + __popc(a.z) * __popc(c.z) + __popc(a.w) * __popc(c.w);
   }
 #pragma unroll
@@ -196,8 +207,8 @@ roi_bwd_plan_kernel(const void* __restrict__ rois, int dtype, int N, int n_pad, 
   }
 
   // pass 2: the entries, RoIs in index order, (ph, pw) row-major inside a RoI
-  unsigned* qroi = s_qroi[warp];
-  unsigned short* qstart = s_qstart[warp];
+  Rec* qroi = s_qroi[warp];
+  Start* qstart = s_qstart[warp];
   for (int round_lo = r_lo; round_lo < r_hi; round_lo += PLAN_ROUND) {
     const int round_hi = min(r_hi, round_lo + PLAN_ROUND);
     int nq = 0, ne = 0;                                  // queued RoIs / entries of this round (warp-uniform)
@@ -224,8 +235,9 @@ roi_bwd_plan_kernel(const void* __restrict__ rois, int dtype, int N, int n_pad, 
       }
       if (cnt > 0) {
         const int q = nq + __popc(hits & ((1u << lane) - 1u));
-        qroi[q] = (unsigned)r | (my << 16) | (mx << 24);
-        qstart[q] = (unsigned short)(ne + incl - cnt);
+        if constexpr (WIDE) qroi[q] = make_uint3((unsigned)r, my, mx);
+        else qroi[q] = (unsigned)r | (my << 16) | (mx << 24);
+        qstart[q] = (Start)(ne + incl - cnt);
       }
       nq += __popc(hits);
       ne += __shfl_sync(0xffffffffu, incl, 31);
@@ -237,7 +249,7 @@ roi_bwd_plan_kernel(const void* __restrict__ rois, int dtype, int N, int n_pad, 
     auto generate = [&](auto eu_tag) {
     constexpr int EU = decltype(eu_tag)::value;
     for (int e0 = lane; e0 < ne; e0 += 32 * EU) {
-      unsigned rec[EU];
+      Rec rec[EU];
       int kk[EU];
 #pragma unroll
       for (int u = 0; u < EU; ++u) {
@@ -254,16 +266,27 @@ roi_bwd_plan_kernel(const void* __restrict__ rois, int dtype, int N, int n_pad, 
 #pragma unroll
       for (int u = 0; u < EU; ++u) {
         const int e = e0 + 32 * u;
-        const int r = (int)(rec[u] & 0xffffu);
-        unsigned my = (rec[u] >> 16) & 0xffu, mx = rec[u] >> 24;
-        const int k = kk[u], nx = __popc(mx);
-        const int iy = (int)((unsigned)k * c_div_magic[nx]) >> 9, ix = k - iy * nx;
+        int r, ph, pw;                                   // entry k of a RoI is bin (iy-th bit of my, ix-th bit of mx)
+        if constexpr (WIDE) {
+          r = (int)rec[u].x;
+          const unsigned my = rec[u].y, mx = rec[u].z;
+          const int k = kk[u], nx = __popc(mx);
+          const int iy = k / nx, ix = k - iy * nx;
+          ph = (int)__fns(my, 0, iy + 1);
+          pw = (int)__fns(mx, 0, ix + 1);
+        } else {
+          r = (int)(rec[u] & 0xffffu);
+          unsigned my = (rec[u] >> 16) & 0xffu, mx = rec[u] >> 24;
+          const int k = kk[u], nx = __popc(mx);
+          const int iy = (int)((unsigned)k * c_div_magic[nx]) >> 9, ix = k - iy * nx;
 #pragma unroll
-        for (int i = 0; i < 7; ++i) {                    // masks have at most 8 bits: drop the iy / ix lowest ones
-          if (i < iy) my &= my - 1u;
-          if (i < ix) mx &= mx - 1u;
+          for (int i = 0; i < 7; ++i) {                  // masks have at most 8 bits: drop the iy / ix lowest ones
+            if (i < iy) my &= my - 1u;
+            if (i < ix) mx &= mx - 1u;
+          }
+          ph = __ffs(my) - 1;
+          pw = __ffs(mx) - 1;
         }
-        const int ph = __ffs(my) - 1, pw = __ffs(mx) - 1;
         const unsigned row = (unsigned)((r * P + ph) * P + pw);
         const unsigned pos = pos_warp + (unsigned)e;
         const bool live = e < ne;
@@ -554,57 +577,72 @@ static int launch_blk_parts(frcnn_handle* h, cudaStream_t stream, int parts, int
 #undef FRCNN_BLK_CASE
 }
 
-// true when the block path takes this problem
-bool roi_bwd_blk_eligible(int mode, int H, int W, int C, int N, int P) {
-  (void)mode;
-  return C % 4 == 0 && P <= 8 && N < 65536 && H < 32768 && W < 32768 && (long long)N * P * P < (1LL << ENT_MASK_SHIFT);
-}
-
-int launch_roi_bwd_blk(frcnn_handle* h, cudaStream_t stream, int mode, const float* gout, const void* rois, int dtype,
-                       const int32_t* argmax, int H, int W, int C, int N, int P, int batch, float* gfeat, int compact) {
-  const int blocks_x = (W + BLK - 1) / BLK, blocks_y = (H + BLK - 1) / BLK, n_blocks = blocks_x * blocks_y;
-  // upper bound of the list entries: a resize bin has taps in <= 2 x 2 blocks; a max bin spans <= ceil(H/P)+1 rows
+// upper bound of the work-list entries of a launch: a resize bin has taps in <= 2 x 2 blocks; a max bin spans
+// <= ceil(H/P)+1 rows and columns
+static long long work_list_entries(int mode, int H, int W, int N, int P, int batch) {
   long long per_bin = 4;
   if (mode == FRCNN_ROI_MAX) {
     const long long ly = (H + P - 1) / P + 1, lx = (W + P - 1) / P + 1;
     per_bin = (ly / BLK + 1) * (lx / BLK + 1);
   }
-  const long long cap = (long long)batch * N * P * P * per_bin;
-  if (cap >= (1LL << 31)) return fail(h, FRCNN_ERR_INVALID, "roi_bwd: work list would exceed 2^31 entries%s%s");
+  return (long long)batch * N * P * P * per_bin;
+}
+
+// true when the work-list path takes this problem: float4 channels, masks of at most 32 bits, dY row indices that fit
+// the entry word and list positions that fit an int
+static bool roi_bwd_blk_eligible(int mode, int H, int W, int C, int N, int P, int batch) {
+  return C % 4 == 0 && P <= ROI_MAX_TABLE_P && H < 32768 && W < 32768 && (long long)N * P * P < (1LL << ENT_MASK_SHIFT) &&
+         work_list_entries(mode, H, W, N, P, batch) < (1LL << 31);
+}
+
+// mask + plan kernels; plan CTAs: 8 warps sweep 2000 RoIs in one queue round each, short RoI lists take smaller CTAs
+// (38912 of them at C1 x 64)
+template <int MODE, typename M>
+static void launch_plan(cudaStream_t stream, const void* rois, int dtype, int N, int n_pad, int H, int W, int P,
+                        int blocks_y, int blocks_x, int batch, unsigned capacity, void* ym, void* xm, unsigned* counter,
+                        int2* tab, unsigned* ent_idx, float4* ent_w) {
+  constexpr int MASK_MODE = MODE == FRCNN_ROI_RESIZE ? FRCNN_ROI_RESIZE : FRCNN_ROI_MAX;
+  M *y = static_cast<M*>(ym), *x = static_cast<M*>(xm);
+  const int n_blocks = blocks_y * blocks_x;
+  roi_bwd_mask_kernel<MASK_MODE, M><<<dim3((n_pad + 255) / 256, blocks_y + blocks_x, batch), 256, 0, stream>>>(
+      rois, dtype, N, n_pad, H, W, P, blocks_y, blocks_x, y, x, counter);
+  if (N > 1024)
+    roi_bwd_plan_kernel<MODE, M, 8, false><<<dim3(n_blocks, batch), 256, 0, stream>>>(
+        rois, dtype, N, n_pad, H, W, P, blocks_y, blocks_x, capacity, y, x, counter, tab, ent_idx, ent_w);
+  else if (N > 512)
+    roi_bwd_plan_kernel<MODE, M, 4, false><<<dim3(n_blocks, batch), 128, 0, stream>>>(
+        rois, dtype, N, n_pad, H, W, P, blocks_y, blocks_x, capacity, y, x, counter, tab, ent_idx, ent_w);
+  else
+    roi_bwd_plan_kernel<MODE, M, 8, true><<<dim3((n_blocks + 7) / 8, batch), 256, 0, stream>>>(
+        rois, dtype, N, n_pad, H, W, P, blocks_y, blocks_x, capacity, y, x, counter, tab, ent_idx, ent_w);
+}
+
+static int launch_roi_bwd_blk(frcnn_handle* h, cudaStream_t stream, int mode, const float* gout, const void* rois,
+                              int dtype, const int32_t* argmax, int H, int W, int C, int N, int P, int batch, float* gfeat,
+                              int compact) {
+  const int blocks_x = (W + BLK - 1) / BLK, blocks_y = (H + BLK - 1) / BLK, n_blocks = blocks_x * blocks_y;
+  const long long cap = work_list_entries(mode, H, W, N, P, batch);
+  const bool wide = P > 8 || N >= 65536;               // the narrow plan's masks are bytes, its queue keeps 16-bit RoIs
+  const size_t mask_bytes = wide ? sizeof(uint32_t) : sizeof(uint8_t);
   const int n_pad = (N + 15) / 16 * 16;
   void *p_cnt = nullptr, *p_tab = nullptr, *p_idx = nullptr, *p_w = nullptr, *p_ym = nullptr, *p_xm = nullptr;
   int rc;
   if ((rc = arena_get(h, stream, align_up((size_t)batch * sizeof(unsigned), 256), &p_cnt))) return rc;
   if ((rc = arena_get(h, stream, (size_t)batch * n_blocks * sizeof(int2), &p_tab))) return rc;
-  if ((rc = arena_get(h, stream, (size_t)batch * blocks_y * n_pad, &p_ym))) return rc;
-  if ((rc = arena_get(h, stream, (size_t)batch * blocks_x * n_pad, &p_xm))) return rc;
+  if ((rc = arena_get(h, stream, (size_t)batch * blocks_y * n_pad * mask_bytes, &p_ym))) return rc;
+  if ((rc = arena_get(h, stream, (size_t)batch * blocks_x * n_pad * mask_bytes, &p_xm))) return rc;
   if ((rc = arena_get(h, stream, (size_t)cap * sizeof(unsigned), &p_idx))) return rc;
   if ((mode == FRCNN_ROI_RESIZE || compact) && (rc = arena_get(h, stream, (size_t)cap * sizeof(float4), &p_w))) return rc;
-  dim3 mgrid((n_pad + 255) / 256, blocks_y + blocks_x, batch), pgrid(n_blocks, batch);
-  uint8_t *ym = static_cast<uint8_t*>(p_ym), *xm = static_cast<uint8_t*>(p_xm);
-  // plan CTAs: 8 warps sweep 2000 RoIs in one queue round each; short RoI lists take smaller CTAs (38912 of them at C1 x 64)
-#define FRCNN_PLAN(MODE, WARPS)                                                                                     \
-  roi_bwd_plan_kernel<MODE, WARPS, false><<<pgrid, WARPS * 32, 0, stream>>>(                                         \
-      rois, dtype, N, n_pad, H, W, P, blocks_y, blocks_x, (unsigned)(cap / batch), ym, xm, static_cast<unsigned*>(p_cnt), \
-      static_cast<int2*>(p_tab), static_cast<unsigned*>(p_idx), static_cast<float4*>(p_w))
-#define FRCNN_PLAN_WARP(MODE)                                                                                       \
-  roi_bwd_plan_kernel<MODE, 8, true><<<dim3((n_blocks + 7) / 8, batch), 256, 0, stream>>>(                            \
-      rois, dtype, N, n_pad, H, W, P, blocks_y, blocks_x, (unsigned)(cap / batch), ym, xm, static_cast<unsigned*>(p_cnt), \
-      static_cast<int2*>(p_tab), static_cast<unsigned*>(p_idx), static_cast<float4*>(p_w))
-#define FRCNN_PLAN_ANY(MODE)                                                                                        \
-  if (N > 1024) FRCNN_PLAN(MODE, 8); else if (N > 512) FRCNN_PLAN(MODE, 4); else FRCNN_PLAN_WARP(MODE)
-  if (mode == FRCNN_ROI_RESIZE) {
-    roi_bwd_mask_kernel<FRCNN_ROI_RESIZE><<<mgrid, 256, 0, stream>>>(rois, dtype, N, n_pad, H, W, P, blocks_y, blocks_x, ym, xm, static_cast<unsigned*>(p_cnt));
-    FRCNN_PLAN_ANY(FRCNN_ROI_RESIZE);
-  } else if (compact) {
-    roi_bwd_mask_kernel<FRCNN_ROI_MAX><<<mgrid, 256, 0, stream>>>(rois, dtype, N, n_pad, H, W, P, blocks_y, blocks_x, ym, xm, static_cast<unsigned*>(p_cnt));
-    FRCNN_PLAN_ANY(ROI_MAX_COMPACT);
-  } else {
-    roi_bwd_mask_kernel<FRCNN_ROI_MAX><<<mgrid, 256, 0, stream>>>(rois, dtype, N, n_pad, H, W, P, blocks_y, blocks_x, ym, xm, static_cast<unsigned*>(p_cnt));
-    FRCNN_PLAN_ANY(FRCNN_ROI_MAX);
-  }
-#undef FRCNN_PLAN_ANY
-#undef FRCNN_PLAN_WARP
+  int2* tab = static_cast<int2*>(p_tab);
+  unsigned* eidx = static_cast<unsigned*>(p_idx);
+  float4* ew = static_cast<float4*>(p_w);
+#define FRCNN_PLAN(MODE, M)                                                                                        \
+  launch_plan<MODE, M>(stream, rois, dtype, N, n_pad, H, W, P, blocks_y, blocks_x, batch, (unsigned)(cap / batch), \
+                       p_ym, p_xm, static_cast<unsigned*>(p_cnt), tab, eidx, ew)
+  if (compact) FRCNN_PLAN(ROI_MAX_COMPACT, uint8_t);   // launch_roi_bwd: the one-byte arg-max has P <= 8, N < 65536
+  else if (mode == FRCNN_ROI_RESIZE) { if (wide) FRCNN_PLAN(FRCNN_ROI_RESIZE, uint32_t); else FRCNN_PLAN(FRCNN_ROI_RESIZE, uint8_t); }
+  else if (wide) FRCNN_PLAN(FRCNN_ROI_MAX, uint32_t);
+  else FRCNN_PLAN(FRCNN_ROI_MAX, uint8_t);
 #undef FRCNN_PLAN
   FRCNN_LAUNCH_CHECK(h, "roi_bwd_mask_kernel");
   FRCNN_LAUNCH_CHECK(h, "roi_bwd_plan_kernel");
@@ -627,9 +665,6 @@ int launch_roi_bwd_blk(frcnn_handle* h, cudaStream_t stream, int mode, const flo
   if (parts < 4 && avg_list >= 256) parts = 4;
   else if (parts < 2 && avg_list >= 128) parts = 2;
   if (N < 256) parts = 1;                              // short lists: one warp walks the whole list (reference order)
-  const int2* tab = static_cast<int2*>(p_tab);
-  const unsigned* eidx = static_cast<unsigned*>(p_idx);
-  const float4* ew = static_cast<float4*>(p_w);
 #define FRCNN_BLK_GO(MODE, CPB, D)                                                                                   \
   return full ? launch_blk_parts<MODE, CPB, D, true>(h, stream, parts, slabs, batch, gout, argmax, tab, eidx, ew, H, \
                                                      W, C, N, P, blocks_x, n_blocks, gfeat)                         \
@@ -645,6 +680,109 @@ int launch_roi_bwd_blk(frcnn_handle* h, cudaStream_t stream, int mode, const flo
   }
   FRCNN_BLK_GO(FRCNN_ROI_MAX, 1, 8)
 #undef FRCNN_BLK_GO
+}
+
+// ---------------------------------------------------------------------------------------
+// scalar-channel fallback for the problems roi_bwd_blk_eligible rejects (C % 4 != 0, pool sizes above
+// ROI_MAX_TABLE_P, ...) and unaligned buffers: 8x8 tile, one channel per thread, every CTA scans all RoIs.
+// Not a performance path.
+// ---------------------------------------------------------------------------------------
+constexpr int BWD_TILE = 8;          // 8x8 cells
+constexpr int BWD_CH = 512;          // channels per CTA = threads per CTA
+
+template <int MODE>
+__global__ void __launch_bounds__(BWD_CH, 1)
+roi_bwd_scalar_kernel(const float* __restrict__ gout, const void* __restrict__ rois, int dtype,
+               const int* __restrict__ argmax, int H, int W, int C, int N, int P, int tiles_x,
+               float* __restrict__ gfeat) {
+  extern __shared__ float acc[];     // [BWD_TILE*BWD_TILE][BWD_CH]
+  const int tile = blockIdx.x, img = blockIdx.z;
+  const int ty0 = (tile / tiles_x) * BWD_TILE, tx0 = (tile % tiles_x) * BWD_TILE;
+  const int ty1 = min(ty0 + BWD_TILE, H), tx1 = min(tx0 + BWD_TILE, W);
+  const int c = blockIdx.y * BWD_CH + threadIdx.x;
+  const bool live = c < C;
+  for (int i = 0; i < BWD_TILE * BWD_TILE; ++i) acc[i * BWD_CH + threadIdx.x] = 0.f;
+
+  const float* g_img = gout + (size_t)img * N * P * P * C + c;
+  const int* a_img = (MODE == FRCNN_ROI_MAX) ? argmax + (size_t)img * N * P * P * C + c : nullptr;
+
+  for (int r = 0; r < N; ++r) {
+    const Crop k = load_crop(rois, dtype, (size_t)img * N + r, W, H);
+    if (k.w <= 0 || k.h <= 0) continue;
+    if (k.x1 >= tx1 || k.x1 + k.w <= tx0 || k.y1 >= ty1 || k.y1 + k.h <= ty0) continue;   // CTA-uniform
+    const float* g_roi = g_img + (size_t)r * P * P * C;
+    if (MODE == FRCNN_ROI_RESIZE) {
+      const float ys = (float)k.h / (float)P, xs = (float)k.w / (float)P;
+      for (int ph = 0; ph < P; ++ph) {
+        const Tap ty = axis_tap(ph, ys, k.h);
+        const int ylo = k.y1 + ty.lo, yhi = k.y1 + ty.hi;
+        const bool rlo = ylo >= ty0 && ylo < ty1, rhi = yhi >= ty0 && yhi < ty1;
+        if (!rlo && !rhi) continue;
+        const float wy1 = ty.lerp, wy0 = 1.0f - ty.lerp;
+        for (int pw = 0; pw < P; ++pw) {
+          const Tap tx = axis_tap(pw, xs, k.w);
+          const int xlo = k.x1 + tx.lo, xhi = k.x1 + tx.hi;
+          const bool clo = xlo >= tx0 && xlo < tx1, chi = xhi >= tx0 && xhi < tx1;
+          if (!clo && !chi) continue;
+          const float g = live ? __ldg(g_roi + (size_t)(ph * P + pw) * C) : 0.f;
+          const float wx1 = tx.lerp, wx0 = 1.0f - tx.lerp;
+          // order TL, TR, BL, BR; weight product (g*wy)*wx as in ResizeBilinearGrad
+          if (rlo && clo) acc[((ylo - ty0) * BWD_TILE + (xlo - tx0)) * BWD_CH + threadIdx.x] += g * wy0 * wx0;
+          if (rlo && chi) acc[((ylo - ty0) * BWD_TILE + (xhi - tx0)) * BWD_CH + threadIdx.x] += g * wy0 * wx1;
+          if (rhi && clo) acc[((yhi - ty0) * BWD_TILE + (xlo - tx0)) * BWD_CH + threadIdx.x] += g * wy1 * wx0;
+          if (rhi && chi) acc[((yhi - ty0) * BWD_TILE + (xhi - tx0)) * BWD_CH + threadIdx.x] += g * wy1 * wx1;
+        }
+      }
+    } else {
+      for (int ph = 0; ph < P; ++ph) {
+        const int ya = k.y1 + (ph * k.h) / P, yb = k.y1 + ((ph + 1) * k.h + P - 1) / P;
+        if (ya >= ty1 || yb <= ty0) continue;
+        for (int pw = 0; pw < P; ++pw) {
+          const int xa = k.x1 + (pw * k.w) / P, xb = k.x1 + ((pw + 1) * k.w + P - 1) / P;
+          if (xa >= tx1 || xb <= tx0) continue;
+          if (!live) continue;
+          const size_t o = (size_t)r * P * P * C + (size_t)(ph * P + pw) * C;
+          const int cell = __ldg(a_img + o);
+          const int ay = cell / W, ax = cell - ay * W;
+          if (ay >= ty0 && ay < ty1 && ax >= tx0 && ax < tx1)
+            acc[((ay - ty0) * BWD_TILE + (ax - tx0)) * BWD_CH + threadIdx.x] += __ldg(g_img + o);
+        }
+      }
+    }
+  }
+  if (!live) return;
+  float* dst = gfeat + (size_t)img * H * W * C + c;
+  for (int y = ty0; y < ty1; ++y)
+    for (int x = tx0; x < tx1; ++x)
+      dst[((size_t)y * W + x) * C] = acc[((y - ty0) * BWD_TILE + (x - tx0)) * BWD_CH + threadIdx.x];
+}
+
+int launch_roi_bwd(frcnn_handle* h, cudaStream_t stream, int mode, const float* gout, const void* rois, int dtype,
+                   const int32_t* argmax, int H, int W, int C, int N, int P, int batch, float* gfeat, int compact) {
+  if (compact) {
+    const bool ok = mode == FRCNN_ROI_MAX && P <= 8 && N < 65536 && roi_compact_supported(H, W, C, P) &&
+                    roi_bwd_blk_eligible(mode, H, W, C, N, P, batch) &&
+                    (reinterpret_cast<uintptr_t>(gout) % 16 == 0) && (reinterpret_cast<uintptr_t>(gfeat) % 16 == 0) &&
+                    (reinterpret_cast<uintptr_t>(argmax) % 4 == 0);
+    if (!ok) return fail(h, FRCNN_ERR_UNSUPPORTED, "roi_bwd: compact arg-max needs max mode, C %% 4 == 0, pool <= 8, fewer than 65536 RoIs, bins of at most 16 x 16 cells and a work list below 2^31 entries%s%s");
+    return launch_roi_bwd_blk(h, stream, mode, gout, rois, dtype, argmax, H, W, C, N, P, batch, gfeat, 1);
+  }
+  const bool aligned = (reinterpret_cast<uintptr_t>(gout) % 16 == 0) && (reinterpret_cast<uintptr_t>(gfeat) % 16 == 0) &&
+                       (mode != FRCNN_ROI_MAX || reinterpret_cast<uintptr_t>(argmax) % 16 == 0);
+  if (aligned && roi_bwd_blk_eligible(mode, H, W, C, N, P, batch))
+    return launch_roi_bwd_blk(h, stream, mode, gout, rois, dtype, argmax, H, W, C, N, P, batch, gfeat, 0);
+  const int tiles_x = (W + BWD_TILE - 1) / BWD_TILE, tiles_y = (H + BWD_TILE - 1) / BWD_TILE;
+  dim3 grid(tiles_x * tiles_y, (C + BWD_CH - 1) / BWD_CH, batch);
+  const size_t smem = (size_t)BWD_TILE * BWD_TILE * BWD_CH * sizeof(float);
+  if (mode == FRCNN_ROI_RESIZE) {
+    FRCNN_CUDA(h, cudaFuncSetAttribute(roi_bwd_scalar_kernel<FRCNN_ROI_RESIZE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    roi_bwd_scalar_kernel<FRCNN_ROI_RESIZE><<<grid, BWD_CH, smem, stream>>>(gout, rois, dtype, argmax, H, W, C, N, P, tiles_x, gfeat);
+  } else {
+    FRCNN_CUDA(h, cudaFuncSetAttribute(roi_bwd_scalar_kernel<FRCNN_ROI_MAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    roi_bwd_scalar_kernel<FRCNN_ROI_MAX><<<grid, BWD_CH, smem, stream>>>(gout, rois, dtype, argmax, H, W, C, N, P, tiles_x, gfeat);
+  }
+  FRCNN_LAUNCH_CHECK(h, "roi_bwd_scalar_kernel");
+  return FRCNN_OK;
 }
 
 }  // namespace frcnn

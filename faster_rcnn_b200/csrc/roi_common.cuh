@@ -4,6 +4,12 @@
 
 namespace frcnn {
 
+// largest pool size of the vectorised kernels: the forward's per-CTA tap table and the backward's 32-bit masks
+constexpr int ROI_MAX_TABLE_P = 32;
+
+// true when the one-byte arg-max format can describe every bin of an H x W map pooled to P x P (roi.cu)
+bool roi_compact_supported(int H, int W, int C, int P);
+
 struct Crop { int x1, y1, w, h; };   // clipped to the map; w,h <= 0 means empty
 
 __device__ __forceinline__ Crop load_crop(const void* rois, int dtype, size_t idx, int W, int H) {

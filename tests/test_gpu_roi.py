@@ -97,15 +97,19 @@ def test_roi_batch_and_pool_sizes(ops):
 
 
 @pytest.mark.parametrize("b,h,w,c,n,pool", [
-    (4, 38, 63, 1024, 24, 7),     # >= 9472 cells: one warp per cell over all 1024 channels, no channel guards
-    (2, 14, 15, 384, 12, 7),      # 3 blocks of 128 channels: two channel chunks per cell, the second one partial
-    (2, 14, 15, 32, 9, 3),        # pool 3: four RoIs per scan pass with unused tap lanes
-    (2, 14, 15, 64, 9, 14),       # pool 14 > 8: one RoI per scan pass
-    (1, 12, 17, 128, 300, 7),     # small launch with >= 256 RoIs: four warps share a cell, each a quarter of the RoIs
-    (1, 9, 11, 1024, 257, 7),     # same with 1024 channels per warp and a ragged last quarter
+    (4, 38, 63, 1024, 24, 7),     # 1024 channels: only full channel slabs (no channel guards), one plan warp per block
+    (2, 14, 15, 384, 12, 7),      # 384 channels: resize mode's second 256-channel slab is partial
+    (2, 14, 15, 32, 9, 3),        # pool 3, one 128-channel slab of which 32 channels exist
+    (2, 14, 15, 64, 9, 14),       # pool 14 > 8: 32-bit masks and RoI records (wide plan)
+    (1, 12, 17, 64, 40, 9),       # pool 9: the smallest pool of the wide plan
+    (1, 38, 63, 128, 64, 32),     # pool 32: every bit of the 32-bit masks
+    (1, 12, 17, 128, 300, 7),     # >= 256 RoIs in a small launch: every block's list sliced across warps
+    (1, 9, 11, 1024, 257, 7),     # same with 1024 channels and a ragged last slice
+    (1, 38, 63, 64, 1100, 14),    # > 1024 RoIs, pool 14: wide plan with 8-warp CTAs per block, sliced lists
 ])
 def test_roi_backward_kernel_variants(ops, b, h, w, c, n, pool):
-    """Every template variant of the cell-stationary backward (channel span, guards, RoIs per scan pass), both modes."""
+    """Variants of the work-list backward, both modes: channel slabs and guards of the streaming kernel, the narrow
+    (pool <= 8) and wide plan, the plan's CTA shapes and the slicing of a block's list across warps."""
     rng = np.random.default_rng(b * h + c + pool)
     feat = rng.standard_normal((b, h, w, c), dtype=np.float32)
     feat[:, ::3, ::2] = feat[0, 0, 0]                              # ties for the max mode
@@ -177,6 +181,35 @@ def test_roi_full_size_properties(ops):
     assert abs(mg.double().sum().item() - gout.double().sum().item()) <= 1e-6 * gout.double().abs().sum().item()
     gathered = torch.gather(feat.reshape(h * w, c), 0, marg.reshape(-1, c).long()).reshape(mout.shape)
     assert torch.equal(gathered, mout)
+
+
+def test_roi_backward_65536_rois_properties(ops):
+    """65536 RoIs of one image (pool 7) take the wide plan, whose queue keeps RoI indices beyond 16 bits.  Too many RoIs
+    for the per-RoI oracle: <dY, fwd(X)> == <bwd(dY), X> in resize mode; in max mode gradient mass conservation and a
+    float64 scatter-add of dY onto the arg-max cells."""
+    import torch
+    h, w, c, n = 12, 17, 16, 65536
+    rng = np.random.default_rng(11)
+    rois = dev(_rois(rng, n, h, w)[None])
+    torch.manual_seed(2)
+    feat = torch.rand((1, h, w, c), device="cuda")              # non-negative: the inner products do not cancel
+    gout = torch.rand((1, n, 7, 7, c), device="cuda")
+    out = ops.roi_forward(feat, rois, 7, "resize")
+    gfeat = ops.roi_backward(gout, rois, (1, h, w, c), "resize")
+    lhs = (out.double() * gout.double()).sum().item()
+    rhs = (gfeat.double() * feat.double()).sum().item()
+    assert abs(lhs - rhs) <= 1e-5 * max(abs(lhs), abs(rhs), 1.0)
+    gout = torch.randn((1, n, 7, 7, c), device="cuda")
+    mout, marg = ops.roi_forward(feat, rois, 7, "max")
+    mg = ops.roi_backward(gout, rois, (1, h, w, c), "max", argmax=marg)
+    assert abs(mg.double().sum().item() - gout.double().sum().item()) <= 1e-6 * gout.double().abs().sum().item()
+    gathered = torch.gather(feat.reshape(h * w, c), 0, marg.reshape(-1, c).long()).reshape(mout.shape)
+    assert torch.equal(gathered, mout)
+    # and every dY element lands on its arg-max cell (float32 sums of ~15000 terms per element against float64 ones)
+    idx, g = marg.reshape(-1, c).long(), gout.reshape(-1, c).double()
+    want = torch.zeros((h * w, c), dtype=torch.float64, device="cuda").scatter_add_(0, idx, g)
+    mass = torch.zeros((h * w, c), dtype=torch.float64, device="cuda").scatter_add_(0, idx, g.abs())
+    assert bool(((mg.reshape(h * w, c).double() - want).abs() <= 1e-6 * mass).all())
 
 
 def test_roi_layer_dropin_and_autograd():
