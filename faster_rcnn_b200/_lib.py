@@ -31,6 +31,10 @@ SIGNATURES = {
     "frcnn_nms_f64": (_i, [_p, _p, _p, _p, _p, _i, _i, _d, _i, _i, _p, _p]),
     "frcnn_proposals": (_i, [_p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _d, _i, _i, _p, _p, _p]),
     "frcnn_label_anchors": (_i, [_p, _p, _p, _p, _p, _i, _i, _i, _i, _p, _i, _i, _p, _p, _p, _p]),
+    "frcnn_decode_topk_ragged": (_i, [_p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _p, _p, _p, _p, _p, _p]),
+    "frcnn_proposals_ragged": (_i, [_p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _d, _i, _i, _p, _p, _p, _p]),
+    "frcnn_label_anchors_ragged": (_i, [_p, _p, _p, _p, _p, _i, _i, _i, _i, _p, _i, _i, _p, _p, _p, _p, _p]),
+    "frcnn_clip_rois": (_i, [_p, _p, _p, _i, _i, _i, _p, _p]),
     "frcnn_pack_rpn_targets": (_i, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _p, _p]),
     "frcnn_label_rois": (_i, [_p, _p, _p, _p, _i, _p, _p, _p, _i, _i, _i, _p, _p, _p, _p, _p]),
     "frcnn_roi_fwd": (_i, [_p, _p, _i, _p, _i, _i, _i, _p, _i, _i, _i, _i, _p, _p]),

@@ -217,4 +217,38 @@ int launch_valid_boxes(frcnn_handle* h, cudaStream_t stream, const float* boxes,
   return FRCNN_OK;
 }
 
+// RoIs of a padded batch clamped to each image's own map: rois [batch][n][4] (int16 / int32 / float32, truncated to int
+// like load_crop, roi_common.cuh), extents [batch][2] (rows, cols).  x1, y1 >= 0 and x2 <= cols_b, y2 <= rows_b; the RoI
+// layer's own clamp to the padded map (load_crop) then completes the clamp of the extents to that map and leaves the
+// crop a call on the image's own map takes, so no kernel reads a padding cell.  out may alias rois.
+template <typename T>
+__global__ void __launch_bounds__(256)
+clip_rois_kernel(const T* rois, int n, const int* __restrict__ extents, T* out) {
+  const int img = blockIdx.y, r = blockIdx.x * 256 + threadIdx.x;
+  if (r >= n) return;
+  const int rows_b = max(extents[2 * img], 0), cols_b = max(extents[2 * img + 1], 0);
+  const size_t o = ((size_t)img * n + r) * 4;
+  const int x1 = (int)rois[o], y1 = (int)rois[o + 1], x2 = (int)rois[o + 2], y2 = (int)rois[o + 3];
+  out[o] = (T)max(x1, 0);
+  out[o + 1] = (T)max(y1, 0);
+  out[o + 2] = (T)min(x2, cols_b);
+  out[o + 3] = (T)min(y2, rows_b);
+}
+
+int launch_clip_rois(frcnn_handle* h, cudaStream_t stream, const void* rois, int dtype, int n, int batch,
+                     const int32_t* extents, void* out) {
+  dim3 grid((n + 255) / 256, batch);
+  if (dtype == FRCNN_ROI_I16)
+    clip_rois_kernel<short><<<grid, 256, 0, stream>>>(static_cast<const short*>(rois), n, extents,
+                                                     static_cast<short*>(out));
+  else if (dtype == FRCNN_ROI_I32)
+    clip_rois_kernel<int><<<grid, 256, 0, stream>>>(static_cast<const int*>(rois), n, extents,
+                                                   static_cast<int*>(out));
+  else
+    clip_rois_kernel<float><<<grid, 256, 0, stream>>>(static_cast<const float*>(rois), n, extents,
+                                                     static_cast<float*>(out));
+  FRCNN_LAUNCH_CHECK(h, "clip_rois_kernel");
+  return FRCNN_OK;
+}
+
 }  // namespace frcnn

@@ -8,13 +8,13 @@ namespace frcnn {
 
 // launchers (one per kernel family)
 int launch_decode_topk(frcnn_handle*, cudaStream_t, const float*, const float*, const AnchorTable&, int, int, int,
-                       int, int16_t*, float*, int32_t*, int32_t*, float*);
+                       int, int16_t*, float*, int32_t*, int32_t*, float*, const int32_t*);
 int launch_nms_i16(frcnn_handle*, cudaStream_t, const int16_t*, const float*, const int32_t*, int, int, double, int,
                    int32_t*, int32_t*, int16_t*, float*);
 int launch_nms_f64(frcnn_handle*, cudaStream_t, const double*, const float*, const int32_t*, int, int, double, int,
                    int, int32_t*, int32_t*);
 int launch_label_anchors(frcnn_handle*, cudaStream_t, const float*, const int32_t*, const int32_t*, int,
-                         const AnchorTable&, int, int, int, int, uint8_t*, uint8_t*, float*, int32_t*);
+                         const AnchorTable&, int, int, int, int, uint8_t*, uint8_t*, float*, int32_t*, const int32_t*);
 int launch_pack_rpn(frcnn_handle*, cudaStream_t, uint8_t*, const uint8_t*, const float*, const int32_t*,
                     const int32_t*, const int32_t*, const int32_t*, int, int, int, int, uint8_t*, float*);
 int launch_label_rois(frcnn_handle*, cudaStream_t, const int16_t*, const int32_t*, int, const double*,
@@ -32,6 +32,7 @@ int launch_anchor_grid(frcnn_handle*, cudaStream_t, const AnchorTable&, int, int
 int launch_valid_boxes(frcnn_handle*, cudaStream_t, const float*, int, int32_t*, int32_t*);
 int launch_gather_det_samples(frcnn_handle*, cudaStream_t, const int16_t*, const int32_t*, const float*, const int32_t*,
                               int, int, int, int, int, int16_t*, int32_t*, float*);
+int launch_clip_rois(frcnn_handle*, cudaStream_t, const void*, int, int, int, const int32_t*, void*);
 int launch_pad_rois(frcnn_handle*, cudaStream_t, const int16_t*, const int32_t*, int, int, int, int, int16_t*,
                     int32_t*);
 
@@ -206,11 +207,10 @@ int frcnn_reserve(frcnn_handle* h, size_t bytes) {
 
 long long frcnn_launch_count(frcnn_handle* h) { return h ? h->launches : 0; }
 
-int frcnn_decode_topk(frcnn_handle* h, void* stream, const float* regr, const float* cls,
-                      const int32_t* anchor_hw_host, int rows, int cols, int n_anchors, int stride, int k,
-                      int batch, int16_t* out_boxes, float* out_scores, int32_t* out_index,
-                      int32_t* out_count, float* dense_boxes) {
-  FRCNN_ENTER(h, stream);
+static int decode_topk_entry(frcnn_handle* h, cudaStream_t st, const float* regr, const float* cls,
+                             const int32_t* anchor_hw_host, int rows, int cols, int n_anchors, int stride, int k,
+                             int batch, const int32_t* extents, int16_t* out_boxes, float* out_scores,
+                             int32_t* out_index, int32_t* out_count, float* dense_boxes) {
   FRCNN_REQUIRE(h, regr && cls && out_boxes && out_scores && out_index && out_count, "decode_topk: null pointer");
   FRCNN_REQUIRE(h, rows > 0 && cols > 0 && stride > 0 && k > 0 && batch > 0, "decode_topk: non-positive size");
   FRCNN_REQUIRE(h, rows <= 32767 && cols <= 32767, "decode_topk: map larger than int16 coordinates");
@@ -218,7 +218,27 @@ int frcnn_decode_topk(frcnn_handle* h, void* stream, const float* regr, const fl
   int rc = make_table(h, anchor_hw_host, n_anchors, stride, &tab);
   if (rc) return rc;
   return launch_decode_topk(h, st, regr, cls, tab, rows, cols, k, batch, out_boxes, out_scores, out_index,
-                            out_count, dense_boxes);
+                            out_count, dense_boxes, extents);
+}
+
+int frcnn_decode_topk(frcnn_handle* h, void* stream, const float* regr, const float* cls,
+                      const int32_t* anchor_hw_host, int rows, int cols, int n_anchors, int stride, int k,
+                      int batch, int16_t* out_boxes, float* out_scores, int32_t* out_index,
+                      int32_t* out_count, float* dense_boxes) {
+  FRCNN_ENTER(h, stream);
+  return decode_topk_entry(h, st, regr, cls, anchor_hw_host, rows, cols, n_anchors, stride, k, batch, nullptr,
+                           out_boxes, out_scores, out_index, out_count, dense_boxes);
+}
+
+int frcnn_decode_topk_ragged(frcnn_handle* h, void* stream, const float* regr, const float* cls,
+                             const int32_t* anchor_hw_host, int rows, int cols, int n_anchors, int stride, int k,
+                             int batch, const int32_t* extents, int16_t* out_boxes, float* out_scores,
+                             int32_t* out_index, int32_t* out_count, float* dense_boxes) {
+  FRCNN_ENTER(h, stream);
+  FRCNN_REQUIRE(h, extents, "decode_topk_ragged: null extents");
+  FRCNN_REQUIRE(h, !dense_boxes, "decode_topk_ragged: dense_boxes must be NULL");
+  return decode_topk_entry(h, st, regr, cls, anchor_hw_host, rows, cols, n_anchors, stride, k, batch, extents,
+                           out_boxes, out_scores, out_index, out_count, nullptr);
 }
 
 int frcnn_nms_i16(frcnn_handle* h, void* stream, const int16_t* boxes, const float* scores, const int32_t* n,
@@ -243,11 +263,10 @@ int frcnn_nms_f64(frcnn_handle* h, void* stream, const double* boxes, const floa
                         keep_index, keep_count);
 }
 
-int frcnn_proposals(frcnn_handle* h, void* stream, const float* regr, const float* cls,
-                    const int32_t* anchor_hw_host, int rows, int cols, int n_anchors, int stride, int k,
-                    double thresh, int max_boxes, int batch, int16_t* out_rois, float* out_scores,
-                    int32_t* out_count) {
-  FRCNN_ENTER(h, stream);
+static int proposals_entry(frcnn_handle* h, cudaStream_t st, const float* regr, const float* cls,
+                           const int32_t* anchor_hw_host, int rows, int cols, int n_anchors, int stride, int k,
+                           double thresh, int max_boxes, int batch, const int32_t* extents, int16_t* out_rois,
+                           float* out_scores, int32_t* out_count) {
   FRCNN_REQUIRE(h, regr && cls && out_rois && out_scores && out_count, "proposals: null pointer");
   FRCNN_REQUIRE(h, rows > 0 && cols > 0 && stride > 0 && k > 0 && batch > 0 && max_boxes > 0,
                 "proposals: non-positive size");
@@ -266,16 +285,35 @@ int frcnn_proposals(frcnn_handle* h, void* stream, const float* regr, const floa
   if ((rc = arena_get(h, st, (size_t)batch * 4, &tc))) return rc;
   if ((rc = arena_get(h, st, (size_t)batch * max_boxes * 4, &ki))) return rc;
   rc = launch_decode_topk(h, st, regr, cls, tab, rows, cols, kk, batch, static_cast<int16_t*>(tb),
-                          static_cast<float*>(ts), static_cast<int32_t*>(ti), static_cast<int32_t*>(tc), nullptr);
+                          static_cast<float*>(ts), static_cast<int32_t*>(ti), static_cast<int32_t*>(tc), nullptr, extents);
   if (rc) return rc;
   return launch_nms_i16(h, st, static_cast<int16_t*>(tb), static_cast<float*>(ts), static_cast<int32_t*>(tc), kk,
                         batch, thresh, max_boxes, static_cast<int32_t*>(ki), out_count, out_rois, out_scores);
 }
 
-int frcnn_label_anchors(frcnn_handle* h, void* stream, const float* gt, const int32_t* n_gt, const int32_t* img_wh,
-                        int g_max, int rows, int cols, int n_anchors, const int32_t* anchor_hw_host, int stride,
-                        int batch, uint8_t* can_use, uint8_t* is_pos, float* bbreg, int32_t* counts) {
+int frcnn_proposals(frcnn_handle* h, void* stream, const float* regr, const float* cls,
+                    const int32_t* anchor_hw_host, int rows, int cols, int n_anchors, int stride, int k,
+                    double thresh, int max_boxes, int batch, int16_t* out_rois, float* out_scores,
+                    int32_t* out_count) {
   FRCNN_ENTER(h, stream);
+  return proposals_entry(h, st, regr, cls, anchor_hw_host, rows, cols, n_anchors, stride, k, thresh, max_boxes, batch,
+                         nullptr, out_rois, out_scores, out_count);
+}
+
+int frcnn_proposals_ragged(frcnn_handle* h, void* stream, const float* regr, const float* cls,
+                           const int32_t* anchor_hw_host, int rows, int cols, int n_anchors, int stride, int k,
+                           double thresh, int max_boxes, int batch, const int32_t* extents, int16_t* out_rois,
+                           float* out_scores, int32_t* out_count) {
+  FRCNN_ENTER(h, stream);
+  FRCNN_REQUIRE(h, extents, "proposals_ragged: null extents");
+  return proposals_entry(h, st, regr, cls, anchor_hw_host, rows, cols, n_anchors, stride, k, thresh, max_boxes, batch,
+                         extents, out_rois, out_scores, out_count);
+}
+
+static int label_anchors_entry(frcnn_handle* h, cudaStream_t st, const float* gt, const int32_t* n_gt,
+                               const int32_t* img_wh, int g_max, int rows, int cols, int n_anchors,
+                               const int32_t* anchor_hw_host, int stride, int batch, const int32_t* extents,
+                               uint8_t* can_use, uint8_t* is_pos, float* bbreg, int32_t* counts) {
   FRCNN_REQUIRE(h, gt && n_gt && img_wh && can_use && is_pos && bbreg && counts, "label_anchors: null pointer");
   FRCNN_REQUIRE(h, rows > 0 && cols > 0 && stride > 0 && batch > 0, "label_anchors: non-positive size");
   FRCNN_REQUIRE(h, g_max > 0 && g_max <= FRCNN_MAX_GT, "label_anchors: g_max must be 1..FRCNN_MAX_GT");
@@ -283,7 +321,34 @@ int frcnn_label_anchors(frcnn_handle* h, void* stream, const float* gt, const in
   int rc = make_table(h, anchor_hw_host, n_anchors, 1, &tab);
   if (rc) return rc;
   return launch_label_anchors(h, st, gt, n_gt, img_wh, g_max, tab, rows, cols, stride, batch, can_use, is_pos,
-                              bbreg, counts);
+                              bbreg, counts, extents);
+}
+
+int frcnn_label_anchors(frcnn_handle* h, void* stream, const float* gt, const int32_t* n_gt, const int32_t* img_wh,
+                        int g_max, int rows, int cols, int n_anchors, const int32_t* anchor_hw_host, int stride,
+                        int batch, uint8_t* can_use, uint8_t* is_pos, float* bbreg, int32_t* counts) {
+  FRCNN_ENTER(h, stream);
+  return label_anchors_entry(h, st, gt, n_gt, img_wh, g_max, rows, cols, n_anchors, anchor_hw_host, stride, batch,
+                             nullptr, can_use, is_pos, bbreg, counts);
+}
+
+int frcnn_label_anchors_ragged(frcnn_handle* h, void* stream, const float* gt, const int32_t* n_gt,
+                               const int32_t* img_wh, int g_max, int rows, int cols, int n_anchors,
+                               const int32_t* anchor_hw_host, int stride, int batch, const int32_t* extents,
+                               uint8_t* can_use, uint8_t* is_pos, float* bbreg, int32_t* counts) {
+  FRCNN_ENTER(h, stream);
+  FRCNN_REQUIRE(h, extents, "label_anchors_ragged: null extents");
+  return label_anchors_entry(h, st, gt, n_gt, img_wh, g_max, rows, cols, n_anchors, anchor_hw_host, stride, batch,
+                             extents, can_use, is_pos, bbreg, counts);
+}
+
+int frcnn_clip_rois(frcnn_handle* h, void* stream, const void* rois, int roi_dtype, int n_rois, int batch,
+                    const int32_t* extents, void* out) {
+  FRCNN_ENTER(h, stream);
+  FRCNN_REQUIRE(h, rois && extents && out, "clip_rois: null pointer");
+  FRCNN_REQUIRE(h, roi_dtype >= FRCNN_ROI_I16 && roi_dtype <= FRCNN_ROI_F32, "clip_rois: unknown roi dtype");
+  FRCNN_REQUIRE(h, n_rois > 0 && batch > 0 && batch <= 65535, "clip_rois: bad size");
+  return launch_clip_rois(h, st, rois, roi_dtype, n_rois, batch, extents, out);
 }
 
 int frcnn_pack_rpn_targets(frcnn_handle* h, void* stream, uint8_t* can_use, const uint8_t* is_pos,

@@ -68,13 +68,19 @@ __device__ __forceinline__ float4 rpn_bbreg(int ax1, int ay1, int ax2, int ay2, 
 // bits order like unsigned ints).  Lanes are in anchor-index order (cell row-major inside the patch), which the
 // "lowest anchor index on ties" rule below relies on.
 constexpr int LBL_PATCH_W = 8, LBL_PATCH_H = 4;
-
+//
+// RAGGED: the batch is padded to one rows x cols map and `extents` [batch][2] (rows, cols) gives each image's own map,
+// clamped to the padded one.  Only cells inside it are live; padding cells get can_use = is_pos = 0 and bbreg = 0.  The
+// patches are the same 8 x 4 tiles as in a call on the image's own map, the padded flat index is monotone in the
+// image's own one, so the per-GT arg-max (lowest index on ties) picks the same anchor, and the ranks that
+// pack_rpn_targets counts among usable anchors are unchanged.  `extents` is unused when RAGGED is false.
+template <bool RAGGED>
 __global__ void __launch_bounds__(LBL_THREADS)
 label_anchors_kernel(const float* __restrict__ gt_all, const int* __restrict__ n_gt_all,
                      const int* __restrict__ img_wh, int g_max, AnchorTable tab, int rows, int cols,
                      int stride, int n, unsigned char* __restrict__ can_use,
                      unsigned char* __restrict__ is_pos, float4* __restrict__ bbreg,
-                     unsigned long long* __restrict__ best_gt) {
+                     unsigned long long* __restrict__ best_gt, const int* __restrict__ extents) {
   __shared__ float4 s_gt[FRCNN_MAX_GT];
   __shared__ float s_garea[FRCNN_MAX_GT];
   const int img = blockIdx.y, tid = threadIdx.x, lane = tid & 31;
@@ -93,7 +99,18 @@ label_anchors_kernel(const float* __restrict__ gt_all, const int* __restrict__ n
   if (patch >= patches_x * patches_y) return;                       // whole warp
   const int py = patch / patches_x, px = patch - py * patches_x;
   const int cx = px * LBL_PATCH_W + (lane & (LBL_PATCH_W - 1)), cy = py * LBL_PATCH_H + lane / LBL_PATCH_W;
-  const bool live = cx < cols && cy < rows;
+  int rows_b = rows, cols_b = cols;
+  if (RAGGED) {
+    rows_b = min(max(extents[2 * img], 0), rows);
+    cols_b = min(max(extents[2 * img + 1], 0), cols);
+  }
+  const bool live = cx < cols_b && cy < rows_b;
+  const bool pad_cell = RAGGED && !live && cx < cols && cy < rows;
+  const size_t o_own = (size_t)img * n + (size_t)(cy * cols + cx) * tab.n + a;
+  if (RAGGED && (px * LBL_PATCH_W >= cols_b || py * LBL_PATCH_H >= rows_b)) {     // whole patch outside the image
+    if (pad_cell) { is_pos[o_own] = 0; can_use[o_own] = 0; bbreg[o_own] = make_float4(0.f, 0.f, 0.f, 0.f); }
+    return;
+  }
   // a lane outside the map computes on the patch's first cell (inside by construction) and stores nothing
   const int ccx = live ? cx : px * LBL_PATCH_W, ccy = live ? cy : py * LBL_PATCH_H;
   const int i = (ccy * cols + ccx) * tab.n + a;
@@ -133,7 +150,10 @@ label_anchors_kernel(const float* __restrict__ gt_all, const int* __restrict__ n
       }
     }
   }
-  if (!live) return;
+  if (!live) {
+    if (pad_cell) { is_pos[o_own] = 0; can_use[o_own] = 0; bbreg[o_own] = make_float4(0.f, 0.f, 0.f, 0.f); }
+    return;
+  }
 
   const int W = img_wh[2 * img], H = img_wh[2 * img + 1];
   const bool oob = (x1 < 0) || (y1 < 0) || (x2 >= W) || (y2 >= H);
@@ -418,7 +438,7 @@ label_rois_kernel(const BoxI16* __restrict__ rois_all, const int* __restrict__ n
 int launch_label_anchors(frcnn_handle* h, cudaStream_t stream, const float* gt, const int32_t* n_gt,
                          const int32_t* img_wh, int g_max, const AnchorTable& tab, int rows, int cols,
                          int stride, int batch, uint8_t* can_use, uint8_t* is_pos, float* bbreg,
-                         int32_t* counts) {
+                         int32_t* counts, const int32_t* extents) {
   const int n = rows * cols * tab.n;
   void* ws = nullptr;
   const size_t best_bytes = (size_t)batch * g_max * sizeof(unsigned long long);
@@ -429,8 +449,9 @@ int launch_label_anchors(frcnn_handle* h, cudaStream_t stream, const float* gt, 
   FRCNN_CUDA(h, cudaMemsetAsync(counts, 0, (size_t)batch * 2 * sizeof(int), stream));
   const int patches = ((cols + LBL_PATCH_W - 1) / LBL_PATCH_W) * ((rows + LBL_PATCH_H - 1) / LBL_PATCH_H);
   dim3 grid((patches * tab.n + LBL_THREADS / 32 - 1) / (LBL_THREADS / 32), batch);
-  label_anchors_kernel<<<grid, LBL_THREADS, 0, stream>>>(gt, n_gt, img_wh, g_max, tab, rows, cols, stride, n,
-                                                        can_use, is_pos, reinterpret_cast<float4*>(bbreg), best);
+  auto kernel = extents ? label_anchors_kernel<true> : label_anchors_kernel<false>;
+  kernel<<<grid, LBL_THREADS, 0, stream>>>(gt, n_gt, img_wh, g_max, tab, rows, cols, stride, n, can_use, is_pos,
+                                           reinterpret_cast<float4*>(bbreg), best, extents);
   FRCNN_LAUNCH_CHECK(h, "label_anchors_kernel");
   dim3 g2((g_max + 63) / 64, batch);
   label_gt_fixup_kernel<<<g2, 64, 0, stream>>>(gt, n_gt, img_wh, g_max, tab, cols, stride, n, best, can_use,

@@ -268,9 +268,14 @@ __device__ __forceinline__ unsigned bucket_last(int d) {
   return d >= TOPK_BINS - 1 ? 0xffffffffu : ((unsigned)(d + FINE_BASE + 1) << (FINE_SHIFT - 32)) - 1u;
 }
 
-template <int THREADS, int E>
+// RAGGED: the images of the batch are padded to one (rows, cols) map and `extents` [batch][2] (rows, cols) gives each
+// image's own map, clamped to the padded one.  Cells outside it are "no box" without a load of regr / cls, boxes are
+// sanitized against the image's own map, and out_index is the image's own flat index (y * cols_b + x) * A + a.  The
+// sort position stays the padded index, which is monotone in the image's own one, so ties resolve as in a call on the
+// cropped map.  `extents` is unused when RAGGED is false.
+template <int THREADS, int E, bool RAGGED>
 __global__ void __launch_bounds__(THREADS, THREADS == 1024 ? 1 : 4)
-proposals_kernel(const ProposalArgs p, const AnchorTable tab) {
+proposals_kernel(const ProposalArgs p, const AnchorTable tab, const int* __restrict__ extents) {
   constexpr int M = SORT_T * E;                      // sort size (power of two), >= slice length
   extern __shared__ __align__(16) unsigned long long sbuf[];      // M + SORT_T sort entries, then the candidate buffer
   __shared__ unsigned hist_own[TOPK_BINS];           // this CTA's share of the bucket histogram; later the select passes'
@@ -286,6 +291,11 @@ proposals_kernel(const ProposalArgs p, const AnchorTable tab) {
   BoxI16* boxes = p.boxes + (size_t)img * n;
   cg::cluster_group cluster = cg::this_cluster();
   int phase = 0;
+  int rows_b = p.rows, cols_b = p.cols;
+  if (RAGGED) {
+    rows_b = min(max(extents[2 * img], 0), p.rows);
+    cols_b = min(max(extents[2 * img + 1], 0), p.cols);
+  }
 
   for (int i = tid; i < TOPK_BINS; i += THREADS) hist_own[i] = 0u;
   if (tid < tab.n)
@@ -297,9 +307,14 @@ proposals_kernel(const ProposalArgs p, const AnchorTable tab) {
   {
     const int chunk = (p.n_pad + splits - 1) / splits;
     const int lo = part * chunk, hi = min(p.n_pad, lo + chunk);
-    const float colmax = (float)(p.cols - 1), rowmax = (float)(p.rows - 1);
+    const float colmax = (float)(cols_b - 1), rowmax = (float)(rows_b - 1);
     for (int i = lo + tid; i < hi; i += THREADS) {
       if (i >= n) { skeys[i] = 0u; continue; }       // padding of the last 128-bit group
+      if (RAGGED) {                                  // a cell outside the image: no box, its inputs are never read
+        const unsigned loc = fast_div((unsigned)i, p.div_a);
+        const unsigned cy = fast_div(loc, p.div_cols);
+        if ((int)cy >= rows_b || (int)loc - (int)cy * p.cols >= cols_b) { skeys[i] = 0u; continue; }
+      }
       const size_t g = (size_t)img * n + i;
       const float4 r = ldg_f4(p.regr + 4 * g);
       const float score = __ldg(p.cls + g);
@@ -625,7 +640,14 @@ proposals_kernel(const ProposalArgs p, const AnchorTable tab) {
       const uint2 bw = __ldcg(reinterpret_cast<const uint2*>(boxes + idx));   // written by a peer CTA: L2, not the read-only path
       reinterpret_cast<uint2*>(p.out_boxes)[o] = bw;
       p.out_scores[o] = __ldg(cls + idx);
-      p.out_index[o] = idx;
+      if (RAGGED) {                                  // the image's own flat anchor index
+        const unsigned loc = fast_div((unsigned)idx, p.div_a);
+        const unsigned cy = fast_div(loc, p.div_cols);
+        const int cx = (int)loc - (int)cy * p.cols;
+        p.out_index[o] = ((int)cy * cols_b + cx) * tab.n + (idx - (int)loc * tab.n);
+      } else {
+        p.out_index[o] = idx;
+      }
     } else {
       p.out_boxes[o] = BoxI16{0, 0, 0, 0};
       p.out_scores[o] = 0.0f;
@@ -638,11 +660,11 @@ proposals_kernel(const ProposalArgs p, const AnchorTable tab) {
 
 // probe_only: configure the kernel for this (cluster size, shared memory) once per handle and report whether a cluster
 // of that size can be resident at all; the answer is cached in the handle, so a steady-state call is one launch.
-template <int THREADS, int E>
+template <int THREADS, int E, bool RAGGED>
 static int launch_proposals(frcnn_handle* h, cudaStream_t stream, const ProposalArgs& args, const AnchorTable& tab,
-                            int batch, bool probe_only) {
+                            const int* extents, int batch, bool probe_only) {
   const size_t smem = (size_t)(SORT_T * E + SORT_T + args.w_cap) * sizeof(unsigned long long);
-  auto kernel = proposals_kernel<THREADS, E>;
+  auto kernel = proposals_kernel<THREADS, E, RAGGED>;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)(batch * args.splits));
   cfg.blockDim = dim3(THREADS);
@@ -657,7 +679,8 @@ static int launch_proposals(frcnn_handle* h, cudaStream_t stream, const Proposal
   cfg.numAttrs = 1;
   if (probe_only) {
     constexpr int LOG_E = E == 1 ? 0 : E == 2 ? 1 : E == 4 ? 2 : 3;
-    unsigned char& state = h->proposals_cfg[THREADS == 1024 ? 1 : 0][LOG_E][args.splits];
+    // cudaFuncSetAttribute is per kernel function: every instance has its own entry
+    unsigned char& state = h->proposals_cfg[RAGGED ? 1 : 0][THREADS == 1024 ? 1 : 0][LOG_E][args.splits];
     if (state == 0) {
       FRCNN_CUDA(h, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       if (args.splits > 8) FRCNN_CUDA(h, cudaFuncSetAttribute(kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
@@ -668,26 +691,34 @@ static int launch_proposals(frcnn_handle* h, cudaStream_t stream, const Proposal
     }
     return state == 1 ? FRCNN_OK : FRCNN_ERR_UNSUPPORTED;
   }
-  FRCNN_CUDA(h, cudaLaunchKernelEx(&cfg, kernel, args, tab));
+  FRCNN_CUDA(h, cudaLaunchKernelEx(&cfg, kernel, args, tab, extents));
   FRCNN_LAUNCH_CHECK(h, "proposals_kernel");
   return FRCNN_OK;
 }
 
-template <int THREADS>
+template <int THREADS, bool RAGGED>
 static int launch_proposals_e(frcnn_handle* h, cudaStream_t stream, const ProposalArgs& args, const AnchorTable& tab,
-                              int batch, int e, bool probe_only) {
+                              const int* extents, int batch, int e, bool probe_only) {
   switch (e) {
-    case 1: return launch_proposals<THREADS, 1>(h, stream, args, tab, batch, probe_only);
-    case 2: return launch_proposals<THREADS, 2>(h, stream, args, tab, batch, probe_only);
-    case 4: return launch_proposals<THREADS, 4>(h, stream, args, tab, batch, probe_only);
-    default: return launch_proposals<THREADS, 8>(h, stream, args, tab, batch, probe_only);
+    case 1: return launch_proposals<THREADS, 1, RAGGED>(h, stream, args, tab, extents, batch, probe_only);
+    case 2: return launch_proposals<THREADS, 2, RAGGED>(h, stream, args, tab, extents, batch, probe_only);
+    case 4: return launch_proposals<THREADS, 4, RAGGED>(h, stream, args, tab, extents, batch, probe_only);
+    default: return launch_proposals<THREADS, 8, RAGGED>(h, stream, args, tab, extents, batch, probe_only);
   }
+}
+
+template <bool RAGGED>
+static int launch_proposals_cfg(frcnn_handle* h, cudaStream_t stream, const ProposalArgs& args, const AnchorTable& tab,
+                                const int* extents, int batch, int e, bool wide, bool probe_only) {
+  return wide ? launch_proposals_e<1024, RAGGED>(h, stream, args, tab, extents, batch, e, probe_only)
+              : launch_proposals_e<256, RAGGED>(h, stream, args, tab, extents, batch, e, probe_only);
 }
 
 int launch_decode_topk(frcnn_handle* h, cudaStream_t stream, const float* regr, const float* cls,
                        const AnchorTable& tab, int rows, int cols, int k, int batch,
                        int16_t* out_boxes, float* out_scores, int32_t* out_index,
-                       int32_t* out_count, float* dense_boxes) {
+                       int32_t* out_count, float* dense_boxes, const int32_t* extents) {
+  if (extents && dense_boxes) return fail(h, FRCNN_ERR_INVALID, "decode_topk: dense_boxes is not available with extents%s%s");
   const long long n_ll = (long long)rows * cols * tab.n;
   if (n_ll >= (1ll << 31)) return fail(h, FRCNN_ERR_UNSUPPORTED, "decode_topk: more than 2^31 anchors per image%s%s");
   const int n = (int)n_ll;
@@ -745,11 +776,9 @@ int launch_decode_topk(frcnn_handle* h, cudaStream_t stream, const float* regr, 
       const bool w = attempt == 0 ? wide : false;
       if (attempt == 1 && !wide) break;
       args.w_cap = w ? 6144 : (e == 8 ? 3072 : 2560);   // >= M + SORT_T: the candidate buffer doubles as the sort's second exchange buffer
-      const int ok = w ? launch_proposals_e<1024>(h, stream, args, tab, batch, e, true)
-                       : launch_proposals_e<256>(h, stream, args, tab, batch, e, true);
-      if (ok == FRCNN_OK)
-        return w ? launch_proposals_e<1024>(h, stream, args, tab, batch, e, false)
-                 : launch_proposals_e<256>(h, stream, args, tab, batch, e, false);
+      auto run = extents ? launch_proposals_cfg<true> : launch_proposals_cfg<false>;
+      if (run(h, stream, args, tab, extents, batch, e, w, true) == FRCNN_OK)
+        return run(h, stream, args, tab, extents, batch, e, w, false);
     }
     if (splits == 1) return fail(h, FRCNN_ERR_UNSUPPORTED, "decode_topk: no cluster configuration fits this device%s%s");
   }

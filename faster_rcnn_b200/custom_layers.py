@@ -43,9 +43,14 @@ class _RoiFunction(torch.autograd.Function):
         return grad_feat, None, None, None
 
 
-def roi_pool(feat, rois, pool_size, mode="resize"):
+def roi_pool(feat, rois, pool_size, mode="resize", extents=None):
     """feat (B,H,W,C) f32 CUDA tensor, rois (B,N,4) int16/int32/float32 CUDA tensor (feature cells,
-    x2/y2 excluded from the crop) -> (B,N,P,P,C) f32, differentiable w.r.t. feat."""
+    x2/y2 excluded from the crop) -> (B,N,P,P,C) f32, differentiable w.r.t. feat.
+    `extents` (B,2) i32 (rows, cols) on the device: feat is a padded batch of differently sized maps (ops.pad_batch);
+    the RoIs are clamped to each image's own map first, so every image pools as on its own map and the gradient of the
+    padding is zero."""
+    if extents is not None:
+        rois = ops.clip_rois(rois, extents)
     return _RoiFunction.apply(feat, rois, int(pool_size), mode)
 
 

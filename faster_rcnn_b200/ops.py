@@ -33,9 +33,19 @@ def _chk_out(t, dtype, name, ndim):
     return _chk(t, dtype, name, ndim)
 
 
-def decode_topk(regr, cls, anchor_dims, stride, k, want_dense=False):
+def _chk_extents(extents, b):
+    """extents (B,2) i32 (rows, cols) per image of a padded batch, a CUDA tensor: the call stays asynchronous."""
+    extents = _chk(extents, torch.int32, "extents", 2)
+    if extents.shape != (b, 2):
+        raise ValueError("extents must be (B, 2) = (%d, 2), got %s" % (b, tuple(extents.shape)))
+    return extents
+
+
+def decode_topk(regr, cls, anchor_dims, stride, k, want_dense=False, extents=None):
     """K-a.  regr (B,R,C,4A) f32, cls (B,R,C,A) f32 -> boxes (B,k,4) i16, scores (B,k) f32,
-    index (B,k) i32, count (B,) i32 [, dense (B,R*C*A,4) f32].  det_util.py:63-76,145-155,370-380."""
+    index (B,k) i32, count (B,) i32 [, dense (B,R*C*A,4) f32].  det_util.py:63-76,145-155,370-380.
+    `extents` (B,2) i32 (rows, cols) on the device: a padded batch of differently sized maps, see `pad_batch`; each
+    image's result is that of the call on its own map, `index` counts in that map, no dense boxes."""
     regr, cls = _chk(regr, torch.float32, "regr", 4), _chk(cls, torch.float32, "cls", 4)
     ctx = get_context(regr.device)
     b, rows, cols, a = cls.shape
@@ -44,9 +54,17 @@ def decode_topk(regr, cls, anchor_dims, stride, k, want_dense=False):
     anc, n_anc = ctx.anchors(anchor_dims)
     if n_anc != a:
         raise ValueError("cls has %d anchors per cell, anchor_dims has %d" % (a, n_anc))
+    if extents is not None:
+        if want_dense:
+            raise ValueError("dense boxes are not available for a padded batch (extents given)")
+        extents = _chk_extents(extents, b)
     k = int(min(k, rows * cols * a))
     boxes, scores = ctx.empty((b, k, 4), torch.int16), ctx.empty((b, k), torch.float32)
     index, count = ctx.empty((b, k), torch.int32), ctx.empty((b,), torch.int32)
+    if extents is not None:
+        ctx.call("frcnn_decode_topk_ragged", ptr(regr), ptr(cls), anc, rows, cols, a, int(stride), k, b, ptr(extents),
+                 ptr(boxes), ptr(scores), ptr(index), ptr(count), None)
+        return boxes, scores, index, count
     dense = ctx.empty((b, rows * cols * a, 4), torch.float32) if want_dense else None
     ctx.call("frcnn_decode_topk", ptr(regr), ptr(cls), anc, rows, cols, a, int(stride), k, b, ptr(boxes),
              ptr(scores), ptr(index), ptr(count), ptr(dense))
@@ -84,10 +102,12 @@ def nms_f64(boxes, scores, seg_offsets, max_seg_len, overlap_thresh=0.5, max_box
     return ki, kc
 
 
-def proposals(regr, cls, anchor_dims, stride, k, overlap_thresh=0.7, max_boxes=300, out=None):
+def proposals(regr, cls, anchor_dims, stride, k, overlap_thresh=0.7, max_boxes=300, out=None, extents=None):
     """K-a -> K-b fused on the device.  Returns rois (B,max_boxes,4) i16, scores (B,max_boxes) f32,
     count (B,) i32 (written into `out` = (rois, scores, count) when given).
-    det_util.py:63-77 (k=12000, 2000) / :136-158 (k=8000, 300)."""
+    det_util.py:63-77 (k=12000, 2000) / :136-158 (k=8000, 300).
+    `extents` (B,2) i32 (rows, cols) on the device: a padded batch of differently sized maps (see `pad_batch`); each
+    image's proposals are those of the call on its own map."""
     regr, cls = _chk(regr, torch.float32, "regr", 4), _chk(cls, torch.float32, "cls", 4)
     ctx = get_context(regr.device)
     b, rows, cols, a = cls.shape
@@ -105,14 +125,20 @@ def proposals(regr, cls, anchor_dims, stride, k, overlap_thresh=0.7, max_boxes=3
     else:
         rois, scores = ctx.empty((b, max_boxes, 4), torch.int16), ctx.empty((b, max_boxes), torch.float32)
         count = ctx.empty((b,), torch.int32)
+    if extents is not None:
+        ctx.call("frcnn_proposals_ragged", ptr(regr), ptr(cls), anc, rows, cols, a, int(stride), int(k),
+                 float(overlap_thresh), max_boxes, b, ptr(_chk_extents(extents, b)), ptr(rois), ptr(scores), ptr(count))
+        return rois, scores, count
     ctx.call("frcnn_proposals", ptr(regr), ptr(cls), anc, rows, cols, a, int(stride), int(k), float(overlap_thresh),
              max_boxes, b, ptr(rois), ptr(scores), ptr(count))
     return rois, scores, count
 
 
-def label_anchors(gt, n_gt, img_wh, rows, cols, anchor_dims, stride):
+def label_anchors(gt, n_gt, img_wh, rows, cols, anchor_dims, stride, extents=None):
     """K-c.  gt (B,Gmax,4) f32 pixel corners, n_gt (B,) i32, img_wh (B,2) i32 (width,height) ->
-    can_use (B,N) u8, is_pos (B,N) u8, bbreg (B,N,4) f32, counts (B,2) i32.  rpn_util.py:54-103."""
+    can_use (B,N) u8, is_pos (B,N) u8, bbreg (B,N,4) f32, counts (B,2) i32.  rpn_util.py:54-103.
+    `extents` (B,2) i32 (rows_b, cols_b) on the device: images of different conv shapes padded to rows x cols; each
+    image's labels are those of the call on its own map, laid into the padded (R,C,A) layout, padding cells zero."""
     gt, n_gt = _chk(gt, torch.float32, "gt", 3), _chk(n_gt, torch.int32, "n_gt", 1)
     img_wh = _chk(img_wh, torch.int32, "img_wh", 2)
     ctx = get_context(gt.device)
@@ -121,6 +147,10 @@ def label_anchors(gt, n_gt, img_wh, rows, cols, anchor_dims, stride):
     n = rows * cols * a
     can_use, is_pos = ctx.empty((b, n), torch.uint8), ctx.empty((b, n), torch.uint8)
     bbreg, counts = ctx.empty((b, n, 4), torch.float32), ctx.empty((b, 2), torch.int32)
+    if extents is not None:
+        ctx.call("frcnn_label_anchors_ragged", ptr(gt), ptr(n_gt), ptr(img_wh), g_max, int(rows), int(cols), a, anc,
+                 int(stride), b, ptr(_chk_extents(extents, b)), ptr(can_use), ptr(is_pos), ptr(bbreg), ptr(counts))
+        return can_use, is_pos, bbreg, counts
     ctx.call("frcnn_label_anchors", ptr(gt), ptr(n_gt), ptr(img_wh), g_max, int(rows), int(cols), a, anc, int(stride),
              b, ptr(can_use), ptr(is_pos), ptr(bbreg), ptr(counts))
     return can_use, is_pos, bbreg, counts
@@ -171,6 +201,52 @@ def label_rois(rois, gt, gt_cls, n_gt, n_classes, n_roi=None):
     ctx.call("frcnn_label_rois", ptr(rois), ptr(n_roi), n_max, ptr(gt), ptr(gt_cls), ptr(n_gt), g_max, k, b,
              ptr(out_rois), ptr(out_cls), ptr(out_bbreg), ptr(src), ptr(count))
     return out_rois, out_cls, out_bbreg, src, count
+
+
+def clip_rois(rois, extents):
+    """rois (B,N,4) i16/i32/f32 of a padded batch -> a new tensor of the same dtype, truncated to int like the RoI layer
+    and clamped to each image's own map (x1, y1 >= 0, x2 <= cols_b, y2 <= rows_b; extents (B,2) i32 on the device).  The
+    RoI layer on the padded features then takes the crops of the call on the image's own map and reads no padding."""
+    if rois.dtype not in _ROI_DTYPES:
+        raise TypeError("rois must be int16, int32 or float32")
+    rois = _chk(rois, rois.dtype, "rois", 3)
+    extents = _chk_extents(extents, rois.shape[0])
+    ctx = get_context(rois.device)
+    out = ctx.empty(tuple(rois.shape), rois.dtype)
+    ctx.call("frcnn_clip_rois", ptr(rois), _ROI_DTYPES[rois.dtype], rois.shape[1], rois.shape[0], ptr(extents), ptr(out))
+    return out
+
+
+def pad_batch(arrays, pad_to=None):
+    """A list of per-image (R_b, C_b, X) arrays (numpy or torch, one dtype) -> (padded (B,R,C,X), extents (B,2) i32), both
+    CUDA tensors.  (R, C) = the largest extents, or `pad_to` (which must hold every image).  Only each image's valid
+    region is copied; the padding is zero, and the ragged entry points never read it."""
+    if not isinstance(arrays, (list, tuple)) or len(arrays) == 0:
+        raise ValueError("pad_batch needs a non-empty list of (R_b, C_b, X) arrays")
+    shapes = [tuple(x.shape) for x in arrays]
+    if any(len(s) != 3 for s in shapes):
+        raise ValueError("every array must have 3 dimensions (R_b, C_b, X), got %s" % (shapes,))
+    if len({s[2] for s in shapes}) != 1:
+        raise ValueError("arrays disagree in their last dimension: %s" % (shapes,))
+    dtypes = {str(x.dtype).replace("torch.", "") for x in arrays}
+    if len(dtypes) != 1:
+        raise ValueError("arrays must share one dtype, got %s" % sorted(dtypes))
+    rows, cols = max(s[0] for s in shapes), max(s[1] for s in shapes)
+    if pad_to is not None:
+        pr, pc = (int(v) for v in pad_to)
+        if pr < rows or pc < cols:
+            raise ValueError("pad_to %s is smaller than the largest extents (%d, %d)" % ((pr, pc), rows, cols))
+        rows, cols = pr, pc
+    if rows <= 0 or cols <= 0:
+        raise ValueError("the padded map is empty")
+    first = arrays[0] if isinstance(arrays[0], torch.Tensor) else torch.from_numpy(np.ascontiguousarray(arrays[0]))
+    ctx = get_context(first.device if first.is_cuda else None)
+    padded = torch.zeros((len(arrays), rows, cols, shapes[0][2]), dtype=first.dtype, device=ctx.device)
+    for b, x in enumerate(arrays):
+        t = x if isinstance(x, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(x))
+        padded[b, :t.shape[0], :t.shape[1]].copy_(t, non_blocking=t.is_cuda)
+    extents = ctx.to_device(np.array([s[:2] for s in shapes], np.int32).reshape(-1, 2))
+    return padded, extents
 
 
 def roi_compact_supported(height, width, channels, pool):

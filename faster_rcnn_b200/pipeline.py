@@ -41,22 +41,27 @@ class ProposalRoiPipeline:
         return pin
 
     # -- the call a user makes ----------------------------------------------------------------------
-    def run_device(self, cls, regr, feat):
+    def run_device(self, cls, regr, feat, extents=None):
         """CUDA tensors in, CUDA tensors out; nothing synchronises.
         cls (B,R,C,A), regr (B,R,C,4A), feat (B,R,C,Cf) ->
         rois (B,max_boxes,4) i16, scores (B,max_boxes) f32, count (B,) i32,
-        padded_rois (B,M,4) i16, pooled (B,M,P,P,Cf) f32 [, argmax in max mode]."""
+        padded_rois (B,M,4) i16, pooled (B,M,P,P,Cf) f32 [, argmax in max mode].
+        `extents` (B,2) i32 (rows, cols) on the device: a padded batch of differently sized maps (ops.pad_batch).  The
+        proposals are sanitized against each image's own map, so the RoI layer reads no padding and every image's result
+        equals the call on its own map."""
         rois, scores, count = ops.proposals(regr, cls, self.anchor_dims, self.stride, self.k, self.thresh,
-                                            self.max_boxes)
+                                            self.max_boxes, extents=extents)
         padded, _ = ops.pad_rois(rois, count, self.num_rois)
         pooled = ops.roi_forward(feat, padded, self.pool_size, self.mode)
         return rois, scores, count, padded, pooled
 
-    def capture(self, cls, regr, feat):
+    def capture(self, cls, regr, feat, extents=None):
         """CUDA-graph capture of `run_device` for fixed shapes (SURVEY 8f-1): returns a `GraphedRun` whose call copies
         new inputs into the captured buffers and replays decode -> top-k -> NMS -> pad -> RoI layer as ONE graph
-        launch (5 kernels, no per-kernel Python/ctypes/launch overhead -- what matters at batch 1)."""
-        return GraphedRun(self, cls, regr, feat)
+        launch (5 kernels, no per-kernel Python/ctypes/launch overhead -- what matters at batch 1).  Captured with
+        `extents`, the extents are an input of the graph too: one graph serves every mix of sizes up to the padded
+        shape."""
+        return GraphedRun(self, cls, regr, feat, extents)
 
     def __call__(self, cls, regr, feat, on_device=None):
         """Host (or device) arrays in; returns (rois, scores, count) as numpy on the host -- what
@@ -68,8 +73,12 @@ class ProposalRoiPipeline:
         Host inputs are uploaded in chunks of `h2d_chunk` images on a copy stream while the kernels of
         the previous chunk run (images are independent, so chunking does not change any result); one
         stream synchronisation at the end.  `feat` may already be a CUDA tensor while cls / regr are host arrays (a GPU
-        backbone next to a host-side RPN head): it is then used in place and only the small head outputs are uploaded."""
-        host_in = not (isinstance(cls, torch.Tensor) and cls.is_cuda)
+        backbone next to a host-side RPN head): it is then used in place and only the small head outputs are uploaded.
+
+        A list of per-image host arrays cls (R_b,C_b,A), regr (R_b,C_b,4A) and feat (R_b,C_b,Cf) is a batch of differently
+        sized images: only each image's valid region is uploaded into the padded device buffers, and the batch runs as one
+        padded batch with extents (a CUDA tensor `feat` must then already be the padded (B,R,C,Cf) batch)."""
+        host_in = isinstance(cls, (list, tuple)) or not (isinstance(cls, torch.Tensor) and cls.is_cuda)
         if not host_in:
             rois, scores, count, padded, pooled = self.run_device(cls, regr, feat)
         else:
@@ -101,14 +110,45 @@ class ProposalRoiPipeline:
             buf = self._dev[name] = torch.empty(shape, dtype=dtype, device=self.ctx.device)
         return buf
 
+    def _pinned_ragged(self, name, arrays):
+        """per-image host arrays -> views of one pinned staging buffer, each image's valid region back to back"""
+        ts = [torch.from_numpy(np.ascontiguousarray(x, dtype=np.float32)) if not isinstance(x, torch.Tensor)
+              else x.to(torch.float32).contiguous() for x in arrays]
+        total = sum(t.numel() for t in ts)
+        pin = self._host.get(name)
+        if pin is None or pin.dim() != 1 or pin.numel() < total:
+            pin = self._host[name] = torch.empty(max(total, 1), dtype=torch.float32).pin_memory()
+        views, off = [], 0
+        for t in ts:
+            v = pin[off:off + t.numel()].view(t.shape)
+            v.copy_(t)
+            views.append(v)
+            off += t.numel()
+        return views
+
     def _run_chunked(self, cls, regr, feat):
         dev = self.ctx.device
         feat_on_device = isinstance(feat, torch.Tensor) and feat.is_cuda     # a GPU backbone hands its features over as is
-        srcs = {"cls": self._pinned("cls", cls), "regr": self._pinned("regr", regr)}
-        if not feat_on_device:
-            srcs["feat"] = self._pinned("feat", feat)
-        b = srcs["cls"].shape[0]
-        bufs = {k: self._device_buffer(k, v.shape, torch.float32) for k, v in srcs.items()}
+        extents = None
+        if isinstance(cls, (list, tuple)):                                   # differently sized images
+            if len(regr) != len(cls) or (not feat_on_device and len(feat) != len(cls)):
+                raise ValueError("cls, regr and feat must list the same images")
+            ext = np.array([tuple(x.shape[:2]) for x in cls], np.int32).reshape(-1, 2)
+            rows, cols = (int(v) for v in ext.max(axis=0))
+            if feat_on_device:
+                rows, cols = feat.shape[1], feat.shape[2]
+            srcs = {"cls": self._pinned_ragged("cls", cls), "regr": self._pinned_ragged("regr", regr)}
+            if not feat_on_device:
+                srcs["feat"] = self._pinned_ragged("feat", feat)
+            b = len(cls)
+            bufs = {k: self._device_buffer(k, (b, rows, cols, v[0].shape[2]), torch.float32) for k, v in srcs.items()}
+            extents = self.ctx.to_device(ext)
+        else:
+            srcs = {"cls": self._pinned("cls", cls), "regr": self._pinned("regr", regr)}
+            if not feat_on_device:
+                srcs["feat"] = self._pinned("feat", feat)
+            b = srcs["cls"].shape[0]
+            bufs = {k: self._device_buffer(k, v.shape, torch.float32) for k, v in srcs.items()}
         if feat_on_device:
             bufs["feat"] = feat if feat.dtype == torch.float32 and feat.is_contiguous() else feat.float().contiguous()
         m = -(-self.max_boxes // self.num_rois) * self.num_rois
@@ -117,7 +157,7 @@ class ProposalRoiPipeline:
         count = self._device_buffer("o_count", (b,), torch.int32)
         padded = self._device_buffer("o_padded", (b, m, 4), torch.int16)
         rows = self._device_buffer("o_rows", (b,), torch.int32)
-        pooled = torch.empty((b, m, self.pool_size, self.pool_size, feat.shape[3]), dtype=torch.float32, device=dev)
+        pooled = torch.empty((b, m, self.pool_size, self.pool_size, bufs["feat"].shape[3]), dtype=torch.float32, device=dev)
         argmax = torch.empty(pooled.shape, dtype=torch.int32, device=dev) if self.mode == "max" else None
         if self._copy_stream is None:
             self._copy_stream = torch.cuda.Stream(device=dev)
@@ -132,14 +172,20 @@ class ProposalRoiPipeline:
             for lo in range(0, b, step):
                 hi = min(b, lo + step)
                 for k in srcs:
-                    bufs[k][lo:hi].copy_(srcs[k][lo:hi], non_blocking=True)
+                    if extents is None:
+                        bufs[k][lo:hi].copy_(srcs[k][lo:hi], non_blocking=True)
+                    else:                                 # the valid region only; the padding is never read
+                        for i in range(lo, hi):
+                            r, c = srcs[k][i].shape[:2]
+                            bufs[k][i, :r, :c].copy_(srcs[k][i], non_blocking=True)
                 ev = torch.cuda.Event()
                 ev.record(self._copy_stream)
                 events.append((lo, hi, ev))
         for lo, hi, ev in events:
             cur.wait_event(ev)
             ops.proposals(bufs["regr"][lo:hi], bufs["cls"][lo:hi], self.anchor_dims, self.stride, self.k, self.thresh,
-                          self.max_boxes, out=(rois[lo:hi], scores[lo:hi], count[lo:hi]))
+                          self.max_boxes, out=(rois[lo:hi], scores[lo:hi], count[lo:hi]),
+                          extents=None if extents is None else extents[lo:hi])
             ops.pad_rois(rois[lo:hi], count[lo:hi], self.num_rois, out=(padded[lo:hi], rows[lo:hi]))
             ops.roi_forward(bufs["feat"][lo:hi], padded[lo:hi], self.pool_size, self.mode, out=pooled[lo:hi],
                             argmax_out=None if argmax is None else argmax[lo:hi])
@@ -160,10 +206,11 @@ class GraphedRun:
     is sized by two eager warm-up runs and can never be moved by other calls, so the device pointers baked into the
     graph stay valid.  Outputs are the captured tensors (overwritten by every replay)."""
 
-    def __init__(self, pipe, cls, regr, feat):
+    def __init__(self, pipe, cls, regr, feat, extents=None):
         from .runtime import Context, use_context
         dev = pipe.ctx.device
-        self.inputs = tuple(torch.empty_like(t, device=dev).copy_(t) for t in (cls, regr, feat))
+        self.inputs = tuple(torch.empty_like(t, device=dev).copy_(t) for t in (cls, regr, feat) +
+                            (() if extents is None else (extents,)))
         self._ctx = Context(dev.index)
         side = torch.cuda.Stream(device=dev)
         side.wait_stream(torch.cuda.current_stream(dev))
@@ -176,13 +223,28 @@ class GraphedRun:
                 self.outputs = pipe.run_device(*self.inputs)
         torch.cuda.current_stream(dev).wait_stream(side)
 
-    def __call__(self, cls=None, regr=None, feat=None):
-        """Replays the graph (after copying any given CUDA tensor into the captured input of the same shape)."""
-        for dst, src in zip(self.inputs, (cls, regr, feat)):
+    def __call__(self, cls=None, regr=None, feat=None, extents=None):
+        """Replays the graph (after copying any given CUDA tensor into the captured input of the same shape).  New
+        `extents` need a graph captured with extents."""
+        if extents is not None and len(self.inputs) < 4:
+            raise ValueError("this graph was captured without extents")
+        for dst, src in zip(self.inputs, (cls, regr, feat, extents)):
             if src is not None and src.data_ptr() != dst.data_ptr():
                 dst.copy_(src, non_blocking=True)
         self.graph.replay()
         return self.outputs
+
+
+def _padded_inputs(cls, regr, feat, extents):
+    """lists of per-image arrays -> padded batches + extents (ops.pad_batch); anything else passes through"""
+    if not isinstance(cls, (list, tuple)):
+        if extents is not None and not isinstance(extents, torch.Tensor):
+            extents = get_context().to_device(np.asarray(extents, np.int32).reshape(-1, 2))
+        return cls, regr, feat, extents
+    cls, extents = ops.pad_batch(cls)
+    regr, _ = ops.pad_batch(regr, pad_to=cls.shape[1:3])
+    feat = feat if isinstance(feat, torch.Tensor) and feat.is_cuda else ops.pad_batch(feat, pad_to=cls.shape[1:3])[0]
+    return cls.float(), regr.float(), feat.float(), extents
 
 
 class DetectionPipeline(ProposalRoiPipeline):
@@ -202,9 +264,11 @@ class DetectionPipeline(ProposalRoiPipeline):
         self.class_mapping = class_mapping
         self.det_threshold, self.det_nms_thresh, self.det_max_boxes = det_threshold, det_nms_thresh, det_max_boxes
 
-    def detect_device(self, cls, regr, feat, resize_ratios, gather=False):
-        """CUDA tensors in -> (det_boxes (B,M,4) i32, det_probs (B,M) f32, det_cls (B,M) i32, det_count (B,) i32)."""
-        rois, scores, count = ops.proposals(regr, cls, self.anchor_dims, self.stride, self.k, self.thresh, self.max_boxes)
+    def detect_device(self, cls, regr, feat, resize_ratios, gather=False, extents=None):
+        """CUDA tensors in -> (det_boxes (B,M,4) i32, det_probs (B,M) f32, det_cls (B,M) i32, det_count (B,) i32).
+        `extents` (B,2) i32 on the device: a padded batch of differently sized maps, as in `run_device`."""
+        rois, scores, count = ops.proposals(regr, cls, self.anchor_dims, self.stride, self.k, self.thresh, self.max_boxes,
+                                            extents=extents)
         padded, rows = ops.pad_rois(rois, count, self.num_rois)
         pooled = ops.roi_forward(feat, padded, self.pool_size, self.mode)
         out_cls, out_reg = self.detector_head(pooled if self.mode == "resize" else pooled[0], padded)
@@ -218,10 +282,13 @@ class DetectionPipeline(ProposalRoiPipeline):
             return parallel.all_gather_detections(packed, counts)
         return dets
 
-    def detect(self, cls, regr, feat, resize_ratios):
-        """Host or device arrays in -> per image the reference's list of {'bbox', 'cls_name', 'prob'} dicts."""
+    def detect(self, cls, regr, feat, resize_ratios, extents=None):
+        """Host or device arrays in -> per image the reference's list of {'bbox', 'cls_name', 'prob'} dicts.  Lists of
+        per-image (R_b,C_b,X) arrays are a batch of differently sized images (padded with ops.pad_batch)."""
+        cls, regr, feat, extents = _padded_inputs(cls, regr, feat, extents)
         dev_in = [x if (isinstance(x, torch.Tensor) and x.is_cuda) else self.ctx.to_device(x, np.float32) for x in (cls, regr, feat)]
-        boxes, probs, dcls, count = (self.ctx.to_host(t) for t in self.detect_device(*dev_in, resize_ratios))
+        boxes, probs, dcls, count = (self.ctx.to_host(t) for t in self.detect_device(*dev_in, resize_ratios,
+                                                                                   extents=extents))
         names = {v: k for k, v in self.class_mapping.items()}
         return [[{'bbox': boxes[b, i].astype(np.int64), 'cls_name': names[int(dcls[b, i])], 'prob': probs[b, i]}
                  for i in range(int(count[b]))] for b in range(len(count))]
@@ -268,11 +335,11 @@ class DetTrainingPipeline:
         n_gt = np.array([len(g) for g, _ in per], np.int32)
         return self.ctx.to_device(gt), self.ctx.to_device(gt_cls), self.ctx.to_device(n_gt)
 
-    def targets(self, cls, regr, gt, gt_cls, n_gt, chunk=32):
+    def targets(self, cls, regr, gt, gt_cls, n_gt, chunk=32, extents=None):
         """CUDA tensors in -> (rois (B,S,4) i16, y_class_num (B,S,K) i32, y_transform (B,S,8(K-1)) f32) on the device and
         has_rois (B,) bool on the host.  The batch is enqueued in chunks of `chunk` images; the host draws the
         mini-batches of chunk i (in image order, so the RNG stream is the per-image one) while the GPU is still
-        labelling chunks i+1.."""
+        labelling chunks i+1..  `extents` (B,2) i32 on the device: a padded batch of differently sized maps."""
         from .det_util import _get_det_samples
         b, dev = cls.shape[0], self.ctx.device
         stream = torch.cuda.current_stream(dev)
@@ -280,7 +347,7 @@ class DetTrainingPipeline:
         for lo in range(0, b, chunk):
             hi = min(b, lo + chunk)
             rois, _, count = ops.proposals(regr[lo:hi], cls[lo:hi], self.anchor_dims, self.stride, self.k, self.thresh,
-                                           self.max_boxes)
+                                           self.max_boxes, extents=None if extents is None else extents[lo:hi])
             l_rois, y_cls, y_tr, _, m = ops.label_rois(rois, gt[lo:hi], gt_cls[lo:hi], n_gt[lo:hi],
                                                        len(self.class_mapping), n_roi=count)
             found_d = (y_cls[:, :, -1] == 0).to(torch.uint8)                      # positives = not background
@@ -306,10 +373,13 @@ class DetTrainingPipeline:
         rois, y_cls, y_tr = (torch.cat([o[j] for o in outs]) for j in range(3))
         return rois, y_cls, y_tr, np.concatenate(has)
 
-    def __call__(self, cls, regr, feat, images):
+    def __call__(self, cls, regr, feat, images, extents=None):
         """Host or device arrays + the images' ground truth -> (rois, y_class_num, y_transform, pooled, has_rois):
-        the detector's training inputs and the RoI layer's output on the sampled RoIs (CUDA tensors)."""
+        the detector's training inputs and the RoI layer's output on the sampled RoIs (CUDA tensors).  Lists of
+        per-image (R_b,C_b,X) arrays, or padded arrays with `extents`, are a batch of differently sized images; the
+        sampled RoIs lie inside each image's own map, so the RoI layer reads no padding."""
+        cls, regr, feat, extents = _padded_inputs(cls, regr, feat, extents)
         dev_in = [x if (isinstance(x, torch.Tensor) and x.is_cuda) else self.ctx.to_device(x, np.float32) for x in (cls, regr, feat)]
-        rois, y_cls, y_tr, has = self.targets(dev_in[0], dev_in[1], *self.ground_truth(images))
+        rois, y_cls, y_tr, has = self.targets(dev_in[0], dev_in[1], *self.ground_truth(images), extents=extents)
         pooled = ops.roi_forward(dev_in[2], rois, self.pool_size, self.mode)
         return rois, y_cls, y_tr, pooled, has

@@ -38,11 +38,13 @@ class RpnTrainingManager:
         return np.expand_dims(self.preprocess_func(image.data), axis=0)
 
     # -- device side ----------------------------------------------------------------------------
-    def _label_batch(self, images):
+    def _label_batch(self, images, extents=None, pad_to=None):
         """Labels a list of images that share one conv shape in a single launch sequence.
-        Returns device tensors can_use (B,N) u8, is_pos (B,N) u8, bbreg (B,N,4) f32, counts (B,2)."""
+        Returns device tensors can_use (B,N) u8, is_pos (B,N) u8, bbreg (B,N,4) f32, counts (B,2).
+        With `extents` ((B,2) host array of the images' conv shapes) the images may differ: they are labelled as one
+        batch padded to `pad_to` (rows, cols)."""
         ctx = get_context()
-        rows, cols = self.calc_conv_dims(images[0].height, images[0].width)
+        rows, cols = pad_to if extents is not None else self.calc_conv_dims(images[0].height, images[0].width)
         g_max = max(len(img.gt_boxes) for img in images)
         if g_max == 0:
             raise ValueError("image without ground-truth boxes (the reference fails in np.amax here too)")
@@ -50,7 +52,7 @@ class RpnTrainingManager:
         n_gt = np.zeros(len(images), dtype=np.int32)
         wh = np.zeros((len(images), 2), dtype=np.int32)
         for b, img in enumerate(images):
-            if tuple(self.calc_conv_dims(img.height, img.width)) != (rows, cols):
+            if extents is None and tuple(self.calc_conv_dims(img.height, img.width)) != (rows, cols):
                 raise ValueError("images of one batch must share the conv feature-map shape")
             if len(img.gt_boxes) == 0:
                 raise ValueError("image without ground-truth boxes (the reference fails in np.amax here too)")
@@ -58,7 +60,8 @@ class RpnTrainingManager:
             gt[b, :n_gt[b]] = get_bbox_coords(img.gt_boxes)
             wh[b] = img.width, img.height
         return ops.label_anchors(ctx.to_device(gt), ctx.to_device(n_gt), ctx.to_device(wh), rows, cols,
-                                 self.anchor_dims, self.stride)
+                                 self.anchor_dims, self.stride,
+                                 extents=None if extents is None else ctx.to_device(extents))
 
     @profile
     def _process(self, image):
@@ -101,6 +104,23 @@ class RpnTrainingManager:
         can_use, is_pos, bbreg, counts = self._label_batch(images)
         y_class, y_bbreg = self._sample_and_pack(can_use, is_pos, bbreg, counts, rows, cols, len(self.anchor_dims))
         return ctx.to_host(y_class).view(np.bool_), ctx.to_host(y_bbreg)
+
+    def rpn_y_true_ragged(self, images, pad_to=None):
+        """Batched variant for images of different conv shapes (not in the reference): list of images ->
+        y_class (B,R,C,2A) bool, y_bbreg (B,R,C,8A) f32, extents (B,2) i32 (each image's conv rows, cols).  (R, C) are the
+        largest conv shape of the batch or `pad_to`.  Image b's targets are y_class[b, :rows_b, :cols_b] (and the same of
+        y_bbreg); the padding is zero, i.e. unusable anchors.  RNG draws happen image by image in list order, so the result
+        equals calling `rpn_y_true` on each image in turn."""
+        ctx = get_context()
+        extents = np.array([tuple(self.calc_conv_dims(img.height, img.width)) for img in images], np.int32).reshape(-1, 2)
+        rows, cols = (int(v) for v in extents.max(axis=0))
+        if pad_to is not None:
+            if pad_to[0] < rows or pad_to[1] < cols:
+                raise ValueError("pad_to %s is smaller than the largest conv shape (%d, %d)" % (tuple(pad_to), rows, cols))
+            rows, cols = int(pad_to[0]), int(pad_to[1])
+        can_use, is_pos, bbreg, counts = self._label_batch(images, extents, (rows, cols))
+        y_class, y_bbreg = self._sample_and_pack(can_use, is_pos, bbreg, counts, rows, cols, len(self.anchor_dims))
+        return ctx.to_host(y_class).view(np.bool_), ctx.to_host(y_bbreg), extents
 
     def _sample_and_pack(self, can_use, is_pos, bbreg, counts, rows, cols, n_anchors):
         ctx = get_context()

@@ -141,6 +141,41 @@ FRCNN_API int frcnn_proposals(frcnn_handle* h, void* stream, const float* regr, 
                     int k, double thresh, int max_boxes, int batch, int16_t* out_rois,
                     float* out_scores, int32_t* out_count);
 
+/* ---- mixed-size batches (the *_ragged entries and frcnn_clip_rois)
+ * Images whose feature maps differ in size share one PADDED layout: rows x cols are the largest
+ * extents of the batch (or any larger map) and extents [batch,2] i32 (device) holds every image's own
+ * (rows_b, cols_b), clamped on the device to [0,rows] x [0,cols].  For every image the result equals the
+ * uniform call on the cropped inputs [:rows_b, :cols_b], laid out in the padded layout: padding cells of
+ * every output are zero and padding cells of the inputs are never read.  An image with a zero extent
+ * gets no proposals and all-zero labels.
+ *   decode_topk_ragged: out_index is the image's OWN flat index (y*cols_b + x)*A + a; dense_boxes must
+ *   be NULL (FRCNN_ERR_INVALID otherwise).
+ *   label_anchors_ragged: can_use / is_pos / bbreg in the padded [batch,rows*cols*A] layout, counts as
+ *   frcnn_label_anchors; frcnn_pack_rpn_targets takes the result unchanged (the ranks of the usable
+ *   anchors are those of the cropped call).
+ *   clip_rois: rois [batch,n_rois,4] (roi_dtype) -> out (same layout, may alias rois), truncated to int
+ *   like the RoI layer and clamped to x1,y1 >= 0, x2 <= cols_b, y2 <= rows_b (extents below 0 count
+ *   as 0); the RoI layer entries then take the padded feature map [batch,rows,cols,C], whose own clamp
+ *   completes the clamp of the extents, and see the cropped call's crops.  Max mode's int32 arg-max
+ *   y*W + x then refers to the PADDED width W. */
+FRCNN_API int frcnn_decode_topk_ragged(frcnn_handle* h, void* stream, const float* regr, const float* cls,
+                                       const int32_t* anchor_hw_host, int rows, int cols, int n_anchors,
+                                       int stride, int k, int batch, const int32_t* extents,
+                                       int16_t* out_boxes, float* out_scores, int32_t* out_index,
+                                       int32_t* out_count, float* dense_boxes);
+FRCNN_API int frcnn_proposals_ragged(frcnn_handle* h, void* stream, const float* regr, const float* cls,
+                                     const int32_t* anchor_hw_host, int rows, int cols, int n_anchors,
+                                     int stride, int k, double thresh, int max_boxes, int batch,
+                                     const int32_t* extents, int16_t* out_rois, float* out_scores,
+                                     int32_t* out_count);
+FRCNN_API int frcnn_label_anchors_ragged(frcnn_handle* h, void* stream, const float* gt, const int32_t* n_gt,
+                                         const int32_t* img_wh, int g_max, int rows, int cols,
+                                         int n_anchors, const int32_t* anchor_hw_host, int stride,
+                                         int batch, const int32_t* extents, uint8_t* can_use,
+                                         uint8_t* is_pos, float* bbreg, int32_t* counts);
+FRCNN_API int frcnn_clip_rois(frcnn_handle* h, void* stream, const void* rois, int roi_dtype, int n_rois,
+                              int batch, const int32_t* extents, void* out);
+
 /* ---- K-c: RPN anchor labelling
  * Replaces RpnTrainingManager._process (rpn_util.py:54-103) incl.
  * _get_all_anchor_coords (:276-298), _get_out_of_bounds_idxs (:302-310),
