@@ -50,10 +50,12 @@ SIGNATURES = {
     "frcnn_pad_rois": (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _p, _p]),
     "frcnn_gather_det_samples": (_i, [_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _p, _p, _p]),
     "frcnn_rpn_losses": (_i, [_p, _p, _p, _p, _p, _p, _p, _i, _i, _p, _p, _p]),
+    "frcnn_rpn_losses_ragged": (_i, [_p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _p, _p, _p, _p]),
     "frcnn_det_losses": (_i, [_p, _p, _p, _p, _p, _p, _i, _i, _i, _p, _p, _p]),
     "frcnn_voc_match": (_i, [_p, _p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _d, _p, _p]),
     "frcnn_voc_pr_ap": (_i, [_p, _p, _p, _p, _i, _d, _p, _i, _p, _p, _p]),
     "frcnn_image_resize_cubic": (_i, [_p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p, _p, _p]),
+    "frcnn_image_resize_cubic_ragged": (_i, [_p, _p, _p, _p, _ll, _p, _p, _i, _i, _i, _i, _p, _p, _p]),
     "frcnn_gt_transform": (_i, [_p, _p, _p, _p, _i, _i, _p, _p, _p]),
 }
 

@@ -38,6 +38,8 @@ int launch_pad_rois(frcnn_handle*, cudaStream_t, const int16_t*, const int32_t*,
 
 int launch_rpn_losses(frcnn_handle*, cudaStream_t, const uint8_t*, const uint8_t*, const float*, const float*,
                       const float*, int, int, float*, float*, float*);
+int launch_rpn_losses_ragged(frcnn_handle*, cudaStream_t, const uint8_t*, const uint8_t*, const float*, const float*,
+                             const float*, int, int, int, int, const int32_t*, float*, float*, float*);
 int launch_det_losses(frcnn_handle*, cudaStream_t, const int32_t*, const float*, const float*, const float*, int, int,
                       int, float*, float*, float*);
 
@@ -48,6 +50,8 @@ int launch_voc_pr_ap(frcnn_handle*, cudaStream_t, const double*, const double*, 
 
 int launch_image_resize(frcnn_handle*, cudaStream_t, const uint8_t*, int, int, int, int, int, int, int, const double*,
                         uint8_t*, float*);
+int launch_image_resize_ragged(frcnn_handle*, cudaStream_t, const uint8_t*, const int64_t*, long long, const int32_t*,
+                               const uint8_t*, int, int, int, int, const double*, uint8_t*, float*);
 int launch_gt_transform(frcnn_handle*, cudaStream_t, const double*, const int32_t*, int, int, const double*, const double*,
                         double*);
 
@@ -518,6 +522,20 @@ int frcnn_rpn_losses(frcnn_handle* h, void* stream, const uint8_t* can_use, cons
   return launch_rpn_losses(h, st, can_use, is_pos, bbreg, cls_pred, reg_pred, n_per_image, batch, loss, grad_cls, grad_reg);
 }
 
+int frcnn_rpn_losses_ragged(frcnn_handle* h, void* stream, const uint8_t* can_use, const uint8_t* is_pos,
+                            const float* bbreg, const float* cls_pred, const float* reg_pred, int rows, int cols,
+                            int n_anchors, int batch, const int32_t* extents, float* loss, float* grad_cls,
+                            float* grad_reg) {
+  FRCNN_ENTER(h, stream);
+  FRCNN_REQUIRE(h, can_use && is_pos && bbreg && cls_pred && reg_pred && extents && loss, "rpn_losses_ragged: null pointer");
+  FRCNN_REQUIRE(h, rows > 0 && cols > 0 && n_anchors > 0 && batch > 0 && batch <= 65535, "rpn_losses_ragged: bad size");
+  FRCNN_REQUIRE(h, (long long)rows * cols * n_anchors < (1LL << 31), "rpn_losses_ragged: map too large");
+  FRCNN_REQUIRE(h, ((reinterpret_cast<uintptr_t>(bbreg) | reinterpret_cast<uintptr_t>(reg_pred) |
+                     reinterpret_cast<uintptr_t>(grad_reg)) & 15) == 0, "rpn_losses_ragged: box arrays must be 16-byte aligned");
+  return launch_rpn_losses_ragged(h, st, can_use, is_pos, bbreg, cls_pred, reg_pred, rows, cols, n_anchors, batch, extents,
+                                  loss, grad_cls, grad_reg);
+}
+
 int frcnn_det_losses(frcnn_handle* h, void* stream, const int32_t* y_class, const float* y_transform,
                      const float* cls_pred, const float* reg_pred, int m_rows, int n_classes, int batch, float* loss,
                      float* grad_cls, float* grad_reg) {
@@ -565,6 +583,21 @@ int frcnn_image_resize_cubic(frcnn_handle* h, void* stream, const uint8_t* src, 
                 "image_resize_cubic: image too large");
   return launch_image_resize(h, st, src, src_height, src_width, channels, dst_height, dst_width, flip, batch, mean_host,
                              out_u8, out_f32);
+}
+
+int frcnn_image_resize_cubic_ragged(frcnn_handle* h, void* stream, const uint8_t* src, const int64_t* src_offsets,
+                                    long long src_bytes, const int32_t* geom, const uint8_t* flip, int channels,
+                                    int dst_height, int dst_width, int batch, const double* mean_host, uint8_t* out_u8,
+                                    float* out_f32) {
+  FRCNN_ENTER(h, stream);
+  FRCNN_REQUIRE(h, src && src_offsets && geom && (out_u8 || out_f32), "image_resize_cubic_ragged: null pointer");
+  FRCNN_REQUIRE(h, src_bytes >= 0 && dst_height > 0 && dst_width > 0 && batch > 0 && batch <= 65535,
+                "image_resize_cubic_ragged: bad size");
+  FRCNN_REQUIRE(h, channels >= 1 && channels <= 4, "image_resize_cubic_ragged: 1..4 channels");
+  FRCNN_REQUIRE(h, (dst_height + 31) / 32 <= 65535 && (long long)dst_width + dst_height < (1LL << 31),
+                "image_resize_cubic_ragged: image too large");
+  return launch_image_resize_ragged(h, st, src, src_offsets, src_bytes, geom, flip, channels, dst_height, dst_width, batch,
+                                    mean_host, out_u8, out_f32);
 }
 
 int frcnn_gt_transform(frcnn_handle* h, void* stream, const double* boxes, const int32_t* n_box, int n_max, int batch,

@@ -14,13 +14,8 @@ namespace frcnn {
 // one record per output column / row: first tap (unclamped) and the four x2048 coefficients
 struct CubicTap { int s; short c[4]; int pad; };
 
-__global__ void __launch_bounds__(256)
-cubic_table_kernel(int src_w, int dst_w, int src_h, int dst_h, CubicTap* __restrict__ xt, CubicTap* __restrict__ yt) {
-  const int i = blockIdx.x * 256 + threadIdx.x;
-  if (i >= dst_w + dst_h) return;
-  const bool is_x = i < dst_w;
-  const int d = is_x ? i : i - dst_w;
-  const int src = is_x ? src_w : src_h, dst = is_x ? dst_w : dst_h;
+// output position d of an axis resized from src to dst
+__device__ __forceinline__ CubicTap cubic_tap(int src, int dst, int d) {
   const double scale = __ddiv_rn(1.0, __ddiv_rn((double)dst, (double)src));
   float f = (float)__dsub_rn(__dmul_rn(__dadd_rn((double)d, 0.5), scale), 0.5);
   const int s = (int)floorf(f);
@@ -36,7 +31,16 @@ cubic_table_kernel(int src_w, int dst_w, int src_h, int dst_h, CubicTap* __restr
   t.pad = 0;
 #pragma unroll
   for (int k = 0; k < 4; ++k) t.c[k] = (short)max(-32768, min(32767, __float2int_rn(__fmul_rn(c[k], 2048.0f))));
-  (is_x ? xt : yt)[d] = t;
+  return t;
+}
+
+__global__ void __launch_bounds__(256)
+cubic_table_kernel(int src_w, int dst_w, int src_h, int dst_h, CubicTap* __restrict__ xt, CubicTap* __restrict__ yt) {
+  const int i = blockIdx.x * 256 + threadIdx.x;
+  if (i >= dst_w + dst_h) return;
+  const bool is_x = i < dst_w;
+  const int d = is_x ? i : i - dst_w;
+  (is_x ? xt : yt)[d] = cubic_tap(is_x ? src_w : src_h, is_x ? dst_w : dst_h, d);
 }
 
 // one thread per output pixel (all channels); out_u8 and / or out_f32 (pixel - mean[c], float64 subtraction stored as
@@ -140,6 +144,126 @@ __global__ void mean_lut_kernel(float* __restrict__ lut, double m0, double m1, d
   lut[768 + v] = (float)__dsub_rn((double)v, m3);
 }
 
+// ---- ragged batch: differently sized sources, each resized to its own size inside one padded output ----------------
+// Every geometry lives on the device, so the launch configuration depends on the padded shape only and one captured
+// graph serves every mix of sizes.  Per image: tap tables at a fixed stride of dst_width + dst_height entries, then one
+// CTA per 32 x 32 output tile of the padded image.  A tile outside the image's extent writes zeros.  A tile whose 32
+// rows span at most 72 source rows (scale <= 2.1, as the uniform launcher's tall tiles) takes the shared-memory
+// horizontal pass; any other computes each pixel straight from the source, the per-pixel kernel's integer sums, which
+// give the same values.  The mirror works within the image's own width.
+struct RaggedImage { long long off; int src_h, src_w, dst_h, dst_w; };
+
+// geom[img] = (src_h, src_w, dst_h, dst_w); the output extent is clamped to the padded image, and a source with a
+// non-positive size or bytes outside [0, src_bytes) gets an empty extent (an all-zero image, nothing read)
+__device__ __forceinline__ RaggedImage ragged_image(const long long* offsets, long long src_bytes, const int* geom, int cn,
+                                                    int dst_height, int dst_width, int img) {
+  RaggedImage r;
+  r.src_h = geom[4 * img];
+  r.src_w = geom[4 * img + 1];
+  r.dst_h = min(max(geom[4 * img + 2], 0), dst_height);
+  r.dst_w = min(max(geom[4 * img + 3], 0), dst_width);
+  r.off = offsets[img];
+  const long long px = (long long)max(r.src_h, 0) * max(r.src_w, 0);
+  if (px == 0 || px > src_bytes || r.off < 0 || r.off > src_bytes || px * cn > src_bytes - r.off) r.dst_h = r.dst_w = 0;
+  return r;
+}
+
+__global__ void __launch_bounds__(256)
+cubic_table_ragged_kernel(const long long* __restrict__ offsets, long long src_bytes, const int* __restrict__ geom, int cn,
+                          int dst_height, int dst_width, CubicTap* __restrict__ tab) {
+  const int i = blockIdx.x * 256 + threadIdx.x, img = blockIdx.y;
+  const RaggedImage r = ragged_image(offsets, src_bytes, geom, cn, dst_height, dst_width, img);
+  CubicTap* xt = tab + (size_t)img * (dst_width + dst_height);
+  if (i < r.dst_w) xt[i] = cubic_tap(r.src_w, r.dst_w, i);
+  else if (i >= dst_width && i - dst_width < r.dst_h) xt[i] = cubic_tap(r.src_h, r.dst_h, i - dst_width);
+}
+
+template <int CN>
+__global__ void __launch_bounds__(256, CN == 4 ? 5 : 6)   // as many CTAs per SM as the shared memory (up to 30 KB, 40 KB at CN 4) allows
+resize_cubic_ragged_kernel(const unsigned char* __restrict__ src, const long long* __restrict__ offsets, long long src_bytes,
+                           const int* __restrict__ geom, const unsigned char* __restrict__ flip, int dst_height, int dst_width,
+                           const CubicTap* __restrict__ tab, const float* __restrict__ lut, unsigned char* __restrict__ out_u8,
+                           float* __restrict__ out_f32) {
+  constexpr int TILE_H = 32, TILE_ROWS = 72;
+  __shared__ int hs[TILE_ROWS][TILE_W * CN];
+  __shared__ float s_lut[CN][256];
+  const int dx0 = blockIdx.x * TILE_W, dy0 = blockIdx.y * TILE_H, img = blockIdx.z;
+  const int tid = threadIdx.x, x = tid & 31, wy = tid >> 5;
+  const int px = dx0 + x, y_end = min(dy0 + TILE_H, dst_height);
+  const RaggedImage r = ragged_image(offsets, src_bytes, geom, CN, dst_height, dst_width, img);
+  const size_t img_base = (size_t)img * dst_height * dst_width * CN;
+  // rows [dy0, y_valid) of column px lie inside the image; the rest of the tile is padding
+  const int y_valid = px < r.dst_w ? min(y_end, r.dst_h) : dy0;
+  if (dx0 < r.dst_w && dy0 < r.dst_h) {
+    for (int i = tid; i < CN * 256; i += 256) s_lut[i >> 8][i & 255] = lut[i];
+    const unsigned char* s_img = src + r.off;
+    const CubicTap* xt = tab + (size_t)img * (dst_width + dst_height);
+    const CubicTap* yt = xt + dst_width;
+    // source-side column of output column px; columns past the extent repeat an edge column and are never stored
+    const int dx = (flip && flip[img]) ? max(r.dst_w - 1 - px, 0) : min(px, r.dst_w - 1);
+    const CubicTap tx = xt[dx];
+    int xo[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) xo[k] = min(max(tx.s + k, 0), r.src_w - 1) * CN;
+    const int r0 = yt[dy0].s;
+    const int n_rows = yt[min(dy0 + TILE_H, r.dst_h) - 1].s + 4 - r0;
+    if (n_rows <= TILE_ROWS) {                                      // the same for the whole CTA
+      for (int row = wy; row < n_rows; row += 8) {
+        const unsigned char* rp = s_img + (size_t)min(max(r0 + row, 0), r.src_h - 1) * r.src_w * CN;
+#pragma unroll
+        for (int c = 0; c < CN; ++c)
+          hs[row][c * TILE_W + x] = (int)rp[xo[0] + c] * tx.c[0] + (int)rp[xo[1] + c] * tx.c[1] +
+                                    (int)rp[xo[2] + c] * tx.c[2] + (int)rp[xo[3] + c] * tx.c[3];
+      }
+      __syncthreads();
+#pragma unroll 1
+      for (int dy = dy0 + wy; dy < y_valid; dy += 8) {
+        const CubicTap ty = yt[dy];
+        const int rr = ty.s - r0;
+        const size_t o = img_base + ((size_t)dy * dst_width + px) * CN;
+#pragma unroll
+        for (int c = 0; c < CN; ++c) {
+          const int acc = hs[rr][c * TILE_W + x] * ty.c[0] + hs[rr + 1][c * TILE_W + x] * ty.c[1] +
+                          hs[rr + 2][c * TILE_W + x] * ty.c[2] + hs[rr + 3][c * TILE_W + x] * ty.c[3];
+          const int v = min(255, max(0, (acc + (1 << 21)) >> 22));
+          if (out_u8) out_u8[o + c] = (unsigned char)v;
+          if (out_f32) out_f32[o + c] = s_lut[c][v];
+        }
+      }
+    } else {
+      __syncthreads();
+#pragma unroll 1
+      for (int dy = dy0 + wy; dy < y_valid; dy += 8) {
+        const CubicTap ty = yt[dy];
+        const size_t o = img_base + ((size_t)dy * dst_width + px) * CN;
+#pragma unroll
+        for (int c = 0; c < CN; ++c) {
+          int acc = 0;
+#pragma unroll
+          for (int j = 0; j < 4; ++j) {
+            const unsigned char* rp = s_img + (size_t)min(max(ty.s + j, 0), r.src_h - 1) * r.src_w * CN + c;
+            acc += ((int)rp[xo[0]] * tx.c[0] + (int)rp[xo[1]] * tx.c[1] + (int)rp[xo[2]] * tx.c[2] +
+                    (int)rp[xo[3]] * tx.c[3]) * ty.c[j];
+          }
+          const int v = min(255, max(0, (acc + (1 << 21)) >> 22));
+          if (out_u8) out_u8[o + c] = (unsigned char)v;
+          if (out_f32) out_f32[o + c] = s_lut[c][v];
+        }
+      }
+    }
+  }
+  if (px >= dst_width) return;
+  for (int dy = dy0 + wy; dy < y_end; dy += 8) {
+    if (dy < y_valid) continue;
+    const size_t o = img_base + ((size_t)dy * dst_width + px) * CN;
+#pragma unroll
+    for (int c = 0; c < CN; ++c) {
+      if (out_u8) out_u8[o + c] = 0;
+      if (out_f32) out_f32[o + c] = 0.0f;
+    }
+  }
+}
+
 // boxes [n,4] f64 -> corners * ratio, then mirrored about flip_width when flip_width >= 0 (per image: ratio[b], width[b])
 __global__ void gt_transform_kernel(const double* __restrict__ boxes, const int* __restrict__ n_box, int n_max,
                                     const double* __restrict__ ratio, const double* __restrict__ flip_width,
@@ -196,6 +320,37 @@ int launch_image_resize(frcnn_handle* h, cudaStream_t stream, const uint8_t* src
   resize_cubic_kernel<<<grid, 256, 0, stream>>>(src, src_h, src_w, cn, dst_h, dst_w, xt, yt, flip, out_u8, out_f32, m[0], m[1],
                                                 m[2], m[3]);
   FRCNN_LAUNCH_CHECK(h, "resize_cubic_kernel");
+  return FRCNN_OK;
+}
+
+int launch_image_resize_ragged(frcnn_handle* h, cudaStream_t stream, const uint8_t* src, const int64_t* src_offsets,
+                               long long src_bytes, const int32_t* geom, const uint8_t* flip, int cn, int dst_height,
+                               int dst_width, int batch, const double* mean_host, uint8_t* out_u8, float* out_f32) {
+  void *tab = nullptr, *lut = nullptr;
+  int rc = arena_get(h, stream, (size_t)batch * (dst_width + dst_height) * sizeof(CubicTap), &tab);
+  if (rc || (rc = arena_get(h, stream, 4 * 256 * sizeof(float), &lut))) return rc;
+  CubicTap* tabc = static_cast<CubicTap*>(tab);
+  float* lutf = static_cast<float*>(lut);
+  const long long* offs = reinterpret_cast<const long long*>(src_offsets);
+  cubic_table_ragged_kernel<<<dim3((dst_width + dst_height + 255) / 256, batch), 256, 0, stream>>>(
+      offs, src_bytes, geom, cn, dst_height, dst_width, tabc);
+  FRCNN_LAUNCH_CHECK(h, "cubic_table_ragged_kernel");
+  double m[4] = {0.0, 0.0, 0.0, 0.0};
+  if (mean_host)
+    for (int c = 0; c < cn && c < 4; ++c) m[c] = mean_host[c];
+  mean_lut_kernel<<<1, 256, 0, stream>>>(lutf, m[0], m[1], m[2], m[3]);
+  FRCNN_LAUNCH_CHECK(h, "mean_lut_kernel");
+  const dim3 grid((dst_width + TILE_W - 1) / TILE_W, (dst_height + 31) / 32, batch);
+#define FRCNN_RAGGED(CN) \
+  resize_cubic_ragged_kernel<CN><<<grid, 256, 0, stream>>>(src, offs, src_bytes, geom, flip, dst_height, dst_width, tabc, lutf, out_u8, out_f32)
+  switch (cn) {
+    case 1: FRCNN_RAGGED(1); break;
+    case 2: FRCNN_RAGGED(2); break;
+    case 3: FRCNN_RAGGED(3); break;
+    default: FRCNN_RAGGED(4); break;
+  }
+#undef FRCNN_RAGGED
+  FRCNN_LAUNCH_CHECK(h, "resize_cubic_ragged_kernel");
   return FRCNN_OK;
 }
 

@@ -91,6 +91,72 @@ rpn_losses_kernel(const unsigned char* __restrict__ can_use, const unsigned char
   }
 }
 
+// The same losses on a padded batch: inputs [B, rows*cols*A] with image b's own map (rows_b, cols_b) = extents[b]
+// (clamped to the padded map).  Threads walk the image's OWN flat index i = ((y*cols_b + x)*A + a) with the thread
+// mapping of rpn_losses_kernel, so every partial sum, the reduction and mean_sel = #sel / n_b are those of the call on
+// the cropped inputs: loss[b] and both gradients equal it bit for bit.  Padding is never read; its gradients are zero.
+// An empty extent gives loss (0, 0) and zero gradients.  One CTA per SM, as rpn_losses_kernel: left free, ptxas aims at
+// two and spills at 32 registers.
+__global__ void __launch_bounds__(LOSS_THREADS, 1)
+rpn_losses_ragged_kernel(const unsigned char* __restrict__ can_use, const unsigned char* __restrict__ is_pos,
+                         const float4* __restrict__ bbreg, const float* __restrict__ cls_pred,
+                         const float4* __restrict__ reg_pred, int rows, int cols, int n_anchors,
+                         const int* __restrict__ extents, float* __restrict__ loss, float* __restrict__ grad_cls,
+                         float4* __restrict__ grad_reg) {
+  __shared__ double scratch[3 * (LOSS_THREADS / 32)];
+  const int img = blockIdx.x, tid = threadIdx.x;
+  const int rows_b = min(max(extents[2 * img], 0), rows), cols_b = min(max(extents[2 * img + 1], 0), cols);
+  const int n = rows * cols * n_anchors, n_b = rows_b * cols_b * n_anchors, row_b = cols_b * n_anchors;
+  const int row = cols * n_anchors;
+  const size_t base = (size_t)img * n;
+  const float eps = 1e-7f, one_m_eps = 1.0f - 1e-7f;
+  double acc[3] = {0.0, 0.0, 0.0};
+  for (int i = tid; i < n_b; i += LOSS_THREADS) {
+    const int y = i / row_b;
+    const size_t j = base + (size_t)y * row + (i - y * row_b);      // the same cell and anchor in the padded layout
+    const bool use = can_use[j] != 0, pos = is_pos[j] != 0;
+    const float p = fminf(fmaxf(cls_pred[j], eps), one_m_eps);
+    const float x = logf(p / (1.0f - p));
+    const float z = pos ? 1.0f : 0.0f;
+    const float bce = fmaxf(x, 0.0f) - x * z + log1pf(expf(-fabsf(x)));
+    if (use) acc[0] += (double)bce;
+    const float4 t = bbreg[j], q = reg_pred[j];
+    acc[1] += (double)smooth_l1(t.x - q.x) + (double)smooth_l1(t.y - q.y) + (double)smooth_l1(t.z - q.z) +
+              (double)smooth_l1(t.w - q.w);
+    if (use && pos) acc[2] += 1.0;
+  }
+  block_sum<3>(acc, scratch);
+  const float mean_sel = n_b > 0 ? (float)(acc[2] / (double)n_b) : 0.0f;
+  if (tid == 0) {
+    loss[2 * img + 0] = (float)acc[0] / 256.0f;
+    loss[2 * img + 1] = mean_sel * (10.0f * (float)acc[1] / 2400.0f);
+  }
+  if (!grad_cls && !grad_reg) return;
+  const float scale = mean_sel * (10.0f / 2400.0f);
+  for (int j = tid; j < n; j += LOSS_THREADS) {                     // padded index: every output element once
+    const int y = j / row, k = j - y * row;
+    const size_t e = base + j;
+    if (y >= rows_b || k >= row_b) {
+      if (grad_cls) grad_cls[e] = 0.0f;
+      if (grad_reg) grad_reg[e] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+      continue;
+    }
+    if (grad_cls) {
+      const bool use = can_use[e] != 0, pos = is_pos[e] != 0;
+      const float p_raw = cls_pred[e];
+      const float p = fminf(fmaxf(p_raw, eps), one_m_eps);
+      const float z = pos ? 1.0f : 0.0f;
+      const bool inside = p_raw >= eps && p_raw <= one_m_eps;
+      grad_cls[e] = (use && inside) ? (p - z) / (p * (1.0f - p)) / 256.0f : 0.0f;
+    }
+    if (grad_reg) {
+      const float4 t = bbreg[e], q = reg_pred[e];
+      grad_reg[e] = make_float4(-scale * smooth_l1_grad(t.x - q.x), -scale * smooth_l1_grad(t.y - q.y),
+                                -scale * smooth_l1_grad(t.z - q.z), -scale * smooth_l1_grad(t.w - q.w));
+    }
+  }
+}
+
 // y_class [B,M,K] i32 one-hot, y_transform [B,M,8Kf] f32 = [labels | targets], cls_pred [B,M,K], reg_pred [B,M,4Kf]
 // loss [B,2] = (cls_loss_det, bbreg_loss_det); grads optional
 __global__ void __launch_bounds__(LOSS_THREADS)
@@ -158,6 +224,17 @@ int launch_rpn_losses(frcnn_handle* h, cudaStream_t stream, const uint8_t* can_u
                                                        reinterpret_cast<const float4*>(reg_pred), n, loss, grad_cls,
                                                        reinterpret_cast<float4*>(grad_reg));
   FRCNN_LAUNCH_CHECK(h, "rpn_losses_kernel");
+  return FRCNN_OK;
+}
+
+int launch_rpn_losses_ragged(frcnn_handle* h, cudaStream_t stream, const uint8_t* can_use, const uint8_t* is_pos,
+                             const float* bbreg, const float* cls_pred, const float* reg_pred, int rows, int cols,
+                             int n_anchors, int batch, const int32_t* extents, float* loss, float* grad_cls,
+                             float* grad_reg) {
+  rpn_losses_ragged_kernel<<<batch, LOSS_THREADS, 0, stream>>>(
+      can_use, is_pos, reinterpret_cast<const float4*>(bbreg), cls_pred, reinterpret_cast<const float4*>(reg_pred), rows,
+      cols, n_anchors, extents, loss, grad_cls, reinterpret_cast<float4*>(grad_reg));
+  FRCNN_LAUNCH_CHECK(h, "rpn_losses_ragged_kernel");
   return FRCNN_OK;
 }
 

@@ -24,15 +24,16 @@ LAMBDA_REG_DET = 1
 
 class _RpnLosses(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, cls_pred, reg_pred, can_use, is_pos, bbreg):
-        loss, g_cls, g_reg = ops.rpn_losses(can_use, is_pos, bbreg, cls_pred.contiguous(), reg_pred.contiguous(), want_grad=True)
+    def forward(ctx, cls_pred, reg_pred, can_use, is_pos, bbreg, extents, padded_shape):
+        loss, g_cls, g_reg = ops.rpn_losses(can_use, is_pos, bbreg, cls_pred.contiguous(), reg_pred.contiguous(), want_grad=True,
+                                            extents=extents, padded_shape=padded_shape)
         ctx.save_for_backward(g_cls, g_reg)
         return loss
 
     @staticmethod
     def backward(ctx, grad_loss):
         g_cls, g_reg = ctx.saved_tensors
-        return g_cls * grad_loss[:, 0:1], g_reg * grad_loss[:, 1].reshape(-1, 1, 1), None, None, None
+        return g_cls * grad_loss[:, 0:1], g_reg * grad_loss[:, 1].reshape(-1, 1, 1), None, None, None, None, None
 
 
 class _DetLosses(torch.autograd.Function):
@@ -48,10 +49,11 @@ class _DetLosses(torch.autograd.Function):
         return g_cls * grad_loss[:, 0].reshape(-1, 1, 1), g_reg * grad_loss[:, 1].reshape(-1, 1, 1), None, None
 
 
-def rpn_losses(cls_pred, reg_pred, can_use, is_pos, bbreg):
+def rpn_losses(cls_pred, reg_pred, can_use, is_pos, bbreg, extents=None, padded_shape=None):
     """cls_pred (B,N) f32 sigmoid outputs, reg_pred (B,N,4) f32, labels as `ops.label_anchors` emits them ->
-    loss (B,2) = (cls_loss_rpn, bbreg_loss_rpn), differentiable w.r.t. the two predictions."""
-    return _RpnLosses.apply(cls_pred, reg_pred, can_use, is_pos, bbreg)
+    loss (B,2) = (cls_loss_rpn, bbreg_loss_rpn), differentiable w.r.t. the two predictions.  A padded batch of
+    differently sized maps passes `extents` and `padded_shape` as `ops.rpn_losses` takes them."""
+    return _RpnLosses.apply(cls_pred, reg_pred, can_use, is_pos, bbreg, extents, padded_shape)
 
 
 def det_losses(cls_pred, reg_pred, y_class_num, y_transform):

@@ -413,9 +413,12 @@ def pad_rois(rois, count, group=64, out=None):
     return out, rows
 
 
-def rpn_losses(can_use, is_pos, bbreg, cls_pred, reg_pred, want_grad=False):
+def rpn_losses(can_use, is_pos, bbreg, cls_pred, reg_pred, want_grad=False, extents=None, padded_shape=None):
     """loss_functions.py:15-48 fused with the unpacked RPN labels.  can_use/is_pos (B,N) u8, bbreg (B,N,4) f32,
-    cls_pred (B,N) f32, reg_pred (B,N,4) f32 -> loss (B,2) f32 = (class, box) [, grad_cls (B,N), grad_reg (B,N,4)]."""
+    cls_pred (B,N) f32, reg_pred (B,N,4) f32 -> loss (B,2) f32 = (class, box) [, grad_cls (B,N), grad_reg (B,N,4)].
+    `extents` (B,2) i32 (rows_b, cols_b) on the device with `padded_shape` = (rows, cols): N = rows*cols*A in the padded
+    (R,C,A) layout of `label_anchors(..., extents=)`; each image's loss and gradients are those of the call on its own
+    map (its box loss averages over its own anchors), the padding is never read and gets zero gradients."""
     can_use, is_pos = _chk(can_use, torch.uint8, "can_use", 2), _chk(is_pos, torch.uint8, "is_pos", 2)
     bbreg, reg_pred = _chk(bbreg, torch.float32, "bbreg", 3), _chk(reg_pred, torch.float32, "reg_pred", 3)
     cls_pred = _chk(cls_pred, torch.float32, "cls_pred", 2)
@@ -423,11 +426,22 @@ def rpn_losses(can_use, is_pos, bbreg, cls_pred, reg_pred, want_grad=False):
     b, n = can_use.shape
     if cls_pred.shape != (b, n) or bbreg.shape != (b, n, 4) or reg_pred.shape != (b, n, 4):
         raise ValueError("rpn_losses: shapes must be (B,N), (B,N), (B,N,4), (B,N), (B,N,4)")
+    if (extents is None) != (padded_shape is None):
+        raise ValueError("rpn_losses: give extents and padded_shape together")
+    if extents is not None:
+        rows, cols = (int(v) for v in padded_shape)
+        if rows <= 0 or cols <= 0 or n % (rows * cols) != 0:
+            raise ValueError("rpn_losses: N = %d is not rows * cols * A for padded_shape %s" % (n, (rows, cols)))
+        extents = _chk_extents(extents, b)
     loss = ctx.empty((b, 2), torch.float32)
     g_cls = ctx.empty((b, n), torch.float32) if want_grad else None
     g_reg = ctx.empty((b, n, 4), torch.float32) if want_grad else None
-    ctx.call("frcnn_rpn_losses", ptr(can_use), ptr(is_pos), ptr(bbreg), ptr(cls_pred), ptr(reg_pred), n, b, ptr(loss),
-             ptr(g_cls), ptr(g_reg))
+    if extents is not None:
+        ctx.call("frcnn_rpn_losses_ragged", ptr(can_use), ptr(is_pos), ptr(bbreg), ptr(cls_pred), ptr(reg_pred), rows, cols,
+                 n // (rows * cols), b, ptr(extents), ptr(loss), ptr(g_cls), ptr(g_reg))
+    else:
+        ctx.call("frcnn_rpn_losses", ptr(can_use), ptr(is_pos), ptr(bbreg), ptr(cls_pred), ptr(reg_pred), n, b, ptr(loss),
+                 ptr(g_cls), ptr(g_reg))
     return (loss, g_cls, g_reg) if want_grad else loss
 
 
@@ -495,6 +509,85 @@ def image_resize_cubic(images, dst_height, dst_width, flip=False, mean=None, wan
         if mean_arr.shape[0] != c:
             raise ValueError("mean must have one entry per channel")
     ctx.call("frcnn_image_resize_cubic", ptr(images), h, w, c, int(dst_height), int(dst_width), int(bool(flip)), b,
+             None if mean_arr is None else mean_arr.ctypes.data_as(C.c_void_p), ptr(out_u8), ptr(out_f))
+    if out_u8 is not None and out_f is not None:
+        return out_u8, out_f
+    return out_u8 if out_u8 is not None else out_f
+
+
+def pack_images(sources):
+    """A list of (h_b, w_b, C) uint8 images (numpy or torch, one channel count) -> (packed (T,) u8, offsets (B,) i64 byte
+    offsets, sizes (B,2) i32 (h_b, w_b)), all CUDA tensors: the source layout of `image_resize_cubic_ragged`.  Host images
+    are staged in one pinned buffer and uploaded with one asynchronous copy."""
+    if not isinstance(sources, (list, tuple)) or len(sources) == 0:
+        raise ValueError("pack_images needs a non-empty list of (h, w, C) uint8 images")
+    for x in sources:
+        if not isinstance(x, (np.ndarray, torch.Tensor)):
+            raise TypeError("pack_images takes numpy arrays or torch tensors, got %s" % type(x).__name__)
+        if x.dtype not in (np.uint8, torch.uint8):
+            raise TypeError("pack_images needs uint8 images, got %s" % x.dtype)
+    shapes = [tuple(x.shape) for x in sources]
+    if any(len(s) != 3 for s in shapes):
+        raise ValueError("every image must have 3 dimensions (h, w, C), got %s" % (shapes,))
+    if len({s[2] for s in shapes}) != 1:
+        raise ValueError("images disagree in their channel count: %s" % (shapes,))
+    nbytes = np.array([s[0] * s[1] * s[2] for s in shapes], np.int64)
+    offsets = np.concatenate([[0], np.cumsum(nbytes)[:-1]]).astype(np.int64)
+    cuda = [x for x in sources if isinstance(x, torch.Tensor) and x.is_cuda]
+    ctx = get_context(cuda[0].device if cuda else None)
+    total = max(int(nbytes.sum()), 1)
+    if cuda:
+        packed = ctx.empty((total,), torch.uint8)
+        for x, o, n in zip(sources, offsets.tolist(), nbytes.tolist()):
+            t = x if isinstance(x, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(x))
+            packed[o:o + n].copy_(t.reshape(-1), non_blocking=True)
+    else:
+        pinned = torch.empty((total,), dtype=torch.uint8, pin_memory=True)
+        view = pinned.numpy()
+        for x, o, n in zip(sources, offsets.tolist(), nbytes.tolist()):
+            view[o:o + n] = (x.numpy() if isinstance(x, torch.Tensor) else np.asarray(x)).reshape(-1)
+        packed = pinned.to(ctx.device, non_blocking=True)
+    sizes = np.array([s[:2] for s in shapes], np.int32).reshape(-1, 2)
+    return packed, ctx.to_device(offsets), ctx.to_device(sizes)
+
+
+def image_resize_cubic_ragged(src, src_offsets, geom, dst_height, dst_width, flip=None, mean=None, want_u8=True, out=None,
+                              channels=3):
+    """`image_resize_cubic` for differently sized sources in one launch.  src (T,) u8 = the images packed back to back
+    (`pack_images`), src_offsets (B,) i64, geom (B,4) i32 = (src_h, src_w, dst_h, dst_w) per image, flip (B,) u8 or None,
+    all CUDA tensors (never read on the host: the call can be captured in a graph).  Image b is resized to its own
+    (dst_h, dst_w) [and mirrored within that width] into the padded (B,dst_height,dst_width,C) output; every padding
+    element is written as zero.  Returns u8, (u8, f32) or f32 as `image_resize_cubic`; `out` = (u8 or None, f32 or None)
+    takes preallocated buffers of that shape."""
+    src, src_offsets = _chk(src, torch.uint8, "src", 1), _chk(src_offsets, torch.int64, "src_offsets", 1)
+    geom = _chk(geom, torch.int32, "geom", 2)
+    b, c, h, w = src_offsets.shape[0], int(channels), int(dst_height), int(dst_width)
+    if geom.shape != (b, 4):
+        raise ValueError("geom must be (B, 4) = (%d, 4), got %s" % (b, tuple(geom.shape)))
+    if flip is not None:
+        flip = _chk(flip, torch.uint8, "flip", 1)
+        if flip.shape != (b,):
+            raise ValueError("flip must be (B,) = (%d,)" % b)
+    if not want_u8 and mean is None:
+        raise ValueError("nothing to compute: want_u8=False and no mean")
+    ctx = get_context(src.device)
+    shape = (b, h, w, c)
+    if out is not None:
+        if len(out) != 2 or (want_u8 and out[0] is None) or (mean is not None and out[1] is None):
+            raise ValueError("out must be (u8, f32) with a u8 buffer when want_u8 and a f32 buffer when mean is given")
+        out_u8 = _chk_out(out[0], torch.uint8, "out u8", 4) if want_u8 else None
+        out_f = _chk_out(out[1], torch.float32, "out f32", 4) if mean is not None else None
+        if any(t is not None and tuple(t.shape) != shape for t in (out_u8, out_f)):
+            raise ValueError("out buffers must be %s" % (shape,))
+    else:
+        out_u8 = ctx.empty(shape, torch.uint8) if want_u8 else None
+        out_f = ctx.empty(shape, torch.float32) if mean is not None else None
+    mean_arr = None
+    if mean is not None:
+        mean_arr = np.ascontiguousarray(np.asarray(mean, dtype=np.float64).reshape(-1))
+        if mean_arr.shape[0] != c:
+            raise ValueError("mean must have one entry per channel")
+    ctx.call("frcnn_image_resize_cubic_ragged", ptr(src), ptr(src_offsets), src.numel(), ptr(geom), ptr(flip), c, h, w, b,
              None if mean_arr is None else mean_arr.ctypes.data_as(C.c_void_p), ptr(out_u8), ptr(out_f))
     if out_u8 is not None and out_f is not None:
         return out_u8, out_f

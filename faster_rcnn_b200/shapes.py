@@ -6,7 +6,8 @@ object works, including the reference's own ``shapes.Image``.  ``Image`` can be
 built from in-memory pixels or from an ``image_path`` (lazy ``cv2.imread`` like
 the reference); ``.data`` is the reference's host path (cv2 resize + flip),
 ``.data_device()`` / ``.preprocessed_device()`` do the resize, flip and mean
-subtraction on the GPU (SURVEY 8f-4, `ops.image_resize_cubic`).
+subtraction on the GPU (SURVEY 8f-4, `ops.image_resize_cubic`); `preprocessed_batch_device` does it for a batch of
+differently sized images in one padded device call (`ops.image_resize_cubic_ragged`).
 """
 import numpy as np
 
@@ -174,3 +175,36 @@ class Image:
     @property
     def num_gt_boxes(self):
         return len(self.gt_boxes)
+
+
+def preprocessed_batch_device(images, mean=None, pad_to=None):
+    """`Image.preprocessed_device` for a batch of differently sized images in one device call: every image is resized
+    (and mirrored, under the rule of `data_device`) to its own height x width, minus the means, into one padded float32
+    (B,H,W,C) CUDA tensor whose padding is zero.  (H, W) = the largest image, or `pad_to` (which must hold every image).
+    Returns (padded, extents (B,2) i32 (height, width) on the device).  The raw pixels are packed on the host and uploaded
+    with one copy (`ops.pack_images`, which uploads their offsets and sizes too), the target sizes and mirror flags with
+    one more; `ops.image_resize_cubic_ragged` does the rest."""
+    from . import ops
+    images = list(images)
+    if not images:
+        raise ValueError("preprocessed_batch_device needs at least one image")
+    raws = [img._raw() for img in images]
+    sizes = np.array([(img.height, img.width) for img in images], np.int32).reshape(-1, 2)
+    height, width = (int(v) for v in sizes.max(axis=0))
+    if pad_to is not None:
+        ph, pw = (int(v) for v in pad_to)
+        if ph < height or pw < width:
+            raise ValueError("pad_to %s is smaller than the largest image (%d, %d)" % ((ph, pw), height, width))
+        height, width = ph, pw
+    import torch
+    from .runtime import get_context
+    src, offsets, src_sizes = ops.pack_images(raws)
+    # target size and mirror flag of every image in one upload; the source sizes come from pack_images
+    flip = np.array([[img.flipped and img.image_path is not None] for img in images], np.int32)
+    meta = get_context(src.device).to_device(np.concatenate([sizes, flip], axis=1))
+    extents = meta[:, :2].contiguous()
+    geom = torch.cat([src_sizes, extents], dim=1)
+    mean = ops.IMAGENET_MEAN_BGR if mean is None else mean
+    out = ops.image_resize_cubic_ragged(src, offsets, geom, height, width, flip=meta[:, 2].to(torch.uint8), mean=mean,
+                                        want_u8=False, channels=raws[0].shape[2])
+    return out, extents

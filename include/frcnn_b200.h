@@ -323,6 +323,16 @@ FRCNN_API int frcnn_gather_det_samples(frcnn_handle* h, void* stream, const int1
 FRCNN_API int frcnn_rpn_losses(frcnn_handle* h, void* stream, const uint8_t* can_use, const uint8_t* is_pos,
                                const float* bbreg, const float* cls_pred, const float* reg_pred,
                                int n_per_image, int batch, float* loss, float* grad_cls, float* grad_reg);
+/* RPN losses of a mixed-size batch: the inputs of frcnn_rpn_losses in the padded [batch,rows*cols*n_anchors] layout
+ * ((R,C,A) order), extents [batch,2] i32 (device) = each image's own (rows_b, cols_b), clamped to [0,rows] x [0,cols].
+ * loss[b] and the gradients of image b equal frcnn_rpn_losses on the cropped inputs [:rows_b, :cols_b] bit for bit
+ * (the box loss's mean(mask) runs over the image's own rows_b*cols_b*A anchors).  Padding cells are never read; their
+ * gradients are written as zero.  An image with a zero extent gets loss (0, 0) and zero gradients (the uniform entry
+ * rejects n_per_image = 0). */
+FRCNN_API int frcnn_rpn_losses_ragged(frcnn_handle* h, void* stream, const uint8_t* can_use, const uint8_t* is_pos,
+                                      const float* bbreg, const float* cls_pred, const float* reg_pred, int rows,
+                                      int cols, int n_anchors, int batch, const int32_t* extents, float* loss,
+                                      float* grad_cls, float* grad_reg);
 FRCNN_API int frcnn_det_losses(frcnn_handle* h, void* stream, const int32_t* y_class,
                                const float* y_transform, const float* cls_pred, const float* reg_pred,
                                int m_rows, int n_classes, int batch, float* loss, float* grad_cls,
@@ -356,6 +366,20 @@ FRCNN_API int frcnn_voc_pr_ap(frcnn_handle* h, void* stream, const double* tp, c
 FRCNN_API int frcnn_image_resize_cubic(frcnn_handle* h, void* stream, const uint8_t* src, int src_height, int src_width,
                              int channels, int dst_height, int dst_width, int flip, int batch,
                              const double* mean_host, uint8_t* out_u8, float* out_f32);
+
+/* The same for a batch of DIFFERENTLY sized sources, each resized to its own size, in one launch.
+ *   src: uint8 images [src_h_b, src_w_b, channels] packed back to back; src_offsets [batch] i64 byte offsets into it,
+ *   src_bytes = size of the buffer.  geom [batch,4] i32 = (src_h_b, src_w_b, dst_h_b, dst_w_b), flip [batch] u8 (NULL =
+ *   no mirror; else image b is mirrored within its own width where flip[b] != 0); all three on the device and never
+ *   read on the host, so one captured graph serves every mix of sizes up to its padded shape.
+ *   out_u8 / out_f32 [batch,dst_height,dst_width,channels] (either may be NULL; mean_host as above): out[b, :dst_h_b,
+ *   :dst_w_b] equals frcnn_image_resize_cubic on image b alone bit for bit; every other element is written as zero.
+ *   dst_h_b / dst_w_b are clamped to [0,dst_height] x [0,dst_width].  An image whose source size is not positive or
+ *   whose bytes do not lie within [0, src_bytes) is written as zeros and none of its bytes are read. */
+FRCNN_API int frcnn_image_resize_cubic_ragged(frcnn_handle* h, void* stream, const uint8_t* src, const int64_t* src_offsets,
+                                              long long src_bytes, const int32_t* geom, const uint8_t* flip, int channels,
+                                              int dst_height, int dst_width, int batch, const double* mean_host,
+                                              uint8_t* out_u8, float* out_f32);
 
 /* GT boxes of a resized / mirrored image (shapes.py:93-101 Box.resize, :292-300 horizontal_flip): boxes
  * [batch,n_max,4] f64 corners, n_box [batch] i32 (NULL = n_max), ratio [batch] f64, flip_width [batch] f64 (NULL or a
