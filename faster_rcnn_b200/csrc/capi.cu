@@ -54,6 +54,10 @@ int launch_image_resize_ragged(frcnn_handle*, cudaStream_t, const uint8_t*, cons
                                const uint8_t*, int, int, int, int, const double*, uint8_t*, float*);
 int launch_gt_transform(frcnn_handle*, cudaStream_t, const double*, const int32_t*, int, int, const double*, const double*,
                         double*);
+int launch_sample_rpn(frcnn_handle*, cudaStream_t, uint8_t*, const uint8_t*, const int32_t*, int, int, int, int,
+                      const int32_t*, int, int, const int64_t*, int);
+int launch_sample_det(frcnn_handle*, cudaStream_t, const uint8_t*, const int32_t*, int, int, const int64_t*, int, int32_t*,
+                      uint8_t*);
 
 // ---- scratch arena -------------------------------------------------------------------------
 // Bump allocator over one device block.  Every public entry point starts with arena_reset();
@@ -606,6 +610,40 @@ int frcnn_gt_transform(frcnn_handle* h, void* stream, const double* boxes, const
   FRCNN_REQUIRE(h, boxes && ratio && out, "gt_transform: null pointer");
   FRCNN_REQUIRE(h, n_max > 0 && batch > 0 && batch <= 65535, "gt_transform: bad size");
   return launch_gt_transform(h, st, boxes, n_box, n_max, batch, ratio, flip_width, out);
+}
+
+static int sample_rpn_entry(frcnn_handle* h, cudaStream_t st, uint8_t* can_use, const uint8_t* is_pos, const int32_t* counts,
+                            int rows, int cols, int n_anchors, const int32_t* extents, int max_pos, int sample_size,
+                            const int64_t* state, int batch) {
+  FRCNN_REQUIRE(h, can_use && is_pos && counts && state, "sample_rpn: null pointer");
+  FRCNN_REQUIRE(h, rows > 0 && cols > 0 && n_anchors > 0 && batch > 0, "sample_rpn: non-positive size");
+  FRCNN_REQUIRE(h, (long long)rows * cols * n_anchors < (1LL << 31), "sample_rpn: map too large");
+  FRCNN_REQUIRE(h, max_pos >= 0 && sample_size >= max_pos, "sample_rpn: need 0 <= max_pos <= sample_size");
+  return launch_sample_rpn(h, st, can_use, is_pos, counts, rows * cols * n_anchors, rows, cols, n_anchors, extents, max_pos,
+                           sample_size, state, batch);
+}
+
+int frcnn_sample_rpn(frcnn_handle* h, void* stream, uint8_t* can_use, const uint8_t* is_pos, const int32_t* counts,
+                     int n_per_image, int max_pos, int sample_size, const int64_t* state, int batch) {
+  FRCNN_ENTER(h, stream);
+  return sample_rpn_entry(h, st, can_use, is_pos, counts, 1, n_per_image, 1, nullptr, max_pos, sample_size, state, batch);
+}
+
+int frcnn_sample_rpn_ragged(frcnn_handle* h, void* stream, uint8_t* can_use, const uint8_t* is_pos, const int32_t* counts,
+                            int rows, int cols, int n_anchors, const int32_t* extents, int max_pos, int sample_size,
+                            const int64_t* state, int batch) {
+  FRCNN_ENTER(h, stream);
+  FRCNN_REQUIRE(h, extents, "sample_rpn_ragged: null extents");
+  return sample_rpn_entry(h, st, can_use, is_pos, counts, rows, cols, n_anchors, extents, max_pos, sample_size, state,
+                          batch);
+}
+
+int frcnn_sample_det(frcnn_handle* h, void* stream, const uint8_t* is_pos, const int32_t* n_rows, int n_max, int n_samples,
+                     const int64_t* state, int batch, int32_t* out_index, uint8_t* out_has) {
+  FRCNN_ENTER(h, stream);
+  FRCNN_REQUIRE(h, is_pos && n_rows && state && out_index && out_has, "sample_det: null pointer");
+  FRCNN_REQUIRE(h, n_max > 0 && n_samples > 0 && batch > 0, "sample_det: non-positive size");
+  return launch_sample_det(h, st, is_pos, n_rows, n_max, n_samples, state, batch, out_index, out_has);
 }
 
 }  // extern "C"

@@ -183,6 +183,67 @@ def pack_rpn_targets(can_use, is_pos, bbreg, rows, cols, n_anchors, off_pos=None
     return y_class, y_bbreg
 
 
+def sampler_state(seed, device=None):
+    """The device RNG state of `sample_rpn_` / `sample_det`: a CUDA int64 tensor [seed, offset = 0].  The kernels read it
+    on the device and the calls advance the offset by the batch size, so a captured CUDA graph draws new samples on
+    every replay.  `seed` is taken modulo 2^64 (stored as its two's complement int64)."""
+    s = int(seed) & 0xffffffffffffffff
+    return torch.tensor([s - (1 << 64) if s >= 1 << 63 else s, 0], dtype=torch.int64, device=get_context(device).device)
+
+
+def _chk_state(state):
+    state = _chk_out(state, torch.int64, "state", 1)
+    if state.shape != (2,):
+        raise ValueError("state must be the (2,) int64 tensor of sampler_state(), got shape %s" % (tuple(state.shape),))
+    return state
+
+
+def sample_rpn_(can_use, is_pos, counts, state, extents=None, padded_shape=None, n_anchors=None, max_pos=128,
+                sample_size=256):
+    """rpn_util.py:324-350 drawn on the device: in each image keeps min(#pos, max_pos) usable positives and
+    min(#neg, sample_size - kept positives) usable negatives, a uniformly random subset of each chosen with the
+    counter-based RNG of `state` (sampler_state), and clears can_use of the others IN PLACE.  can_use / is_pos (B,N) u8
+    and counts (B,2) i32 as label_anchors returns them.  `extents` (B,2) i32 with `padded_shape` = (rows, cols) and
+    `n_anchors`: the padded layout of label_anchors(..., extents=); each image's draw equals the call on its own map.
+    Advances state[1] by B (stream-ordered).  Returns can_use."""
+    can_use = _chk_out(can_use, torch.uint8, "can_use", 2)
+    is_pos, counts = _chk(is_pos, torch.uint8, "is_pos", 2), _chk(counts, torch.int32, "counts", 2)
+    state = _chk_state(state)
+    ctx = get_context(can_use.device)
+    b, n = can_use.shape
+    if is_pos.shape != (b, n) or counts.shape != (b, 2):
+        raise ValueError("sample_rpn_: shapes must be (B,N), (B,N), (B,2)")
+    if extents is not None:
+        if padded_shape is None or n_anchors is None:
+            raise ValueError("sample_rpn_: extents need padded_shape and n_anchors")
+        rows, cols = (int(v) for v in padded_shape)
+        if rows * cols * int(n_anchors) != n:
+            raise ValueError("sample_rpn_: N = %d is not rows * cols * n_anchors" % n)
+        ctx.call("frcnn_sample_rpn_ragged", ptr(can_use), ptr(is_pos), ptr(counts), rows, cols, int(n_anchors),
+                 ptr(_chk_extents(extents, b)), int(max_pos), int(sample_size), ptr(state), b)
+    else:
+        ctx.call("frcnn_sample_rpn", ptr(can_use), ptr(is_pos), ptr(counts), n, int(max_pos), int(sample_size), ptr(state), b)
+    state[1:].add_(b)
+    return can_use
+
+
+def sample_det(is_pos, n_rows, n_samples, state):
+    """det_util.py:260-306 drawn on the device with the counter-based RNG of `state` (sampler_state).  is_pos (B,n_max)
+    u8 flags of label_rois's rows, n_rows (B,) i32 its count -> index (B,S) i32 (the input of gather_det_samples,
+    positives first; -1 rows for an image without an eligible row), has (B,) bool.  Advances state[1] by B."""
+    is_pos, n_rows = _chk(is_pos, torch.uint8, "is_pos", 2), _chk(n_rows, torch.int32, "n_rows", 1)
+    state = _chk_state(state)
+    ctx = get_context(is_pos.device)
+    b, n_max = is_pos.shape
+    if n_rows.shape != (b,):
+        raise ValueError("sample_det: n_rows must be (B,)")
+    s = int(n_samples)
+    index, has = ctx.empty((b, s), torch.int32), ctx.empty((b,), torch.bool)
+    ctx.call("frcnn_sample_det", ptr(is_pos), ptr(n_rows), n_max, s, ptr(state), b, ptr(index), ptr(has))
+    state[1:].add_(b)
+    return index, has
+
+
 def label_rois(rois, gt, gt_cls, n_gt, n_classes, n_roi=None):
     """K-c'.  rois (B,n_max,4) i16, gt (B,Gmax,4) f64 feature units, gt_cls (B,Gmax) i32, n_gt (B,) ->
     out_rois (B,n_max,4) i16, y_class (B,n_max,K) i32, y_transform (B,n_max,8(K-1)) f32,

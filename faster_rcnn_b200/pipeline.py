@@ -302,10 +302,11 @@ class DetTrainingPipeline:
         >= 0.5, one-hot classes, class-specific regression targets) -> 64-RoI mini-batch (<= 25 % positives)
         [-> RoI layer on the sampled RoIs]
 
-    Only the mini-batch draw runs on the host: it replays `det_util._get_det_samples` with numpy's legacy global RNG,
-    image by image in batch order, so the result equals calling the reference-shaped manager on each image in turn
-    (one D2H of the positive flags and counts, one H2D of the B x 64 sample rows).  An image without an eligible RoI
-    (the reference returns 4 x None) gets zero rows and `has_rois[b] = False`."""
+    By default only the mini-batch draw runs on the host: it replays `det_util._get_det_samples` with numpy's legacy
+    global RNG, image by image in batch order, so the result equals calling the reference-shaped manager on each image in
+    turn (one D2H of the positive flags and counts, one H2D of the B x 64 sample rows).  Given a `state`
+    (ops.sampler_state) the draw runs on the device with a counter-based RNG instead (same rule, different stream).  An
+    image without an eligible RoI (the reference returns 4 x None) gets zero rows and `has_rois[b] = False`."""
 
     def __init__(self, class_mapping, anchor_dims=DEFAULT_ANCHORS, stride=16, num_rois=64, pre_nms_topk=12000,
                  nms_thresh=0.7, max_boxes=2000, pool_size=7, mode="resize", device=None):
@@ -335,12 +336,16 @@ class DetTrainingPipeline:
         n_gt = np.array([len(g) for g, _ in per], np.int32)
         return self.ctx.to_device(gt), self.ctx.to_device(gt_cls), self.ctx.to_device(n_gt)
 
-    def targets(self, cls, regr, gt, gt_cls, n_gt, chunk=32, extents=None):
+    def targets(self, cls, regr, gt, gt_cls, n_gt, chunk=32, extents=None, state=None):
         """CUDA tensors in -> (rois (B,S,4) i16, y_class_num (B,S,K) i32, y_transform (B,S,8(K-1)) f32) on the device and
         has_rois (B,) bool on the host.  The batch is enqueued in chunks of `chunk` images; the host draws the
         mini-batches of chunk i (in image order, so the RNG stream is the per-image one) while the GPU is still
-        labelling chunks i+1..  `extents` (B,2) i32 on the device: a padded batch of differently sized maps."""
-        from .det_util import _get_det_samples
+        labelling chunks i+1..  `extents` (B,2) i32 on the device: a padded batch of differently sized maps.
+
+        With `state` (ops.sampler_state) the mini-batches are drawn on the device instead (ops.sample_det: the same rule,
+        a counter-based RNG stream): nothing returns to the host, has_rois is a CUDA bool tensor, the call can be
+        captured in a CUDA graph, and image b's draw depends on (seed, offset + b) only, so not on `chunk`.  The
+        state's offset advances by B."""
         b, dev = cls.shape[0], self.ctx.device
         stream = torch.cuda.current_stream(dev)
         staged = []
@@ -351,6 +356,10 @@ class DetTrainingPipeline:
             l_rois, y_cls, y_tr, _, m = ops.label_rois(rois, gt[lo:hi], gt_cls[lo:hi], n_gt[lo:hi],
                                                        len(self.class_mapping), n_roi=count)
             found_d = (y_cls[:, :, -1] == 0).to(torch.uint8)                      # positives = not background
+            if state is not None:
+                index, has = ops.sample_det(found_d, m, self.num_rois, state)
+                staged.append(ops.gather_det_samples(l_rois, y_cls, y_tr, index) + (has,))
+                continue
             found_h = self._pin(("found", lo), found_d.shape, torch.uint8)     # cached: cudaHostAlloc costs ~0.1 ms
             m_h = self._pin(("m", lo), m.shape, m.dtype)
             found_h.copy_(found_d, non_blocking=True)
@@ -358,6 +367,9 @@ class DetTrainingPipeline:
             ev = torch.cuda.Event()
             ev.record(stream)
             staged.append((l_rois, y_cls, y_tr, found_h, m_h, ev))
+        if state is not None:
+            return tuple(torch.cat([o[j] for o in staged]) for j in range(4))
+        from .det_util import _get_det_samples
         outs, has = [], []
         for l_rois, y_cls, y_tr, found_h, m_h, ev in staged:
             ev.synchronize()
@@ -373,13 +385,15 @@ class DetTrainingPipeline:
         rois, y_cls, y_tr = (torch.cat([o[j] for o in outs]) for j in range(3))
         return rois, y_cls, y_tr, np.concatenate(has)
 
-    def __call__(self, cls, regr, feat, images, extents=None):
+    def __call__(self, cls, regr, feat, images, extents=None, state=None):
         """Host or device arrays + the images' ground truth -> (rois, y_class_num, y_transform, pooled, has_rois):
         the detector's training inputs and the RoI layer's output on the sampled RoIs (CUDA tensors).  Lists of
         per-image (R_b,C_b,X) arrays, or padded arrays with `extents`, are a batch of differently sized images; the
-        sampled RoIs lie inside each image's own map, so the RoI layer reads no padding."""
+        sampled RoIs lie inside each image's own map, so the RoI layer reads no padding.  `state`
+        (ops.sampler_state): mini-batches drawn on the device, see `targets`."""
         cls, regr, feat, extents = _padded_inputs(cls, regr, feat, extents)
         dev_in = [x if (isinstance(x, torch.Tensor) and x.is_cuda) else self.ctx.to_device(x, np.float32) for x in (cls, regr, feat)]
-        rois, y_cls, y_tr, has = self.targets(dev_in[0], dev_in[1], *self.ground_truth(images), extents=extents)
+        rois, y_cls, y_tr, has = self.targets(dev_in[0], dev_in[1], *self.ground_truth(images), extents=extents,
+                                              state=state)
         pooled = ops.roi_forward(dev_in[2], rois, self.pool_size, self.mode)
         return rois, y_cls, y_tr, pooled, has

@@ -4,6 +4,7 @@ Same call signatures, array layouts and RNG stream as the reference (citations: 
 /root/reference/faster_rcnn).  The anchor x GT labelling, the sampling switch-offs and the Keras
 `y_true` packing run in libfrcnn_b200.so (label.cu); only the draws of Python's `random` stay
 on the host, because bit-exact parity needs the reference's own MT19937 stream in its order.
+`RpnTrainingManager.rpn_targets_device` draws with the same rule on the device instead (sample.cu).
 """
 import random
 
@@ -41,7 +42,7 @@ class RpnTrainingManager:
     def _label_batch(self, images, extents=None, pad_to=None):
         """Labels a list of images that share one conv shape in a single launch sequence.
         Returns device tensors can_use (B,N) u8, is_pos (B,N) u8, bbreg (B,N,4) f32, counts (B,2).
-        With `extents` ((B,2) host array of the images' conv shapes) the images may differ: they are labelled as one
+        With `extents` ((B,2) i32 conv shapes of the images, a host array or a CUDA tensor) the images may differ: they are labelled as one
         batch padded to `pad_to` (rows, cols)."""
         ctx = get_context()
         rows, cols = pad_to if extents is not None else self.calc_conv_dims(images[0].height, images[0].width)
@@ -59,9 +60,10 @@ class RpnTrainingManager:
             n_gt[b] = len(img.gt_boxes)
             gt[b, :n_gt[b]] = get_bbox_coords(img.gt_boxes)
             wh[b] = img.width, img.height
+        if extents is not None and not isinstance(extents, torch.Tensor):
+            extents = ctx.to_device(extents)
         return ops.label_anchors(ctx.to_device(gt), ctx.to_device(n_gt), ctx.to_device(wh), rows, cols,
-                                 self.anchor_dims, self.stride,
-                                 extents=None if extents is None else ctx.to_device(extents))
+                                 self.anchor_dims, self.stride, extents=extents)
 
     @profile
     def _process(self, image):
@@ -112,15 +114,34 @@ class RpnTrainingManager:
         y_bbreg); the padding is zero, i.e. unusable anchors.  RNG draws happen image by image in list order, so the result
         equals calling `rpn_y_true` on each image in turn."""
         ctx = get_context()
+        extents, rows, cols = self._padded_extents(images, pad_to)
+        can_use, is_pos, bbreg, counts = self._label_batch(images, extents, (rows, cols))
+        y_class, y_bbreg = self._sample_and_pack(can_use, is_pos, bbreg, counts, rows, cols, len(self.anchor_dims))
+        return ctx.to_host(y_class).view(np.bool_), ctx.to_host(y_bbreg), extents
+
+    def rpn_targets_device(self, images, state, pad_to=None):
+        """RPN targets drawn on the device (not in the reference): list of images (any conv shapes) + the RNG state of
+        ops.sampler_state -> can_use (B,N) u8, is_pos (B,N) u8, bbreg (B,N,4) f32, extents (B,2) i32, all CUDA tensors
+        in the padded (R,C,A) layout of the largest conv shape or `pad_to`: exactly the inputs of
+        loss_functions.rpn_losses(..., extents=extents, padded_shape=(R, C)).  The 256-anchor mini-batch follows the
+        reference's rule with the counter-based RNG (ops.sample_rpn_), so nothing returns to the host; image b's draw
+        depends on (seed, offset + b) only, and state's offset advances by B."""
+        ext, rows, cols = self._padded_extents(images, pad_to)
+        extents = get_context().to_device(ext)
+        can_use, is_pos, bbreg, counts = self._label_batch(images, extents, (rows, cols))
+        ops.sample_rpn_(can_use, is_pos, counts, state, extents=extents, padded_shape=(rows, cols),
+                        n_anchors=len(self.anchor_dims), max_pos=MAX_POS_SAMPLES, sample_size=SAMPLE_SIZE)
+        return can_use, is_pos, bbreg, extents
+
+    def _padded_extents(self, images, pad_to):
+        """(B,2) i32 host array of the images' conv shapes and the padded (rows, cols): the largest of them or `pad_to`"""
         extents = np.array([tuple(self.calc_conv_dims(img.height, img.width)) for img in images], np.int32).reshape(-1, 2)
         rows, cols = (int(v) for v in extents.max(axis=0))
         if pad_to is not None:
             if pad_to[0] < rows or pad_to[1] < cols:
                 raise ValueError("pad_to %s is smaller than the largest conv shape (%d, %d)" % (tuple(pad_to), rows, cols))
             rows, cols = int(pad_to[0]), int(pad_to[1])
-        can_use, is_pos, bbreg, counts = self._label_batch(images, extents, (rows, cols))
-        y_class, y_bbreg = self._sample_and_pack(can_use, is_pos, bbreg, counts, rows, cols, len(self.anchor_dims))
-        return ctx.to_host(y_class).view(np.bool_), ctx.to_host(y_bbreg), extents
+        return extents, rows, cols
 
     def _sample_and_pack(self, can_use, is_pos, bbreg, counts, rows, cols, n_anchors):
         ctx = get_context()

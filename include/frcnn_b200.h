@@ -388,6 +388,43 @@ FRCNN_API int frcnn_image_resize_cubic_ragged(frcnn_handle* h, void* stream, con
 FRCNN_API int frcnn_gt_transform(frcnn_handle* h, void* stream, const double* boxes, const int32_t* n_box, int n_max,
                        int batch, const double* ratio, const double* flip_width, double* out);
 
+/* ---- training mini-batch draws on the device (counter-based RNG)
+ * The opt-in alternative to the host draws that replay the reference's MT19937 streams (frcnn_pack_rpn_targets'
+ * rank lists, frcnn_gather_det_samples' host-drawn index): the same sampling RULE, a different stream, no host round
+ * trip, and the calls can be captured in a CUDA graph.
+ *   state [2] i64 (device) = (seed, offset), read and never written: the caller advances offset by `batch` after a
+ *   call (ops.sample_rpn_ / ops.sample_det do, stream-ordered).  Image b draws from
+ *     word(j, tag) = word j & 3 of curand_Philox4x32_10(ctr = (j >> 2, img_lo, img_hi, tag), key = (seed_lo, seed_hi))
+ *   with img = offset + b (64-bit), tag 0 = RPN anchor keys, 1 = detector RoI keys, 2 = detector draws with
+ *   replacement.  Integer arithmetic only: oracle/sample_oracle.py reproduces every result bit for bit.
+ *
+ * RPN (rule of rpn_util.py:324-350): P = usable positives (can_use && is_pos), Q = usable negatives, sizes from
+ *   counts [batch,2] (frcnn_label_anchors*'s output).  keep_p = min(|P|, max_pos), keep_q = min(|Q|, sample_size -
+ *   keep_p) (the reference's 128 / 256).  In each category the kept anchors are the `keep` ones with the smallest
+ *   (word(i, 0), i); every other anchor of the category gets can_use = 0 in place; is_pos and bbreg are untouched.  The
+ *   kept set is a uniformly random subset of the size the reference keeps, i.e. the distribution of the reference's
+ *   switch-off of a uniformly random complement.  i is the anchor's flat index on the image's OWN map,
+ *   (y*cols_b + x)*A + a, so the ragged entry equals the uniform entry on each cropped map; padding is not touched.
+ *   Requires 0 <= max_pos <= sample_size.
+ *
+ * Detector (rule of det_util.py:260-306): per image the rows r < n_rows[b] (clamped to n_max) of frcnn_label_rois'
+ *   output, is_pos [batch,n_max] u8; P = rows with is_pos, Q = the other rows, S = n_samples, want_pos = S / 4.
+ *   Positives: all of P if |P| < want_pos, else the want_pos rows with the smallest (word(r, 1), r).
+ *   want_neg = S - #chosen positives.  |Q| >= want_neg: the want_neg rows of Q with the smallest (word(r, 1), r).
+ *   0 < |Q| < want_neg: draws with replacement Q[(uint64(word(t, 2)) * |Q|) >> 32], t = 0..want_neg-1, Q ascending
+ *   (each row's probability is off from 1/|Q| by at most |Q| / 2^32).  |Q| = 0: the reference's tiling of P,
+ *   P[t % |P|].  Rows chosen without replacement are written in ascending row order, positives first; draws with
+ *   replacement in draw order.  out_index [batch,n_samples] i32 (frcnn_gather_det_samples' index), out_has [batch] u8;
+ *   an image without an eligible row gets an all -1 row and out_has = 0.  n_max <= 4096 (FRCNN_ERR_UNSUPPORTED above). */
+FRCNN_API int frcnn_sample_rpn(frcnn_handle* h, void* stream, uint8_t* can_use, const uint8_t* is_pos,
+                               const int32_t* counts, int n_per_image, int max_pos, int sample_size,
+                               const int64_t* state, int batch);
+FRCNN_API int frcnn_sample_rpn_ragged(frcnn_handle* h, void* stream, uint8_t* can_use, const uint8_t* is_pos,
+                                      const int32_t* counts, int rows, int cols, int n_anchors, const int32_t* extents,
+                                      int max_pos, int sample_size, const int64_t* state, int batch);
+FRCNN_API int frcnn_sample_det(frcnn_handle* h, void* stream, const uint8_t* is_pos, const int32_t* n_rows, int n_max,
+                               int n_samples, const int64_t* state, int batch, int32_t* out_index, uint8_t* out_has);
+
 #ifdef __cplusplus
 }
 #endif
