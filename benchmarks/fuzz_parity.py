@@ -4,7 +4,8 @@
     python benchmarks/fuzz_parity.py [--cases 300] [--seed 0]
 
 Draws shapes / thresholds / limits the fixed test parametrisations do not cover (NMS stopping inside a tile, 1-box
-inputs, heavy ties, thresholds at 0 and 1, odd channel counts and pool sizes, ragged batches, RoI labelling, detector
+inputs, heavy ties, thresholds at 0 and 1 and off the p/q ratios, NMS boxes with negative, invalid or near-16000
+coordinates, odd channel counts and pool sizes, ragged batches, RoI labelling, detector
 post-processing) and compares every result bit for bit with the oracle (resize-mode RoI backward: 1e-5 relative;
 log()-based regression targets: 1 float32 ulp).  Prints one JSON summary line."""
 import argparse
@@ -33,12 +34,22 @@ def host(t):
 def case_nms(rng):
     n = int(rng.choice([1, 2, 63, 64, 65, 200, 1000, 3000]))
     span = int(rng.choice([20, 60, 200]))
-    x1, y1 = rng.integers(0, span, n), rng.integers(0, span, n)
-    boxes = np.stack([x1, y1, x1 + rng.integers(0, 40, n), y1 + rng.integers(0, 40, n)], 1).astype(np.int16)
+    # offsets: non-negative (16-bit packed pair test), negative, or around 16000 (both leave the packed test)
+    dx, dy = (int(rng.choice([0, 0, -int(rng.integers(1, 60)), 16000 - span - int(rng.integers(0, 60))])) for _ in range(2))
+    x1, y1 = dx + rng.integers(0, span, n), dy + rng.integers(0, span, n)
+    w, h = rng.integers(1, 41, n), rng.integers(1, 41, n)
+    if rng.random() < 0.3:                                      # invalid boxes: a side in [-11, 0], areas <= 0
+        bad = np.where(rng.random(n) < 0.05 + rng.random() * 0.3)[0]
+        side, in_x = rng.integers(-11, 1, len(bad)), rng.random(len(bad)) < 0.5
+        w[bad[in_x]], h[bad[~in_x]] = side[in_x], side[~in_x]
+    # every area, intersection and pairwise area sum stays far inside int16: the oracle's arithmetic does not wrap
+    boxes = np.stack([x1, y1, x1 + w - 1, y1 + h - 1], 1).astype(np.int16)
     if rng.random() < 0.3:                                      # heavy duplicates -> many exact-threshold / IoU 1 pairs
         boxes = boxes[rng.integers(0, max(1, n // 4), n)]
     probs = rng.permutation(n).astype(np.float32) / n if rng.random() < 0.7 else rng.integers(0, 5, n).astype(np.float32)
-    thresh = float(rng.choice([0.0, 0.3, 0.5, 0.7, 0.999, 1.0]))
+    # ratios p/q take the integer pair tests, the others the fixed-point screen (0 < t < 1) or the exact predicate
+    thresh = float(rng.choice([0.0, 0.3, 0.5, 0.7, 0.999, 1.0, 0.65432, 0.71234, np.nextafter(0.7, 1.0),
+                               np.nextafter(0.7, 0.0), 0.3141, 1e-7, -0.5, 1.5]))
     max_boxes = int(rng.choice([1, 2, 7, 64, 65, 300, 2000]))
     pick = O.greedy_nms(boxes, probs, thresh, max_boxes)
     ki, kc, kb, ks = ops.nms_i16(dev(boxes[None]), dev(probs[None]), None, thresh, max_boxes)

@@ -58,7 +58,9 @@ __device__ __forceinline__ bool suppressed_i16(int ax1, int ay1, int ax2, int ay
 
 // Branch-free screening test in 64-bit fixed point: d = inter*2^32 - round(t*2^32)*union.  |d| > union
 // decides (the rounding of t moves d by < union/2); anything inside the band is "uncertain" and is
-// re-examined with the exact double division above.  Valid for 0 < t < 1 and 0 < union < 2^31.
+// re-examined with the exact double division above.  Valid for 0 < t < 1 and 0 < union < 2^31.  A union <= 0
+// (boxes with x2 < x1 - 1 or y2 < y1 - 1 have a negative area) would wrap the unsigned product, so it is
+// "uncertain" too and the exact predicate decides it (inter / union <= t in float64, as numpy does).
 // returns 1 = suppressed, 0 = survives, 2 = uncertain
 __device__ __forceinline__ int screen_i16(int ax1, int ay1, int ax2, int ay2, int a_area, int bx1, int by1,
                                           int bx2, int by2, int b_area, unsigned long long t_fix) {
@@ -68,7 +70,7 @@ __device__ __forceinline__ int screen_i16(int ax1, int ay1, int ax2, int ay2, in
   const int uni = a_area + b_area - inter;
   const long long d = (long long)(((unsigned long long)(unsigned)inter << 32) - t_fix * (unsigned long long)(unsigned)uni);
   const long long band = (long long)uni;
-  return (d > band) ? 1 : ((d < -band && uni > 0) ? 0 : 2);
+  return uni <= 0 ? 2 : (d > band ? 1 : (d < -band ? 0 : 2));
 }
 
 // Thresholds that are a ratio of small integers (0.7 = 7/10 as a double: the RPN's value) need no fixed point and no
@@ -87,20 +89,9 @@ __device__ __forceinline__ int screen_rational(int ax1, int ay1, int ax2, int ay
   return uni > 0 ? (over ? 1 : 0) : 2;
 }
 
-// The same test with 32-bit products, for images whose boxes are small enough that neither product can overflow
-// (3 * maxdim^2 * max(p, q) < 2^31, checked once per image): two IMADs and one compare instead of two wide multiplies
-// and a 64-bit compare.  The kept-list sweep is issue-bound, every instruction of the pair test counts.
-__device__ __forceinline__ int screen_rational32(int ax1, int ay1, int ax2, int ay2, int a_area, int bx1, int by1,
-                                                 int bx2, int by2, int b_area, int p, int q) {
-  const int iw = min(ax2, bx2) - max(ax1, bx1) + 1;
-  const int ih = min(ay2, by2) - max(ay1, by1) + 1;
-  const int inter = max(iw, 0) * max(ih, 0);
-  const int uni = a_area + b_area - inter;
-  const bool over = inter * q > uni * p;
-  return uni > 0 ? (over ? 1 : 0) : 2;
-}
-
-// ... and when, in addition, every box of the image is valid (x2 >= x1, y2 >= y1: union > 0 always, no "uncertain" case):
+// The same test with 32-bit products, for images whose boxes are small enough that no product can overflow
+// (3 * maxdim^2 * max(p, q) < 2^31, checked once per image) and all valid (x2 >= x1, y2 >= y1: union > 0 always, no
+// "uncertain" case).  The kept-list sweep is issue-bound, every instruction of the pair test counts, so it is folded:
 // inter*q > (A + B - inter)*p  <=>  inter*(p+q) - A*p > B*p.  The kept list then stores -A*p instead of A and the
 // candidate carries B*p: one IMAD and one compare after the intersection (12 ALU instructions per pair in all).
 __device__ __forceinline__ bool screen_small_valid(int ax1, int ay1, int ax2, int ay2, int neg_ap, int bx1, int by1,
@@ -240,13 +231,14 @@ nms_i16_kernel(const BoxI16* __restrict__ boxes_all, const float* __restrict__ s
     if (tid < NMS_TILE) row_mask[tid] = 0ull;
   }
   __syncthreads();
+  // An invalid box sets s_maxdim = 2^20, which fails the bound, so `small` also means every box is valid; kept_area then
+  // holds -area * p (see screen_small_valid).
   const bool small = rat_q > 0 && 3.0 * (double)s_maxdim * (double)s_maxdim * (double)max(rat_p, rat_q) < 2147483647.0;
-  const bool small_valid = small && s_maxdim < (1 << 20);     // kept_area then holds -area * p (see screen_small_valid)
   // ... and with coordinates below 16000 both corner pairs live in one register each and the intersection is three
   // packed 16-bit DPX instructions: (-max x1, -max y1) = VIMNMX.S16x2 of the negated lows, (min x2+1, min y2+1) =
   // VIMNMX.S16x2, (iw, ih) = relu(sum) = VIADDMNMX.S16x2.RELU; 8 ALU instructions per pair.  kept_box then holds
   // (pack(-x1,-y1), pack(x2+1,y2+1), -area*p, -) -- one 128-bit load per pair and no kept_area load.
-  const bool packed = small_valid && s_maxabs < 16000;
+  const bool packed = small && s_maxabs < 16000;
 
   int parity = 0;
   for (int base = 0; base < n; base += NMS_TILE, parity ^= 1) {
@@ -273,7 +265,7 @@ nms_i16_kernel(const BoxI16* __restrict__ boxes_all, const float* __restrict__ s
           hit |= (int)(d & 0xffffu) * (int)(d >> 16) * pq + kb.z > bp;
         }
         flags = hit ? 1 : 0;
-      } else if (small_valid) {
+      } else if (small) {
         const int bp = b_area * rat_p, pq = rat_p + rat_q;
         bool hit = false;
 #pragma unroll 4
@@ -282,12 +274,6 @@ nms_i16_kernel(const BoxI16* __restrict__ boxes_all, const float* __restrict__ s
           hit |= screen_small_valid(kb.x, kb.y, kb.z, kb.w, kept_area[j], bx1, by1, bx2, by2, bp, pq);
         }
         flags = hit ? 1 : 0;
-      } else if (small) {
-#pragma unroll 4
-        for (int j = slice; j < nlocal; j += SLICES) {
-          const int4 kb = kept_box[j];
-          flags |= screen_rational32(kb.x, kb.y, kb.z, kb.w, kept_area[j], bx1, by1, bx2, by2, b_area, rat_p, rat_q);
-        }
       } else if (rat_q > 0) {
 #pragma unroll 4
         for (int j = slice; j < nlocal; j += SLICES) {
@@ -353,7 +339,7 @@ nms_i16_kernel(const BoxI16* __restrict__ boxes_all, const float* __restrict__ s
           lo1 |= first ? blo : 0u; hi1 |= first ? bhi : 0u;
           lo2 |= first ? 0u : blo; hi2 |= first ? 0u : bhi;
         }
-      } else if (small_valid) {
+      } else if (small) {
         const int pq = rat_p + rat_q;
         const int na1 = -(a1_area * rat_p), na2 = -(a2_area * rat_p);
 #pragma unroll
@@ -473,7 +459,7 @@ nms_i16_kernel(const BoxI16* __restrict__ boxes_all, const float* __restrict__ s
                                           (int)(((unsigned)(bx2 + 1) & 0xffffu) | ((unsigned)(by2 + 1) << 16)), -(b_area * rat_p), 0);
         else
           kept_box[slot / cl] = make_int4(bx1, by1, bx2, by2);
-        kept_area[slot / cl] = small_valid ? -(b_area * rat_p) : b_area;
+        kept_area[slot / cl] = small ? -(b_area * rat_p) : b_area;
       }
       kept_slot[slot] = base + tid;
     }

@@ -74,7 +74,9 @@ def decode_topk(regr, cls, anchor_dims, stride, k, want_dense=False, extents=Non
 def nms_i16(boxes, scores, n=None, overlap_thresh=0.7, max_boxes=300):
     """K-b.  boxes (B,n_max,4) i16, scores (B,n_max) f32, n (B,) i32 or None ->
     keep_index (B,max_boxes) i32 (-1 padded), keep_count (B,), keep_boxes, keep_scores.
-    det_util.py:209-256."""
+    det_util.py:209-256.  Areas, intersections and unions are exact integers while every side x2 - x1 + 1, y2 - y1 + 1 is at most 32767 in magnitude, so the result
+    equals the reference's int16 numpy arithmetic wherever that does not wrap (|area|, intersection and
+    |area_i + area_j| < 32768), and that of the same boxes as int64 everywhere else."""
     boxes, scores = _chk(boxes, torch.int16, "boxes", 3), _chk(scores, torch.float32, "scores", 2)
     ctx = get_context(boxes.device)
     b, n_max, _ = boxes.shape
