@@ -5,9 +5,10 @@
 
 Draws shapes / thresholds / limits the fixed test parametrisations do not cover (NMS stopping inside a tile, 1-box
 inputs, heavy ties, thresholds at 0 and 1 and off the p/q ratios, NMS boxes with negative, invalid or near-16000
-coordinates, odd channel counts and pool sizes, ragged batches, RoI labelling, detector
-post-processing) and compares every result bit for bit with the oracle (resize-mode RoI backward: 1e-5 relative;
-log()-based regression targets: 1 float32 ulp).  Prints one JSON summary line."""
+coordinates, odd channel counts and pool sizes, ragged batches, RoI labelling at K up to 128 and 256 GT boxes,
+detector post-processing at K up to 128, M up to 1024, any max_boxes and 'bg' first, last or in the middle) and
+compares every result bit for bit with the oracle (resize-mode RoI backward: 1e-5 relative; log()-based regression
+targets: 1 float32 ulp).  Prints one JSON summary line."""
 import argparse
 import json
 import os
@@ -192,31 +193,41 @@ def _ulp_close(got, want, max_ulp=1):
 
 def case_label_rois(rng):
     rows, cols = int(rng.integers(4, 40)), int(rng.integers(4, 64))
-    n, g = int(rng.choice([1, 17, 300, 2000])), int(rng.choice([1, 3, 12, 50]))
+    n, g = int(rng.choice([1, 17, 300, 1023, 1025, 2000])), int(rng.choice([1, 3, 12, 50, 256]))
+    k = int(rng.choice([2, 21, 81, 128]))
     rois = synth.random_rois(n, rows, cols, int(rng.integers(1 << 30)))
     gts = synth.gt_boxes(g, cols * 16, rows * 16, int(rng.integers(1 << 30)))
     gt64 = np.array([[v * (1 / 16) for v in x[1:]] for x in gts], np.float64)
-    gidx = np.array([synth.VOC_CLASS_MAPPING[x[0]] for x in gts], np.int32)
-    out = ops.label_rois(dev(rois[None]), dev(gt64[None]), dev(gidx[None]), dev(np.array([g], np.int32)), 21)
-    e_rois, w_cls, w_tr = O.label_rois(rois, gt64, gidx, 21)
+    gidx = (rng.permutation(g) % (k - 1)).astype(np.int32)     # GT classes covering 0..K-2
+    out = ops.label_rois(dev(rois[None]), dev(gt64[None]), dev(gidx[None]), dev(np.array([g], np.int32)), k)
+    e_rois, w_cls, w_tr = O.label_rois(rois, gt64, gidx, k)
     m = int(host(out[4])[0])
     ok = m == len(e_rois) and np.array_equal(host(out[0])[0, :m], e_rois) and np.array_equal(host(out[1])[0, :m], w_cls)
     ok = ok and _ulp_close(host(out[2])[0, :m], w_tr)           # log() in the targets: <= 1 ulp after the f32 store
-    return bool(ok), dict(kind="label_rois", n=n, g=g)
+    return bool(ok), dict(kind="label_rois", n=n, g=g, k=k)
 
 
 def case_postprocess(rng):
-    m, k = int(rng.choice([64, 128, 320])), 21
+    k = int(rng.choice([21, 33, 81, 128]))
+    m = int(rng.choice([64, 128, 320, 1000, 1024, int(rng.integers(1, 1025))]))
+    bg = int(rng.choice([k - 1, k - 1, 0, k // 2]))
+    max_boxes = int(rng.choice([1, 2, 7, 300, 2000]))
     rois = synth.random_rois(m, 37, 62, int(rng.integers(1 << 30)))
     oc, orr = synth.detector_outputs(m, k, int(rng.integers(1 << 30)))
     ratio, thr = float(rng.choice([0.75, 1.0, 1.6, 2.2])), float(rng.choice([0.0, 0.2, 0.5]))
-    boxes, probs, dcls, count = ops.det_postprocess(dev(rois[None]), dev(oc[None]), dev(orr[None]), dev(np.array([ratio])), 20, 16, thr)
-    want = O.det_postprocess(rois, oc, orr, 20, 16, ratio, det_threshold=thr)
+    boxes, probs, dcls, count = ops.det_postprocess(dev(rois[None]), dev(oc[None]), dev(orr[None]), dev(np.array([ratio])), bg,
+                                                    16, thr, max_boxes=max_boxes)
+    ocl = oc.copy()
+    if bg != k - 1:                                             # class K-1 has no regression columns: dropped like 'bg'
+        drop = np.argmax(ocl, axis=1) == k - 1
+        ocl[drop] = 0.0
+        ocl[drop, bg] = 1.0
+    want = O.det_postprocess(rois, ocl, orr, bg, 16, ratio, det_threshold=thr, max_boxes=max_boxes)
     c = int(host(count)[0])
     ok = c == len(want)
     for i, (wc, wbox, wp) in enumerate(want if ok else []):
         ok &= int(host(dcls)[0, i]) == wc and host(boxes)[0, i].tolist() == wbox.tolist() and float(host(probs)[0, i]) == float(wp)
-    return bool(ok), dict(kind="postprocess", m=m, ratio=ratio, thr=thr)
+    return bool(ok), dict(kind="postprocess", m=m, k=k, bg=bg, max_boxes=max_boxes, ratio=ratio, thr=thr)
 
 
 def main():

@@ -134,7 +134,7 @@ pad_rois_kernel(const unsigned long long* __restrict__ rois, const int* __restri
                 int m_out, unsigned long long* __restrict__ out, int* __restrict__ out_rows) {
   const int img = blockIdx.y;
   const int r = blockIdx.x * 256 + threadIdx.x;
-  const int n = min(count[img], n_max);
+  const int n = min(max(count[img], 0), n_max);               // a negative count is an empty list: rows = 0
   const int rows = (n + group - 1) / group * group;
   if (r == 0) out_rows[img] = rows;
   if (r >= m_out) return;

@@ -1,6 +1,7 @@
 // K-e: detector post-processing, one CTA per image (voc_dets.py:51-86).
 //
-//   per row: class = argmax(out_cls[row]) (first maximum), skip 'bg' / below threshold;
+//   per row: class = argmax(out_cls[row]) (first maximum), skip 'bg' / below threshold / class K-1 when 'bg' is not
+//            last (no regression columns);
 //            deltas = out_reg[row, 4c:4c+4] / [10,10,5,5] (float32);
 //            box = util.transform(roi, deltas) (util.py:55-74: tx*wa in float32, rest float64,
 //            no rounding, no clipping) * stride;
@@ -56,7 +57,9 @@ det_postprocess_kernel(const BoxI16* __restrict__ rois_all, const float* __restr
     int c = 0;
     float conf = p[0];
     for (int q = 1; q < K; ++q) { const float v = p[q]; if (v > conf) { conf = v; c = q; } }
-    if (c == bg || conf < det_thr) { s_cls[r] = -1; s_key[r] = ~0ull; continue; }
+    // out_reg holds 4(K-1) columns indexed by class: with 'bg' not last, class K-1 has none and its rows are dropped
+    // (the reference's slice out_reg[4c:4c+4] is empty there)
+    if (c == bg || c == K - 1 || conf < det_thr) { s_cls[r] = -1; s_key[r] = ~0ull; continue; }
     const float* t = oreg + (size_t)r * 4 * (K - 1) + 4 * c;
     const float tx = __fdiv_rn(t[0], 10.f), ty = __fdiv_rn(t[1], 10.f), tw = __fdiv_rn(t[2], 5.f), th = __fdiv_rn(t[3], 5.f);
     const BoxI16 b = rois[r];

@@ -258,7 +258,9 @@ FRCNN_API int frcnn_roi_max_bwd_compact(frcnn_handle* h, void* stream, const flo
  *   rows >= n_rows[b] are ignored (fixed-shape batches; frcnn_pad_rois gives the
  *   count the reference's batching would have run).  det_boxes [batch,M,4] i32, det_probs
  *   [batch,M] f32, det_cls [batch,M] i32, det_count [batch]; order = classes by
- *   first appearance, rows in NMS pick order. */
+ *   first appearance, rows in NMS pick order.  out_reg's columns 4c..4c+3 belong
+ *   to class c, so with bg_index != K-1 class K-1 has none: rows whose arg-max
+ *   is K-1 are then dropped like 'bg' rows. */
 FRCNN_API int frcnn_det_postprocess(frcnn_handle* h, void* stream, const int16_t* rois, const float* out_cls,
                           const float* out_reg, const double* resize_ratio, const int32_t* n_rows,
                           int m_rows, int n_classes, int bg_index, int stride, double det_threshold,
@@ -295,7 +297,8 @@ FRCNN_API int frcnn_valid_boxes(frcnn_handle* h, void* stream, const float* boxe
 /* RoI batching rule of voc_dets.get_dets (voc_dets.py:37-46): the detector takes `group` RoIs at
  * a time and the last batch is padded with copies of its first RoI.  rois [batch,n_max,4] i16,
  * count [batch] -> out [batch,m_out,4] i16 with m_out >= n_max rounded up to `group`; rows past
- * the padded length are the empty box [0,0,0,0]; out_rows [batch] = count rounded up. */
+ * the padded length are the empty box [0,0,0,0]; out_rows [batch] = count (clamped to 0..n_max)
+ * rounded up. */
 FRCNN_API int frcnn_pad_rois(frcnn_handle* h, void* stream, const int16_t* rois, const int32_t* count,
                              int n_max, int group, int m_out, int batch, int16_t* out, int32_t* out_rows);
 
