@@ -14,7 +14,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 OUT = os.path.join(_HERE, "libfrcnn_b200.so")
 SOURCES = ["capi.cu", "proposals.cu", "nms.cu", "label.cu", "roi.cu", "roi_bwd.cu", "postproc.cu", "boxes.cu", "losses.cu", "evalmatch.cu", "image.cu",
-           "sample.cu"]
+           "sample.cu", "jpeg.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-fmad=false", "-std=c++17",
               "-shared", "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden"]
 

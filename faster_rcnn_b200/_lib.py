@@ -56,6 +56,8 @@ SIGNATURES = {
     "frcnn_voc_pr_ap": (_i, [_p, _p, _p, _p, _i, _d, _p, _i, _p, _p, _p]),
     "frcnn_image_resize_cubic": (_i, [_p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p, _p, _p]),
     "frcnn_image_resize_cubic_ragged": (_i, [_p, _p, _p, _p, _ll, _p, _p, _i, _i, _i, _i, _p, _p, _p]),
+    "frcnn_jpeg_inspect": (_i, [_p, _ll, _p]),
+    "frcnn_jpeg_decode": (_i, [_p, _p, _p, _p, _p, _p, _i, _p, _p, _ll, _p]),
     "frcnn_gt_transform": (_i, [_p, _p, _p, _p, _i, _i, _p, _p, _p]),
     "frcnn_sample_rpn": (_i, [_p, _p, _p, _p, _p, _i, _i, _i, _p, _i]),
     "frcnn_sample_rpn_ragged": (_i, [_p, _p, _p, _p, _p, _i, _i, _i, _p, _i, _i, _p, _i]),

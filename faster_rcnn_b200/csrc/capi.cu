@@ -52,6 +52,9 @@ int launch_image_resize(frcnn_handle*, cudaStream_t, const uint8_t*, int, int, i
                         uint8_t*, float*);
 int launch_image_resize_ragged(frcnn_handle*, cudaStream_t, const uint8_t*, const int64_t*, long long, const int32_t*,
                                const uint8_t*, int, int, int, int, const double*, uint8_t*, float*);
+int jpeg_inspect(const uint8_t*, long long, int32_t*);
+int launch_jpeg_decode(frcnn_handle*, cudaStream_t, const uint8_t*, const uint8_t*, const int64_t*, const int64_t*, int,
+                       uint8_t*, const int64_t*, long long, int32_t*);
 int launch_gt_transform(frcnn_handle*, cudaStream_t, const double*, const int32_t*, int, int, const double*, const double*,
                         double*);
 int launch_sample_rpn(frcnn_handle*, cudaStream_t, uint8_t*, const uint8_t*, const int32_t*, int, int, int, int,
@@ -99,6 +102,20 @@ int arena_get(frcnn_handle* h, cudaStream_t stream, size_t bytes, void** out) {
   h->overflow_bytes[h->n_overflow] = bytes;
   h->n_overflow++;
   *out = p;
+  return FRCNN_OK;
+}
+
+int host_staging(frcnn_handle* h, cudaStream_t stream, size_t bytes) {
+  (void)stream;
+  if (h->pinned_used) FRCNN_CUDA(h, cudaEventSynchronize(h->pinned_done));
+  if (bytes > h->pinned_bytes) {
+    if (h->pinned) cudaFreeHost(h->pinned);
+    h->pinned = nullptr;
+    h->pinned_bytes = 0;
+    FRCNN_CUDA(h, cudaMallocHost(&h->pinned, bytes));
+    h->pinned_bytes = bytes;
+  }
+  h->pinned_used = 1;
   return FRCNN_OK;
 }
 
@@ -180,6 +197,11 @@ int frcnn_create(frcnn_handle** out, int device) {
     delete h;
     return FRCNN_ERR_CUDA;
   }
+  if (cudaEventCreateWithFlags(&h->pinned_done, cudaEventDisableTiming) != cudaSuccess) {
+    cudaEventDestroy(h->handover);
+    delete h;
+    return FRCNN_ERR_CUDA;
+  }
   *out = h;
   return FRCNN_OK;
 }
@@ -190,6 +212,9 @@ void frcnn_destroy(frcnn_handle* h) {
   for (int i = 0; i < h->n_overflow; ++i) cudaFree(h->overflow[i]);
   if (h->arena) cudaFree(h->arena);
   if (h->handover) cudaEventDestroy(h->handover);
+  if (h->pinned_used) cudaEventSynchronize(h->pinned_done);
+  if (h->pinned) cudaFreeHost(h->pinned);
+  if (h->pinned_done) cudaEventDestroy(h->pinned_done);
   delete h;
 }
 
@@ -602,6 +627,21 @@ int frcnn_image_resize_cubic_ragged(frcnn_handle* h, void* stream, const uint8_t
                 "image_resize_cubic_ragged: image too large");
   return launch_image_resize_ragged(h, st, src, src_offsets, src_bytes, geom, flip, channels, dst_height, dst_width, batch,
                                     mean_host, out_u8, out_f32);
+}
+
+int frcnn_jpeg_inspect(const uint8_t* file_host, long long n_bytes, int32_t* hw_host) {
+  return jpeg_inspect(file_host, n_bytes, hw_host);
+}
+
+int frcnn_jpeg_decode(frcnn_handle* h, void* stream, const uint8_t* files_host, const uint8_t* files,
+                      const int64_t* file_offsets_host, const int64_t* file_bytes_host, int batch, uint8_t* out,
+                      const int64_t* out_offsets, long long out_bytes, int32_t* status) {
+  FRCNN_ENTER(h, stream);
+  FRCNN_REQUIRE(h, files_host && files && file_offsets_host && file_bytes_host && out && out_offsets && status,
+                "jpeg_decode: null pointer");
+  FRCNN_REQUIRE(h, batch > 0 && batch <= 65535 && out_bytes >= 0, "jpeg_decode: bad size");
+  return launch_jpeg_decode(h, st, files_host, files, file_offsets_host, file_bytes_host, batch, out, out_offsets,
+                            out_bytes, status);
 }
 
 int frcnn_gt_transform(frcnn_handle* h, void* stream, const double* boxes, const int32_t* n_box, int n_max, int batch,

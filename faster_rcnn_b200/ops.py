@@ -605,13 +605,66 @@ def pack_images(sources):
             t = x if isinstance(x, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(x))
             packed[o:o + n].copy_(t.reshape(-1), non_blocking=True)
     else:
-        pinned = torch.empty((total,), dtype=torch.uint8, pin_memory=True)
-        view = pinned.numpy()
-        for x, o, n in zip(sources, offsets.tolist(), nbytes.tolist()):
-            view[o:o + n] = (x.numpy() if isinstance(x, torch.Tensor) else np.asarray(x)).reshape(-1)
-        packed = pinned.to(ctx.device, non_blocking=True)
+        packed = _stage_pinned([x.numpy() if isinstance(x, torch.Tensor) else np.asarray(x) for x in sources], offsets,
+                               total).to(ctx.device, non_blocking=True)
     sizes = np.array([s[:2] for s in shapes], np.int32).reshape(-1, 2)
     return packed, ctx.to_device(offsets), ctx.to_device(sizes)
+
+
+def _stage_pinned(arrays, offsets, total):
+    """The host arrays written back to back at `offsets` into one pinned (total,) u8 buffer (one upload's source)."""
+    pinned = torch.empty((total,), dtype=torch.uint8, pin_memory=True)
+    view = pinned.numpy()
+    for x, o in zip(arrays, offsets.tolist()):
+        flat = x.reshape(-1).view(np.uint8)
+        view[o:o + flat.size] = flat
+    return pinned
+
+
+def _jpeg_bytes(data):
+    if isinstance(data, (bytes, bytearray, memoryview)):
+        return np.frombuffer(data, np.uint8)
+    if isinstance(data, np.ndarray) and data.dtype == np.uint8 and data.ndim == 1:
+        return np.ascontiguousarray(data)
+    raise TypeError("a JPEG file must be bytes or a 1-D uint8 array, got %s" % type(data).__name__)
+
+
+def jpeg_supported(data):
+    """(height, width) when the device decoder takes this JPEG file (frcnn_jpeg_inspect: baseline Huffman, 8-bit,
+    greyscale or YCbCr 4:4:4 / 4:2:2 / 4:4:0 / 4:2:0 / 4:1:1, no Exif rotation), else None.  Runs on the CPU."""
+    a = _jpeg_bytes(data)
+    hw = np.zeros(2, np.int32)
+    rc = _lib.load().frcnn_jpeg_inspect(a.ctypes.data_as(C.c_void_p), a.size, hw.ctypes.data_as(C.c_void_p))
+    return (int(hw[0]), int(hw[1])) if rc == _lib.OK else None
+
+
+def jpeg_decode(files):
+    """cv2.imdecode(file, IMREAD_COLOR) of every file on the device, bit for bit: files = list of bytes or 1-D uint8
+    arrays, each `jpeg_supported`.  Returns (packed (T,) u8, offsets (B,) i64, sizes (B,2) i32 (h, w), status (B,) i32),
+    CUDA tensors: `pack_images`' layout of the (h, w, 3) BGR images plus a status per image (0, or < 0 when the file's
+    entropy-coded data is corrupt: that image's pixels are zero).  The files are staged in one pinned buffer and uploaded
+    with one copy."""
+    if not isinstance(files, (list, tuple)) or len(files) == 0:
+        raise ValueError("jpeg_decode needs a non-empty list of JPEG files")
+    arrays = [_jpeg_bytes(f) for f in files]
+    hw = [jpeg_supported(a) for a in arrays]
+    bad = [i for i, x in enumerate(hw) if x is None]
+    if bad:
+        raise ValueError("files %s are not JPEG files the device decoder supports (check with jpeg_supported)" % bad)
+    nbytes = np.array([a.size for a in arrays], np.int64)
+    offsets = np.concatenate([[0], np.cumsum(nbytes)[:-1]]).astype(np.int64)
+    sizes = np.array(hw, np.int32).reshape(-1, 2)
+    out_n = sizes[:, 0].astype(np.int64) * sizes[:, 1] * 3
+    out_off = np.concatenate([[0], np.cumsum(out_n)[:-1]]).astype(np.int64)
+    ctx = get_context()
+    pinned = _stage_pinned(arrays, offsets, int(nbytes.sum()))
+    files_dev = pinned.to(ctx.device, non_blocking=True)
+    out = ctx.empty((max(int(out_n.sum()), 1),), torch.uint8)
+    out_offsets = ctx.to_device(out_off)
+    status = ctx.empty((len(arrays),), torch.int32)
+    ctx.call("frcnn_jpeg_decode", C.c_void_p(pinned.data_ptr()), ptr(files_dev), offsets.ctypes.data_as(C.c_void_p),
+             nbytes.ctypes.data_as(C.c_void_p), len(arrays), ptr(out), ptr(out_offsets), out.numel(), ptr(status))
+    return out, out_offsets, ctx.to_device(sizes), status
 
 
 def image_resize_cubic_ragged(src, src_offsets, geom, dst_height, dst_width, flip=None, mean=None, want_u8=True, out=None,

@@ -135,15 +135,25 @@ class Image:
     def data_device(self, mean=None, want_u8=True):
         """The same pixels computed on the GPU from the raw decoded image (one H2D of the uint8 pixels): returns the
         (height,width,C) u8 CUDA tensor, or with `mean` the float32 mean-subtracted tensor as well (ops.image_resize_cubic).
-        Within one grey level of `.data` (OpenCV's own SIMD / generic code paths differ by as much, oracle/image_oracle.py)."""
+        Within one grey level of `.data` (OpenCV's own SIMD / generic code paths differ by as much, oracle/image_oracle.py).
+        A path-backed JPEG file the device decoder supports is decoded on the device (ops.jpeg_decode, bit-exact with
+        cv2.imread), and its compressed bytes are what is uploaded."""
         from . import ops
         from .runtime import get_context
-        raw = np.ascontiguousarray(self._raw())
-        if raw.dtype != np.uint8 or raw.ndim != 3:
-            raise TypeError("data_device needs (H,W,C) uint8 pixels")
-        dev = get_context().to_device(raw[None])
+        files = _jpeg_files([self])
+        if files is not None:
+            packed, _, _, status = ops.jpeg_decode([files[0][0]])
+            h, w = files[0][1]
+            dev = packed[:h * w * 3].view(1, h, w, 3)
+        else:
+            raw = np.ascontiguousarray(self._raw())
+            if raw.dtype != np.uint8 or raw.ndim != 3:
+                raise TypeError("data_device needs (H,W,C) uint8 pixels")
+            dev = get_context().to_device(raw[None])
         out = ops.image_resize_cubic(dev, self.height, self.width, flip=self.flipped and self.image_path is not None,
                                      mean=mean, want_u8=want_u8)
+        if files is not None and int(status[0]) != 0:
+            return _host_decoded(self).data_device(mean=mean, want_u8=want_u8)   # corrupt data: cv2's own recovery
         return tuple(t[0] for t in out) if isinstance(out, tuple) else out[0]
 
     def preprocessed_device(self, mean=None):
@@ -177,18 +187,44 @@ class Image:
         return len(self.gt_boxes)
 
 
+def _jpeg_files(images):
+    """[(file bytes, (h, w))] when every image is path-backed (no in-memory pixels) and every file is a JPEG the device
+    decoder supports, else None."""
+    from . import ops
+    if any(img._data is not None or img.image_path is None for img in images):
+        return None
+    out = []
+    for img in images:
+        try:
+            with open(img.image_path, "rb") as f:
+                data = f.read()
+        except OSError:
+            return None
+        hw = ops.jpeg_supported(data)
+        if hw is None:
+            return None
+        out.append((data, hw))
+    return out
+
+
+def _host_decoded(img):
+    """`img` with its pixels read by cv2.imread (mirrored on access like a path-backed image)."""
+    return Image(img.name, img.width, img.height, img.gt_boxes, img.flipped, img._raw(), img.image_path)
+
+
 def preprocessed_batch_device(images, mean=None, pad_to=None):
     """`Image.preprocessed_device` for a batch of differently sized images in one device call: every image is resized
     (and mirrored, under the rule of `data_device`) to its own height x width, minus the means, into one padded float32
     (B,H,W,C) CUDA tensor whose padding is zero.  (H, W) = the largest image, or `pad_to` (which must hold every image).
-    Returns (padded, extents (B,2) i32 (height, width) on the device).  The raw pixels are packed on the host and uploaded
-    with one copy (`ops.pack_images`, which uploads their offsets and sizes too), the target sizes and mirror flags with
-    one more; `ops.image_resize_cubic_ragged` does the rest."""
+    Returns (padded, extents (B,2) i32 (height, width) on the device).  When every image is a path-backed JPEG file
+    the device decoder supports, the compressed files are uploaded with one copy and decoded on the device
+    (`ops.jpeg_decode`, bit-exact with cv2.imread); otherwise the raw pixels are read with cv2.imread, packed on the host
+    and uploaded with one copy (`ops.pack_images`).  The target sizes and mirror flags take one more upload;
+    `ops.image_resize_cubic_ragged` does the rest."""
     from . import ops
     images = list(images)
     if not images:
         raise ValueError("preprocessed_batch_device needs at least one image")
-    raws = [img._raw() for img in images]
     sizes = np.array([(img.height, img.width) for img in images], np.int32).reshape(-1, 2)
     height, width = (int(v) for v in sizes.max(axis=0))
     if pad_to is not None:
@@ -198,13 +234,24 @@ def preprocessed_batch_device(images, mean=None, pad_to=None):
         height, width = ph, pw
     import torch
     from .runtime import get_context
-    src, offsets, src_sizes = ops.pack_images(raws)
-    # target size and mirror flag of every image in one upload; the source sizes come from pack_images
+    files = _jpeg_files(images)
+    status = None
+    if files is not None:
+        src, offsets, src_sizes, status = ops.jpeg_decode([f for f, _ in files])
+        channels = 3
+    else:
+        raws = [img._raw() for img in images]
+        src, offsets, src_sizes = ops.pack_images(raws)
+        channels = raws[0].shape[2]
+    # target size and mirror flag of every image in one upload; the source sizes come with the sources
     flip = np.array([[img.flipped and img.image_path is not None] for img in images], np.int32)
     meta = get_context(src.device).to_device(np.concatenate([sizes, flip], axis=1))
     extents = meta[:, :2].contiguous()
     geom = torch.cat([src_sizes, extents], dim=1)
     mean = ops.IMAGENET_MEAN_BGR if mean is None else mean
     out = ops.image_resize_cubic_ragged(src, offsets, geom, height, width, flip=meta[:, 2].to(torch.uint8), mean=mean,
-                                        want_u8=False, channels=raws[0].shape[2])
+                                        want_u8=False, channels=channels)
+    if status is not None and bool((status != 0).any()):
+        # corrupt entropy data in some file: cv2.imread's own recovery defines those pixels
+        return preprocessed_batch_device([_host_decoded(img) for img in images], mean=mean, pad_to=pad_to)
     return out, extents

@@ -384,6 +384,40 @@ FRCNN_API int frcnn_image_resize_cubic_ragged(frcnn_handle* h, void* stream, con
                                               int dst_height, int dst_width, int batch, const double* mean_host,
                                               uint8_t* out_u8, float* out_f32);
 
+/* ---- JPEG decode on the device
+ * Replaces the cv2.imread of shapes.Image (shapes.py:19-29): pixels equal to cv2.imdecode(file, IMREAD_COLOR) of
+ * OpenCV 4.13 / libjpeg-turbo 3.1 bit for bit (ISLOW integer IDCT, fancy upsampling, table-driven YCbCr -> BGR;
+ * greyscale files replicated into B, G and R).
+ * Supported files (anything else is FRCNN_ERR_UNSUPPORTED and stays with cv2.imread):
+ *   - SOF0 or SOF1 (baseline / extended sequential, Huffman coded), 8-bit samples, one scan carrying every component,
+ *     no DNL;
+ *   - 1 component, or 3 components that libjpeg takes for YCbCr: a JFIF APP0, else an Adobe APP14 whose transform is
+ *     not 0, else component IDs other than 'R','G','B';
+ *   - chroma sampled 1x1 and luma 1x1, 2x1, 1x2, 2x2 or 4x1 (4:4:4, 4:2:2, 4:4:0, 4:2:0, 4:1:1);
+ *   - no Exif orientation other than 1 (IMREAD_COLOR rotates by it);
+ *   - any DRI restart interval, APPn / COM segments anywhere before the scan, any number of tables per DQT / DHT
+ *     segment, 0xFF fill bytes before markers.
+ * A malformed header (a segment past the end of the file, a table the scan references but nobody defined, a zero
+ * dimension, Huffman counts that overflow their code lengths) is FRCNN_ERR_INVALID.  Every header read is bounds-checked.
+ *
+ * frcnn_jpeg_inspect: no handle, runs on the CPU only.  file_host [n_bytes]; hw_host [2] i32 receives (height, width)
+ * when the file is supported.  Returns FRCNN_OK, FRCNN_ERR_UNSUPPORTED or FRCNN_ERR_INVALID.
+ *
+ * frcnn_jpeg_decode: files_host (pinned or pageable host memory) and files (device) hold the same packed bytes;
+ * file b is [file_offsets_host[b], + file_bytes_host[b]).  Headers are parsed from the host copy; the descriptors are
+ * uploaded from the handle's pinned staging in one copy.  Image b's h*w*3 BGR bytes go to out + out_offsets[b]
+ * (out_offsets [batch] i64 on the device, the layout of frcnn_image_resize_cubic_ragged's src; out_bytes = size of
+ * out); status [batch] i32 (device) = 0, or < 0 for corrupt entropy data: -1 a code missing from its table or a
+ * coefficient index past 63, -2 the data ends before the last block, -3 RSTn markers that do not match DRI, -4 a slot
+ * outside [0, out_bytes) (nothing written).  An image with status -1..-3 gets an all-zero slot; the others are not
+ * affected, and no kernel reads outside an interval's bytes or writes outside an image's slot.  libjpeg's
+ * warn-and-continue output on corrupt data is NOT reproduced.  Returns FRCNN_ERR_UNSUPPORTED / FRCNN_ERR_INVALID
+ * before any launch when a header fails (callers inspect first). */
+FRCNN_API int frcnn_jpeg_inspect(const uint8_t* file_host, long long n_bytes, int32_t* hw_host);
+FRCNN_API int frcnn_jpeg_decode(frcnn_handle* h, void* stream, const uint8_t* files_host, const uint8_t* files,
+                                const int64_t* file_offsets_host, const int64_t* file_bytes_host, int batch, uint8_t* out,
+                                const int64_t* out_offsets, long long out_bytes, int32_t* status);
+
 /* GT boxes of a resized / mirrored image (shapes.py:93-101 Box.resize, :292-300 horizontal_flip): boxes
  * [batch,n_max,4] f64 corners, n_box [batch] i32 (NULL = n_max), ratio [batch] f64, flip_width [batch] f64 (NULL or a
  * negative entry = not mirrored; else the width the box is mirrored about) -> out [batch,n_max,4] f64; float64 like
